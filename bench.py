@@ -4,12 +4,13 @@
     python bench.py --gpus N --steps K --warmup W [--config c2] [--batches-per-launch L]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the CPU implementation of the same path on the host cores
+    python bench.py ... --dump-outputs DIR    # also write a sample of what the last timed step returned
 
 A "step" is one launch of the hot path producing `batches_per_launch` successive GCDataset.sample(batch) calls
 (config.batches_per_launch; 1 reproduces the reference's one-call-per-step usage and is launch-latency bound), made
-through the public call `GCDataset.sample_many(L, B)`.  K steps are a few milliseconds of device time, so the K-step
-loop is repeated R times back to back inside one timed region of >= 250 ms (`repeats`, `timed_region_ms`);
-`ms_per_step` is the region divided by K * R.
+through the public call `GCDataset.sample_many(L, B)`.  Every timed loop runs exactly K steps back to back inside one
+timed region (`timed_region_ms`, `steps_timed`); `ms_per_step` is the region divided by K.  A launch lasts about a
+millisecond, so a region that should not be dominated by clock and scheduler noise wants K of a few hundred.
 
 The headline (top-level keys) is C2 = BASELINE.json configs[1]; the same line carries every config of BASELINE.json
 under `configs` (c1..c5, each with value / roofline / e2e / cpu_baseline), C5 as one trajectory-aligned shard per GPU.
@@ -23,6 +24,12 @@ timed on this box's host cores in the same run.  A launch costs 8-19 us beyond i
 to last about a millisecond (`default_batches_per_launch`) and every config also carries `launch_size_sweep`: the same
 measurement at a quarter and a sixteenth of that size.  `e2e.value` and `e2e.link_gbs` are each the faster of two passes
 (`e2e.passes`): the hosts of this pool are shared and their PCIe rate dips for seconds at a time.
+
+`--dump-outputs DIR` writes, after the headline timed loop of every config, what the last timed step returned: for each
+key of the batch, the same fixed, seeded sample of its L * B transitions as `DIR/<config>.<key>.npy` (float32, or float64
+for keys whose values float32 cannot hold exactly), at most `DUMP_BYTES` in all.  The dataset, the sampler seed and the
+number of launches before that step depend only on the arguments, so two builds run with the same arguments can be
+compared file by file.
 """
 
 from __future__ import annotations
@@ -46,7 +53,8 @@ FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md, used only whe
 NOMINAL_HBM_GBS = 8000.0   # B200 data sheet (SURVEY.md 8(d): quoted next to the measured copy peak)
 HEADLINE = 'c2'
 ALL_CONFIGS = ['c1', 'c2', 'c3', 'c4', 'c5']
-MIN_REGION_MS = 250.0
+DUMP_BYTES = 60_000_000     # --dump-outputs: array bytes written in all (npy headers stay within 64 MB), shared by ALL_CONFIGS
+DUMP_SEED = 0
 
 
 def parse_args():
@@ -62,7 +70,8 @@ def parse_args():
     ap.add_argument('--cpu-seconds', type=float, default=10.0, help='budget of the headline cpu_baseline leg')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
-    ap.add_argument('--min-region-ms', type=float, default=MIN_REGION_MS)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write a fixed, seeded sample of the last timed step of every config as DIR/<config>.<key>.npy')
     return ap.parse_args()
 
 
@@ -300,6 +309,27 @@ def link_probe(torch, device, nbytes, reps=8):
     return best
 
 
+def dump_sample(tensors, key, out_dir):
+    """Write one batch ({name: tensor [L, B, ...]}) as out_dir/<key>.<name>.npy: the same DUMP_SEED-chosen transitions of
+    every name, as many as fit this config's share of DUMP_BYTES, in float32 where that holds every value exactly and in
+    float64 otherwise."""
+    import torch
+
+    narrow = {torch.float32, torch.float16, torch.bfloat16, torch.bool, torch.uint8, torch.int8, torch.int16, torch.uint16}
+    kinds = {name: torch.float32 if t.dtype in narrow else torch.float64 for name, t in tensors.items()}
+    lead = {tuple(t.shape[:2]) for t in tensors.values()}
+    assert len(lead) == 1, lead
+    n = int(np.prod(lead.pop()))
+    row_bytes = sum(int(np.prod(t.shape[2:])) * kinds[name].itemsize for name, t in tensors.items())
+    count = max(1, min(n, DUMP_BYTES // len(ALL_CONFIGS) // row_bytes))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=count, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        idx = torch.from_numpy(rows).to(t.device)
+        sample = t.reshape(n, *t.shape[2:]).index_select(0, idx).to(kinds[name]).cpu().numpy()
+        np.save(os.path.join(out_dir, f'{key}.{name}.npy'), sample)
+
+
 def measure_config(key, args, ctx, headline):
     """All measurements of one workload on this rank; collective calls inside (every rank runs the same sequence)."""
     import ctypes as C
@@ -330,8 +360,14 @@ def measure_config(key, args, ctx, headline):
         dist_util.barrier()
         torch.cuda.synchronize(local)
 
+    keep_last = args.dump_outputs is not None     # the headline loop holds on to its newest batch for --dump-outputs
+    last_batch = None
+
     def launch():
+        nonlocal last_batch
         batch = sampler.sample_many(cur_L[0], w.batch)           # the public call: dict of DeviceArray, [L, B, ...] per key
+        if keep_last:
+            last_batch = batch
         handle = next(iter(batch.values()))._batch
         n = C.c_int32()
         lib.ogb_batch_launches(handle.ptr, C.byref(n))
@@ -381,16 +417,16 @@ def measure_config(key, args, ctx, headline):
     tail = run(warmup + 2, False)   # same hand-over pattern as the timed loop: every recycled block exists
     del tail
     barrier()
-    # how many times the K-step loop must repeat for a region of >= min_region_ms (same R on every rank)
-    probe_ms = dist_util.reduce_scalar(timed(args.steps, False), 'max', device=dev)
-    repeats = max(1, int(np.ceil(args.min_region_ms / max(probe_ms, 1e-3))))
-    n_steps = args.steps * repeats
-    barrier()
+    n_steps = args.steps
     clocks = ClockSampler(local)
     clocks.start()
     elapsed_ms = timed(n_steps, True)
     clocks.stop_flag.set()
     clocks.join()
+    if keep_last:
+        if rank == 0:
+            dump_sample({name: arr.torch() for name, arr in last_batch.items()}, key, args.dump_outputs)
+        keep_last, last_batch = False, None
     kernel_ms = float(np.mean(dominant_ms)) if dominant_ms else elapsed_ms / n_steps
     kernel_name = dominant_seen[0]
     elapsed_ms = dist_util.reduce_scalar(elapsed_ms, 'max', device=dev)   # slowest rank
@@ -398,7 +434,7 @@ def measure_config(key, args, ctx, headline):
     value = dist_util.reduce_scalar(n_steps * per_step, 'sum', device=dev) / (elapsed_ms * 1e-3)
     resident = dataset.native(local).resident_bytes()
 
-    # ---- the same launch at a quarter and a sixteenth of the size (c2: 1024 = the round-1 launch, 256): short regions ----
+    # ---- the same launch at a quarter and a sixteenth of the size (c2: 1024 = the round-1 launch, 256) ----
     sweep = []
     if not os.environ.get('OGB_BENCH_NO_SWEEP'):
         n_launches, n_kernel_ms = launches, len(dominant_ms)
@@ -408,11 +444,8 @@ def measure_config(key, args, ctx, headline):
             cur_L[0] = Ls
             del run(5, False)[:]
             barrier()
-            probe = dist_util.reduce_scalar(timed(10, False), 'max', device=dev)
-            n = 10 * max(1, int(np.ceil(60.0 / max(probe, 1e-3))))
-            barrier()
             before = len(dominant_ms)
-            ms = dist_util.reduce_scalar(timed(n, True), 'max', device=dev) / n
+            ms = dist_util.reduce_scalar(timed(args.steps, True), 'max', device=dev) / args.steps
             k_ms = float(np.mean(dominant_ms[before:])) if len(dominant_ms) > before else ms
             bytes_launch = w.bytes_per_transition * w.batch * Ls
             sweep.append({'batches_per_launch': Ls, 'ms_per_step': ms, 'kernel_ms': k_ms, 'value': world * w.batch * Ls / (ms * 1e-3),
@@ -435,7 +468,7 @@ def measure_config(key, args, ctx, headline):
         rng = np.random.default_rng(rank)
         pos = rng.integers(0, n_valid, size=(4, rows))
         pool[:] = pos + pos // (w.steps - 1)  # valid_idxs[j] = j + j // (T-1) for fixed-length compact trajectories
-        steps_e = max(3, min(args.steps, 50))
+        steps_e = args.steps
         for i in range(3):
             out = host_sampler.sample_many(Le, w.batch, idxs=pool[i % 4])
         # keys the reference fills with equal values share one buffer here (dedup): count every copied byte once
@@ -500,7 +533,7 @@ def measure_config(key, args, ctx, headline):
     traffic, traffic_note = committed_traffic(key, kernel_name, kernel_ms, per_step)
     out_bytes = w.bytes_per_transition * per_step // 2
     result = {
-        'value': value, 'ms_per_step': elapsed_ms / n_steps, 'batches_per_launch': L, 'repeats': repeats,
+        'value': value, 'ms_per_step': elapsed_ms / n_steps, 'batches_per_launch': L,
         'timed_region_ms': elapsed_ms, 'steps_timed': n_steps,
         'roofline': {'bound': 'hbm', 'achieved': achieved, 'peak': peak, 'unit': 'GB/s', 'frac': achieved / peak, 'traffic': traffic,
                      'traffic_source': traffic_note, 'kernel': kernel_name, 'kernel_ms': kernel_ms,
@@ -558,7 +591,7 @@ def run_gpu_arm(args):
             'ms_per_step': head['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
             'dtype': 'u8' if w.obs_dtype == 'uint8' else 'f32', 'data': 'synthetic',
             'config': config_dict(head_key, head['batches_per_launch']),
-            'repeats': head['repeats'], 'timed_region_ms': head['timed_region_ms'], 'steps_timed': head['steps_timed'],
+            'timed_region_ms': head['timed_region_ms'], 'steps_timed': head['steps_timed'],
             'rng': 'on-device Philox4x32-10', 'api': 'GCDataset.sample_many(batches_per_launch, batch) -> dict of device arrays',
             'notes': head['notes'],
             'roofline': head['roofline'], 'clocks': head['clocks'], 'gpu_launches': head['gpu_launches'],

@@ -12,7 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_bench_gpu_arm_prints_the_contract_line():
-    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '20', '--warmup', '3', '--cpu-seconds', '1'],
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '400', '--warmup', '3', '--cpu-seconds', '1'],
                          capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
@@ -22,20 +22,20 @@ def test_bench_gpu_arm_prints_the_contract_line():
                 'dtype', 'data', 'config', 'roofline', 'cpu_baseline', 'e2e', 'clocks', 'gpu_launches'):
         assert key in line, key
     assert line['metric'] == 'relabeled transitions/sec' and line['unit'] == 'transitions/s' and line['n_gpus'] == 1
-    assert line['steps'] == 20 and line['warmup'] == 3 and line['scaling'] == 'weak' and line['data'] == 'synthetic'
+    assert line['steps'] == 400 and line['warmup'] == 3 and line['scaling'] == 'weak' and line['data'] == 'synthetic'
     assert line['config']['key'] == 'c2' and 'workload' in line['config']
     roof = line['roofline']
     assert roof['bound'] == 'hbm' and roof['unit'] == 'GB/s' and 0.05 < roof['frac'] < 1.05
     assert abs(roof['frac'] - roof['achieved'] / roof['peak']) < 1e-6
-    assert line['gpu_launches'] >= 20                        # at least one kernel of ours per timed step
+    assert line['gpu_launches'] >= 400                       # at least one kernel of ours per timed step
     e2e = line['e2e']
     assert e2e['unit'] == line['unit'] and 0 < e2e['value'] < line['value']       # host buffers: PCIe-bound, below the resident rate
-    assert e2e['h2d_bytes_per_step'] > 0 and e2e['d2h_bytes_per_step'] > 0
+    assert e2e['h2d_bytes_per_step'] > 0 and e2e['d2h_bytes_per_step'] > 0 and e2e['steps'] == line['steps']
     cpu = line['cpu_baseline']
     assert cpu['kind'] == 'port' and cpu['cores'] == 1 and cpu['value'] > 0 and cpu['sample']
     assert set(line['clocks']) >= {'sm_mhz', 'sm_max_mhz', 'reasons'}
-    # the timed region is stretched to >= 250 ms by repeating the K-step loop, and says so
-    assert line['repeats'] >= 1 and line['timed_region_ms'] >= 200 and line['steps_timed'] == line['steps'] * line['repeats']
+    # the timed region is exactly --steps launches (~0.7 ms each on C2), and says so
+    assert line['steps_timed'] == line['steps'] and line['timed_region_ms'] >= 200
     assert line['clocks']['samples'] >= 5       # (~125 on most boxes: one NVML poll per 2 ms; some boxes answer NVML in ~20 ms)
     assert 0 < e2e['frac_of_link'] < 1.25 and e2e['link_gbs'] > 1   # (back-to-back copies can edge past the probe's serial copies)
     # every BASELINE.json config rides in the same line
@@ -49,6 +49,28 @@ def test_bench_gpu_arm_prints_the_contract_line():
         assert all(0.05 < s['frac'] < 1.05 and s['value'] > 0 for s in sweep), key
     assert line['configs']['c2']['value'] == line['value']
 
+
+
+def test_bench_dump_outputs_repeat_from_run_to_run(tmp_path):
+    """--dump-outputs DIR: a sample of every key of the last timed step's batch as DIR/<config>.<key>.npy in float32 /
+    float64, at most 64 MB in all, and the same arrays from a second run with the same arguments."""
+    import numpy as np
+
+    dumps = []
+    for run in ('a', 'b'):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--config', 'c4', '--steps', '3', '--warmup', '1',
+                              '--no-cpu-baseline', '--no-e2e', '--dump-outputs', str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT, env=dict(os.environ, OGB_BENCH_NO_SWEEP='1'))
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.splitlines()[-1])['steps_timed'] == 3
+        dumps.append({f: np.load(tmp_path / run / f) for f in os.listdir(tmp_path / run)})
+    a, b = dumps
+    assert set(a) == set(b) and {f'c4.{k}.npy' for k in ('observations', 'next_observations', 'value_goals', 'actor_goals',
+                                                          'actions', 'masks', 'rewards')} <= set(a)
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in a) <= 64e6
+    assert len({len(v) for v in a.values()}) == 1                    # the same transitions of every key
+    for name, v in a.items():
+        assert v.dtype in (np.float32, np.float64) and len(v) > 0 and np.array_equal(v, b[name]), name
 
 def test_bench_reference_arm_prints_the_same_config():
     common = ['--steps', '3', '--warmup', '1']
