@@ -67,7 +67,7 @@ typedef struct {
   int32_t has_p_aug;             /* 0 <=> config['p_aug'] is None */
   double p_aug;
   int32_t frame_stack;           /* 0 <=> config['frame_stack'] is None */
-  int32_t crop_padding;          /* 3 in GCDataset.augment (datasets.py:331) */
+  int32_t crop_padding;          /* 3 in GCDataset.augment (datasets.py:331); 0..127 (shifts are kept as int8) */
   int32_t value_subgoal_steps, actor_subgoal_steps, low_subgoal_steps; /* HGC only, already resolved */
   int32_t has_low_discount;
   double low_discount;
@@ -180,7 +180,7 @@ int ogb_sampler_sample_goals(ogb_sampler* s, const int64_t* idxs, int64_t n, dou
 int ogb_sampler_compute_high_next_idxs(ogb_sampler* s, const int64_t* idxs, const int64_t* final_state_idxs, const int64_t* goal_idxs,
                                        int64_t n, int64_t subgoal_steps, int64_t* out_next, int64_t* out_steps);
 /* GCDataset.augment / batched_random_crop (datasets.py:329-339, :17-33) for one image array: rows `idxs` of the
- * observations, row r cropped at crop[r] = (cy, cx) after edge padding by `padding`. */
+ * observations, row r cropped at crop[r] = (cy, cx) after edge padding by `padding` (0..127). */
 int ogb_sampler_gather_cropped(ogb_sampler* s, const int64_t* idxs, int64_t n, const int64_t* crop, int32_t padding, ogb_batch** out);
 
 /* ATCDataset (datasets.py:369-464), for samplers created with OGB_KIND_ATC.  The anchor set of a temporal offset k

@@ -99,8 +99,13 @@ __device__ __forceinline__ void set_byte(uint32_t* w, int byte_index, uint32_t v
   w[byte_index >> 2] = (w[byte_index >> 2] & ~(0xffu << sh)) | (v << sh);
 }
 
+// Shared-memory distance between the FS source bands: a tensor (TMA) copy needs a 128-byte-aligned shared destination,
+// and band_rows * W * 3 is not a multiple of 128 for every band height (17 rows of 16 px: 816 B).
+__host__ __device__ constexpr int frame_stride_bytes(int band_bytes) { return (band_bytes + 127) & ~127; }
+
 // ------------------------------------------------ TMA kernel ------------------------------------------------
-// grid: one CTA per (batch row g, job, band); dynamic smem = 2 * FS * band_rows * W * 3 bytes (+ alignment).
+// grid: one CTA per (batch row g, job, band); dynamic smem = FS * (frame_stride_bytes(band_bytes) + band_bytes), with
+// band_bytes = band_rows * W * 3.
 template <int FS>
 __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const __grid_constant__ CUtensorMap tmap,
                                                                            const __grid_constant__ FramesParams p) {
@@ -114,8 +119,9 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
   const int row_bytes = p.W * C;                     // one image row of one frame
   const int RB = p.band_rows;
   const int band_bytes = RB * row_bytes;             // per frame
+  const int frame_stride = frame_stride_bytes(band_bytes);
   uint8_t* s_in = smem;
-  uint8_t* s_out = smem + (size_t)FS * band_bytes;
+  uint8_t* s_out = smem + (size_t)FS * frame_stride;
 
   const int64_t item = blockIdx.x;
   const int band = (int)(item % p.n_bands);
@@ -143,7 +149,7 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
     for (int f = 0; f < FS; ++f) {
       int32_t fr = row - (FS - 1 - f);
       fr = fr > first ? fr : first;                  // np.maximum(idxs - i, initial_state_idxs)  datasets.py:364
-      tma_load_3d(s_in + (size_t)f * band_bytes, &tmap, 0, y0 + dy, fr, &bar);
+      tma_load_3d(s_in + (size_t)f * frame_stride, &tmap, 0, y0 + dy, fr, &bar);
     }
   }
   mbar_wait(&bar, 0);
@@ -160,7 +166,7 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
     if (dx == 0) {                                   // aligned fast path: 3 x 16-byte shared loads per frame
 #pragma unroll
       for (int f = 0; f < FS; ++f) {
-        const uint4* sp = reinterpret_cast<const uint4*>(s_in + (size_t)f * band_bytes + (size_t)rc * row_bytes + gq * (kGroupPx * C));
+        const uint4* sp = reinterpret_cast<const uint4*>(s_in + (size_t)f * frame_stride + (size_t)rc * row_bytes + gq * (kGroupPx * C));
 #pragma unroll
         for (int q = 0; q < kSrcWords / 4; ++q) {
           const uint4 v = sp[q];
@@ -177,7 +183,7 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
       const int last_word = (row_bytes >> 2) - 1;
 #pragma unroll
       for (int f = 0; f < FS; ++f) {
-        const uint32_t* rowp = reinterpret_cast<const uint32_t*>(s_in + (size_t)f * band_bytes + (size_t)rc * row_bytes);
+        const uint32_t* rowp = reinterpret_cast<const uint32_t*>(s_in + (size_t)f * frame_stride + (size_t)rc * row_bytes);
         uint32_t w[kSrcWords + 1];
 #pragma unroll
         for (int k = 0; k <= kSrcWords; ++k) w[k] = rowp[min(max(w0 + k, 0), last_word)];
@@ -188,7 +194,7 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
       if (dx < 0 && gq == 0) {
 #pragma unroll
         for (int f = 0; f < FS; ++f) {
-          const uint8_t* px = s_in + (size_t)f * band_bytes + (size_t)rc * row_bytes;   // source pixel 0
+          const uint8_t* px = s_in + (size_t)f * frame_stride + (size_t)rc * row_bytes;   // source pixel 0
           const uint32_t e0 = px[0], e1 = px[1], e2 = px[2];
 #pragma unroll
           for (int k = 0; k < kMaxPad; ++k) {
@@ -198,7 +204,7 @@ __global__ void __launch_bounds__(kFramesThreads) gather_frames_tma_kernel(const
       } else if (dx > 0 && gq == groups - 1) {
 #pragma unroll
         for (int f = 0; f < FS; ++f) {
-          const uint8_t* px = s_in + (size_t)f * band_bytes + (size_t)rc * row_bytes + (p.W - 1) * C;  // source pixel W-1
+          const uint8_t* px = s_in + (size_t)f * frame_stride + (size_t)rc * row_bytes + (p.W - 1) * C;  // source pixel W-1
           const uint32_t e0 = px[0], e1 = px[1], e2 = px[2];
 #pragma unroll
           for (int k = 0; k < kMaxPad; ++k) {

@@ -1129,6 +1129,8 @@ int ogb_sampler_create(ogb_dataset* ds, const ogb_config* cfg, int32_t kind, uin
   if (!ds || !cfg || !out) return fail(OGB_ERR_INVALID, "ogb_sampler_create: null argument");
   if (kind < OGB_KIND_GC || kind > OGB_KIND_ATC) return fail(OGB_ERR_INVALID, "unknown sampler kind %d", kind);
   if (stream_id >= (1u << 24)) return fail(OGB_ERR_INVALID, "stream_id must be < 2^24");
+  // a row's crop shift is stored as int8 (dy, dx) with -128 meaning "not augmented"
+  if (cfg->crop_padding < 0 || cfg->crop_padding > 127) return fail(OGB_ERR_INVALID, "crop padding %d out of [0, 127]", cfg->crop_padding);
   DeviceGuard device_guard(ds->device);
   OGB_CUDA(device_guard.status);
   if (kind == OGB_KIND_ATC) {
@@ -2137,6 +2139,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   }
 
   // image keys: frame stacking + crop fused into the gather
+  bool any_frames_tma = false;
   if (any_frames) {
     std::vector<size_t> frame_keys;
     for (size_t i = 0; i < plan.size(); ++i)
@@ -2158,7 +2161,8 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         for (int d = 1; d < f.ndim - 1; ++d) outer *= f.shape[d];
         fp.H = 1; fp.W = (int)outer; fp.inner_bytes = (int)((f.ndim > 1 ? f.shape[f.ndim - 1] : 1) * f.itemsize);
       }
-      const bool tma = tma_eligible(f, cfg, ka.fs) && crop_pad_eff <= 4;
+      // rb == 0: not a TMA shape, or no band height in (padding, 32] divides H; the generic kernel serves those
+      const int rb = tma_eligible(f, cfg, ka.fs) && crop_pad_eff <= 4 ? band_rows_for(fp.H, crop_pad_eff) : 0;
       for (size_t c = a; c < frame_keys.size() && fp.n_jobs < kMaxFrameJobs; ++c) {
         const KeyPlan& kc = plan[frame_keys[c]];
         if (taken[c] || kc.field != ka.field || kc.fs != ka.fs) continue;
@@ -2171,16 +2175,16 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         job.crop = kc.crop;
         job.fs = kc.fs;
       }
-      if (tma) {
-        const int rb = band_rows_for(fp.H, crop_pad_eff);
-        if (rb == 0) return bail(fail(OGB_ERR_UNSUPPORTED, "no band size for image height %d", fp.H));
+      if (rb > 0) {
         fp.band_rows = rb;
         fp.n_bands = fp.H / rb;
         CUtensorMap tm;
         int rc = get_tmap(s, ka.field, rb, &tm);
         if (rc) return bail(rc);
-        const size_t smem = 2 * (size_t)ka.fs * rb * fp.W * 3;
+        const int band_bytes = rb * fp.W * 3;
+        const size_t smem = (size_t)ka.fs * (ogb::frame_stride_bytes(band_bytes) + band_bytes);
         const int fs = ka.fs;
+        any_frames_tma = true;
         if (b->name_frames.empty()) b->name_frames = kernel_name("gather_frames_tma_kernel", {fs >= 1 && fs <= 3 ? fs : 4});
         gather_launches.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
           fp.row_begin = begin;
@@ -2227,7 +2231,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     phase.mark();   // prepare
     // dominant kernel = the one that moves the batch's bytes: the frame gather, else the row gather (fused or not),
     // else the index kernel itself (datasets whose rows are all <= 16 bytes)
-    b->dominant = any_frames ? "gather_frames_tma_kernel" : fused_launch ? fused_name
+    b->dominant = any_frames ? (any_frames_tma ? "gather_frames_tma_kernel" : "gather_frames_generic_kernel") : fused_launch ? fused_name
                 : any_async ? "gather_rows_async_kernel" : !lsu_keys.empty() ? "gather_rows_kernel" : "relabel_index_kernel";
     // row chunks (multiples of 32 rows, each at least kChunkMinRows): one unless the batch is headed for host memory
     constexpr int64_t kChunkMinRows = 16384;
@@ -2331,6 +2335,7 @@ int ogb_sampler_gather(ogb_sampler* s, int32_t which, const int64_t* idxs, int64
 // reference's randint(0, 2 * padding + 1, (n, 2)).
 int ogb_sampler_gather_cropped(ogb_sampler* s, const int64_t* idxs, int64_t n, const int64_t* crop, int32_t padding, ogb_batch** out) try {
   if (!s || !idxs || !crop || !out || n < 1 || padding < 0) return fail(OGB_ERR_INVALID, "ogb_sampler_gather_cropped: bad argument");
+  if (padding > 127) return fail(OGB_ERR_INVALID, "crop padding %d out of [0, 127]", padding);   // int8 shifts, as in ogb_sampler_create
   for (int64_t r = 0; r < 2 * n; ++r)
     if (crop[r] < 0 || crop[r] > 2 * (int64_t)padding) return fail(OGB_ERR_INVALID, "crop shift out of [0, 2 * padding]");
   PlanBuilder pb;
