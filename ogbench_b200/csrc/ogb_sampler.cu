@@ -164,6 +164,22 @@ int largest_vec_log2(size_t a, size_t b) {  // largest power of two <= 16 dividi
   return v;
 }
 
+// Row gathers: rows per item, the largest power of two whose rows fit the stage budget, so that the items of a 32-row
+// tile are equal (an uneven split, e.g. 28 + 4 rows, makes the short item hold a pipeline slot for little data).
+size_t rows_per_item(size_t pitch, size_t budget) {
+  size_t r = 32;
+  while (r > 1 && r * pitch > budget) r >>= 1;
+  return r;
+}
+
+// Stage budget of a row-gather launch whose widest span is max_pitch bytes: 4 KB stages (2 CTAs per SM) for rows up to
+// 256 bytes, 6 KB (16-row items, 1 CTA per SM) beyond -- C3's 384/288-byte spans run 15 % faster with 16-row items than
+// with 8-row ones.  OGB_STAGE_BYTES overrides the default.
+size_t stage_budget(size_t max_pitch) {
+  const int env = ab().stage_bytes;
+  return std::max<size_t>(env ? (size_t)env : (max_pitch > 256 ? 6144 : 4096), max_pitch);
+}
+
 bool positive_at(const void* data, int dtype, int64_t i) {
   switch (dtype) {
     case OGB_U8: case OGB_BOOL: return ((const uint8_t*)data)[i] > 0;
@@ -1714,13 +1730,17 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         return ds->fields[(size_t)plan[a].field].rec_off < ds->fields[(size_t)plan[c].field].rec_off;
       });
       for (size_t k0 = 0; k0 < keys.size();) {
-        // extend the span while the next field starts within 32 bytes of the end of the current one
+        // extend the span while the next field starts within 32 bytes of the end of the current one, and while one
+        // gather launch still holds the span's outputs (items x fields, at the span's own stage budget: a launch's
+        // budget is never smaller, so it never has more items per span); an over-full span becomes two at a field boundary
         const Field& f0 = ds->fields[(size_t)plan[keys[k0]].field];
         size_t lo = f0.rec_off & ~(size_t)15, hi = f0.rec_off + f0.row_bytes, k1 = k0 + 1;
         bool has_long = f0.row_bytes > 16;
         while (k1 < keys.size()) {
           const Field& fn = ds->fields[(size_t)plan[keys[k1]].field];
           if (fn.rec_off > hi + 32) break;
+          const size_t pitch = round_up(std::max(hi, fn.rec_off + fn.row_bytes) - lo, 16);
+          if ((32 / rows_per_item(pitch, stage_budget(pitch))) * (k1 - k0 + 1) > (size_t)kMaxItemOuts) break;
           hi = std::max(hi, fn.rec_off + fn.row_bytes);
           has_long |= fn.row_bytes > 16;
           ++k1;
@@ -1800,8 +1820,9 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     static const int kWord[5] = {0, 2, 4, 5, 6}, kCount[5] = {2, 2, 1, 1, 2};
     for (int f = 0; f < 5; ++f) point_record = point_record && p.tiny_fields[f].word == kWord[f] && p.tiny_fields[f].n_words == kCount[f];
   }
-  // the index vectors only go to memory when a later launch (or the debug interface) reads them
-  p.write_vecs = ((!fuse && any_async) || span_jobs.size() > (size_t)kMaxRowJobs || !lsu_keys.empty() || any_frames || s->debug) ? 1 : 0;
+  // the index vectors only go to memory when a later launch (or the debug interface) reads them; a fused launch that
+  // leaves span jobs to a second row-gather launch sets it below, where the launch split is known
+  p.write_vecs = ((!fuse && any_async) || !lsu_keys.empty() || any_frames || s->debug) ? 1 : 0;
 
   phase.mark();   // classify
   // ---- prepare every launch once; each is then issued per row chunk ----
@@ -1809,6 +1830,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   std::vector<LaunchFn> gather_launches;
   LaunchFn fused_launch;
   const char* fused_name = "relabel_gather_kernel";
+  bool fused_writes_vecs = false;
 
   LaunchFn index_launch = [&, p](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
     p.row_begin = begin;
@@ -1884,20 +1906,14 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     ap.vec_rows = b->vec_rows;
     ap.total_rows = total;
     const size_t q0 = q;
-    const int env_stage = ab().stage_bytes;
     auto magic = [](uint32_t d) -> uint32_t { return d <= 1 ? 0u : (uint32_t)((((uint64_t)1 << 32) + d - 1) / d); };
-    // rows per item: the largest power of two whose rows fit the stage budget, so that the items of a 32-row tile are
-    // equal (an uneven split, e.g. 28 + 4 rows, makes the short item hold a pipeline slot for little data).
-    // budget: 4 KB stages (2 CTAs per SM) for rows up to 256 bytes, 6 KB (16-row items, 1 CTA per SM) beyond -- C3's
-    // 384/288-byte spans run 15 % faster with 16-row items than with 8-row ones
     size_t q1 = std::min(span_jobs.size(), q0 + (size_t)kMaxRowJobs), budget = 0;
     for (;; --q1) {   // the largest prefix of the remaining jobs whose items and outputs fit one launch
       size_t max_pitch = 0, n_items = 0, n_outs = 0;
       for (size_t t = q0; t < q1; ++t) max_pitch = std::max(max_pitch, span_jobs[t].bytes);
-      budget = std::max<size_t>(env_stage ? (size_t)env_stage : (max_pitch > 256 ? 6144 : 4096), max_pitch);
+      budget = stage_budget(max_pitch);
       for (size_t t = q0; t < q1; ++t) {
-        size_t r = 32;
-        while (r > 1 && r * span_jobs[t].bytes > budget) r >>= 1;
+        const size_t r = rows_per_item(span_jobs[t].bytes, budget);
         n_items += 32 / r;
         n_outs += (32 / r) * span_jobs[t].outs.size();
       }
@@ -1907,7 +1923,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         break;
       }
     }
-    auto rows_for = [&](size_t pitch) { size_t r = 32; while (r > 1 && r * pitch > budget) r >>= 1; return r; };
+    auto rows_for = [&](size_t pitch) { return rows_per_item(pitch, budget); };
     size_t stage = 0;
     for (size_t t = q0; t < q1; ++t) stage = std::max(stage, rows_for(span_jobs[t].bytes) * span_jobs[t].bytes);
     ap.stage_bytes = (int)round_up(stage, 128);
@@ -2006,7 +2022,10 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     // compiled for gather_min_blocks(warps) CTAs per SM, so registers allow at least that many)
     const int ctas_per_sm = (int)std::max<size_t>(1, std::min<size_t>(n_warps <= 8 ? 2 : 1, (size_t)(220 * 1024) / smem));
     if (fuse && q0 == 0) {
-      // index algebra + the first (normally the only) group of row jobs in ONE launch
+      // index algebra + the first (normally the only) group of row jobs in ONE launch; the launches that take the
+      // remaining jobs read the index vectors this one computes
+      if (q1 < span_jobs.size()) p.write_vecs = 1;
+      fused_writes_vecs = p.write_vecs != 0;
       FusedParams* fp = new FusedParams();
       fp->relabel = p;
       fp->gather = ap;
@@ -2217,6 +2236,11 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
       }
     }
   }
+
+  // every launch after a fused one reads the index vectors from memory: the fused launch must have stored them
+  if (fused_launch && !gather_launches.empty() && !fused_writes_vecs)
+    return bail(fail(OGB_ERR_UNSUPPORTED, "internal: a fused launch followed by %zu gather launches does not store the index vectors",
+                     gather_launches.size()));
 
   // ---- issue: index kernel on `first`, gathers on the main stream behind it ----
   {

@@ -135,8 +135,10 @@ CANARY = [
     ('gc', (2,), np.float32, 2, None, 77, 5),         # everything tiny: index kernel only
     ('hgc', (69,), np.float32, 21, None, 250, 3),     # long rows: 16-row items, split launch
     ('hgc', (55,), np.float32, 5, None, 4096, 9),     # big enough for the auxiliary-stream path (>= 32768 rows)
-    ('gc', (7,), np.float16, 3, None, 129, 3),        # 14-byte rows: two-byte element drain
-    ('gc', (13,), np.uint8, 5, None, 95, 2),          # odd-sized byte rows
+    ('gc', (7,), np.float16, 3, None, 129, 3),        # 14-byte rows, 12-byte actions: everything tiny, index kernel only
+    ('gc', (13,), np.uint8, 5, None, 95, 2),          # 13-byte rows: byte drain inside the record span (goal rows tiny)
+    ('gc', (9,), np.float16, 3, None, 129, 3),        # 18-byte rows: two-byte element drain, goal rows too
+    ('gc', (17,), np.uint8, 5, None, 95, 2),          # 17-byte rows: byte drain, goal rows too
     ('gc', (64, 64, 3), np.uint8, 5, 3, 19, 2),       # frames (TMA) + small record span
     ('gc', (20, 12, 4), np.uint8, 5, 3, 21, 1),       # frames (generic kernel)
     ('gc', (300,), np.float32, 4, None, 64, 2),       # 1200-byte rows: few rows per stage
