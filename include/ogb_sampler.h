@@ -132,6 +132,21 @@ int ogb_dataset_set_active_rows(ogb_dataset* ds, int64_t n);      /* ReplayBuffe
 int ogb_dataset_resident_bytes(const ogb_dataset* ds, size_t* out);
 int ogb_dataset_destroy(ogb_dataset* ds);
 
+/* Resident build of a dataset too large to hand over in one call (a directory of shards): the record layout
+ * ogb_dataset_create would give these fields (shape[0] = capacity, data NULL), zero-filled, with no tables yet. */
+int ogb_dataset_create_empty(const ogb_field* fields, int32_t n_fields, int32_t device, ogb_dataset** out);
+/* Write dense host rows of every field (field order, NULL = leave untouched) into rows [row0, row0 + n_rows), through a
+ * pinned double buffer; synchronous at return.  Refused on views, past the capacity, and while a sampler or a view holds
+ * the dataset.  The dataset is unsealed until ogb_dataset_seal. */
+int ogb_dataset_write_rows(ogb_dataset* ds, int64_t row0, int64_t n_rows, const void* const* field_rows, int32_t n_fields);
+/* size = n_rows (<= capacity); builds the shadow next observation and the terminal and valid tables from the device
+ * contents, exactly as ogb_dataset_create does. */
+int ogb_dataset_seal(ogb_dataset* ds, int64_t n_rows);
+/* The dataset of rows [row0, row0 + n_rows) of a sealed parent, sharing its memory (and holding a reference on it), with
+ * its own size, terminal flags and valid tables: every entry point sees a dataset of n_rows rows.  Refused where a field's
+ * base pointer would lose an alignment the kernels assume (OGB_ERR_UNSUPPORTED). */
+int ogb_dataset_view(ogb_dataset* parent, int64_t row0, int64_t n_rows, ogb_dataset** out);
+
 /* GCDataset.__post_init__ (datasets.py:182-211): trajectory boundaries from `terminals`, the asserts, search
  * acceleration tables.  `seed`/`stream_id` key the Philox streams (stream_id = rank or replica number). */
 int ogb_sampler_create(ogb_dataset* ds, const ogb_config* cfg, int32_t kind, uint64_t seed, uint32_t stream_id,

@@ -81,6 +81,10 @@ SIGNATURES = [
     ('ogb_dataset_set_active_rows', C.c_int, [_P, C.c_int64]),
     ('ogb_dataset_resident_bytes', C.c_int, [_P, C.POINTER(C.c_size_t)]),
     ('ogb_dataset_destroy', C.c_int, [_P]),
+    ('ogb_dataset_create_empty', C.c_int, [C.POINTER(Field), C.c_int32, C.c_int32, C.POINTER(_P)]),
+    ('ogb_dataset_write_rows', C.c_int, [_P, C.c_int64, C.c_int64, C.POINTER(C.c_void_p), C.c_int32]),
+    ('ogb_dataset_seal', C.c_int, [_P, C.c_int64]),
+    ('ogb_dataset_view', C.c_int, [_P, C.c_int64, C.c_int64, C.POINTER(_P)]),
     ('ogb_sampler_create', C.c_int, [_P, C.POINTER(Config), C.c_int32, C.c_uint64, C.c_uint32, C.POINTER(_P)]),
     ('ogb_sampler_set_stream', C.c_int, [_P, _P]),
     ('ogb_sampler_set_debug', C.c_int, [_P, C.c_int32]),

@@ -332,11 +332,41 @@ struct DLManagedTensor_ {
 }  // namespace
 
 // ----------------------------------------------------------------------------------------------------------------
+// Pinned double buffer of ogb_dataset_write_rows: block k is packed into host[k & 1] while block k - 1 is still on its way
+// to dev[k & 1 ^ 1] (copy stream) or being repadded into the records (pack stream).
+struct WriteStage {
+  size_t bytes = 0;
+  uint8_t* host[2] = {nullptr, nullptr};
+  uint8_t* dev[2] = {nullptr, nullptr};
+  cudaEvent_t copied[2] = {nullptr, nullptr}, packed[2] = {nullptr, nullptr};
+  cudaStream_t copy = nullptr, pack = nullptr;
+  uint64_t block = 0;
+  ~WriteStage() {
+    if (copy) cudaStreamSynchronize(copy);
+    if (pack) cudaStreamSynchronize(pack);
+    for (int b = 0; b < 2; ++b) {
+      if (host[b]) cudaFreeHost(host[b]);
+      if (dev[b]) cudaFree(dev[b]);
+      if (copied[b]) cudaEventDestroy(copied[b]);
+      if (packed[b]) cudaEventDestroy(packed[b]);
+    }
+    if (copy) cudaStreamDestroy(copy);
+    if (pack) cudaStreamDestroy(pack);
+  }
+};
+
 struct ogb_dataset {
   std::atomic<int> refs{1};
   int device = 0;
-  int64_t size = 0;         // rows allocated
+  int64_t capacity = 0;     // rows allocated
+  int64_t size = 0;         // rows of the dataset (== capacity except for a dataset sealed with fewer rows)
   int64_t active_rows = 0;  // rows that hold data (== size except for a ReplayBuffer that is still filling up)
+  // ogb_dataset_create_empty: the tables below are built by ogb_dataset_seal; no sampler is created before that
+  bool sealed = true;
+  std::unique_ptr<WriteStage> stage;
+  // A view (ogb_dataset_view) shares the rows [row0, row0 + size) of `parent`'s memory -- its field pointers and
+  // record_base are offset by row0 rows -- and holds a reference on it; its terminal and valid tables are its own.
+  ogb_dataset* parent = nullptr;
   std::vector<Field> fields;    // the caller's fields, then (hidden, index >= n_public) the shadow field if there is one
   size_t n_public = 0;
   // Shadow copy of the NEXT row's observation inside every record (row r holds observations[min(r + 1, size - 1)],
@@ -354,6 +384,7 @@ struct ogb_dataset {
   int32_t* d_gap_bucket = nullptr;
   int gap_shift = 0;
   std::vector<int32_t> gaps_host;       // c[m] of valid_mode 2, kept for the sampler's segment table
+  size_t table_bytes = 0;               // device bytes of the valid-row tables (part of resident_bytes)
   uint8_t* record_base = nullptr;       // packed record table: one record per row holding every small field
   size_t record_stride = 0;
   std::vector<uint8_t> terminals_host;  // terminals > 0, one byte per row (tiny next to the data)
@@ -559,15 +590,93 @@ void block_give(ogb_sampler* s, uint8_t* block, size_t bytes, std::vector<cudaEv
   }
 }
 
-void dataset_unref(ogb_dataset* ds) {
-  if (ds->refs.fetch_sub(1) != 1) return;
-  DeviceGuard device_guard(ds->device);
-  for (auto& f : ds->fields) if (f.dptr && !f.in_record) cudaFree(f.dptr);
-  if (ds->record_base) cudaFree(ds->record_base);
+void free_valid_tables(ogb_dataset* ds) {
   if (ds->d_valid_table) cudaFree(ds->d_valid_table);
   if (ds->d_gap_c) cudaFree(ds->d_gap_c);
   if (ds->d_gap_bucket) cudaFree(ds->d_gap_bucket);
+  ds->d_valid_table = ds->d_gap_c = ds->d_gap_bucket = nullptr;
+  ds->resident_bytes -= ds->table_bytes;
+  ds->table_bytes = 0;
+}
+
+void dataset_unref(ogb_dataset* ds) {
+  if (ds->refs.fetch_sub(1) != 1) return;
+  {
+    DeviceGuard device_guard(ds->device);
+    ds->stage.reset();
+    if (!ds->parent) {            // a view's memory belongs to its parent
+      for (auto& f : ds->fields) if (f.dptr && !f.in_record) cudaFree(f.dptr);
+      if (ds->record_base) cudaFree(ds->record_base);
+    }
+    free_valid_tables(ds);
+  }
+  ogb_dataset* parent = ds->parent;
   delete ds;
+  if (parent) dataset_unref(parent);
+}
+
+// Dataset.__init__ (datasets.py:62-63): valid_idxs = nonzero(valids > 0), from the host flags valid_host, as a table of the
+// valid rows or, when at most one row in eight is invalid, as the ranks of the gaps (c[m] = (m-th invalid row) - m).
+int build_valid_tables(ogb_dataset* ds) {
+  free_valid_tables(ds);
+  ds->valid_mode = 0;
+  ds->n_valid = -1;
+  ds->gaps_host.clear();
+  if (ds->valids_field < 0) return 0;
+  const int64_t size = ds->size;
+  const std::vector<uint8_t>& valid = ds->valid_host;
+  std::vector<int32_t> table, gaps;
+  for (int64_t r = 0; r < size; ++r) {
+    if (valid[(size_t)r]) table.push_back((int32_t)r);
+    else gaps.push_back((int32_t)(r - (int64_t)gaps.size()));
+  }
+  ds->n_valid = (int64_t)table.size();
+  if (ds->n_valid == 0) return fail(OGB_ERR_INVALID, "dataset has no valid rows");
+  int rc = 0;
+  if ((int64_t)gaps.size() * 8 <= size) {
+    ds->valid_mode = 2;
+    ds->gap_shift = shift_for(ds->n_valid + 1, (int64_t)gaps.size());
+    std::vector<int32_t> bucket = build_buckets(gaps, ds->n_valid + 1, ds->gap_shift);
+    rc = upload_vector(gaps, &ds->d_gap_c);
+    if (!rc) rc = upload_vector(bucket, &ds->d_gap_bucket);
+    ds->gaps_host = gaps;
+    ds->table_bytes = (gaps.size() + bucket.size()) * 4;
+  } else {
+    ds->valid_mode = 1;
+    rc = upload_vector(table, &ds->d_valid_table);
+    ds->table_bytes = table.size() * 4;
+  }
+  ds->resident_bytes += ds->table_bytes;
+  return rc;
+}
+
+// Everything ogb_dataset_create derives from the uploaded rows [0, size): the shadow next observation, the host flags of
+// `terminals` and `valids`, and the valid-row tables.  ogb_dataset_seal runs the same after the rows have been written.
+int build_tables(ogb_dataset* ds) {
+  const int64_t size = ds->size;
+  if (ds->fields.size() > ds->n_public) {       // the hidden shadow field (the only one)
+    const Field& obs = ds->fields[(size_t)ds->obs_field];
+    const Field& sh = ds->fields[ds->n_public];
+    ds->shadow_next_field = (int)ds->n_public;
+    shadow_next_kernel<<<ds->sm_count * 8, 256>>>(ds->record_base, ds->record_stride, (uint32_t)obs.rec_off, (uint32_t)sh.rec_off,
+                                                   (uint32_t)obs.row_bytes, size, 0, size);
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) return fail(OGB_ERR_CUDA, "shadow fill: %s", cudaGetErrorString(e));
+  }
+  auto host_copy_1d = [&](int fi, std::vector<uint8_t>* flags) -> int {
+    const Field& f = ds->fields[fi];
+    if (f.row_bytes != f.itemsize) return fail(OGB_ERR_UNSUPPORTED, "field '%s' must be one value per row", f.name.c_str());
+    std::vector<uint8_t> raw((size_t)size * f.row_bytes);
+    OGB_CUDA(cudaMemcpy2D(raw.data(), f.row_bytes, f.dptr, f.stride, f.row_bytes, (size_t)size, cudaMemcpyDeviceToHost));
+    flags->resize((size_t)size);
+    for (int64_t r = 0; r < size; ++r) (*flags)[(size_t)r] = positive_at(raw.data(), f.dtype, r) ? 1 : 0;
+    return 0;
+  };
+  ds->terminals_host.clear();
+  ds->valid_host.clear();
+  if (ds->terminals_field >= 0) OGB_TRY(host_copy_1d(ds->terminals_field, &ds->terminals_host));
+  if (ds->valids_field >= 0) OGB_TRY(host_copy_1d(ds->valids_field, &ds->valid_host));
+  return build_valid_tables(ds);
 }
 
 void sampler_unref(ogb_sampler* s) {
@@ -903,7 +1012,9 @@ int ogb_device_count(int* out) try {
   return 0;
 } OGB_CATCH_ALL
 
-int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device, ogb_dataset** out) try {
+// ogb_dataset_create (empty = false) and ogb_dataset_create_empty (empty = true: zero-filled fields of the same layout,
+// tables left to ogb_dataset_seal)
+static int create_dataset(const ogb_field* fields, int32_t n_fields, int32_t device, bool empty, ogb_dataset** out) {
   if (!fields || n_fields <= 0 || !out) return fail(OGB_ERR_INVALID, "ogb_dataset_create: bad arguments");
   DeviceGuard device_guard(device);
   OGB_CUDA(device_guard.status);
@@ -915,8 +1026,9 @@ int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device
   int64_t size = 0;
   for (int i = 0; i < n_fields; ++i) {
     const ogb_field& in = fields[i];
-    if (!in.name || (!in.data && in.on_device != 2) || in.ndim < 1 || in.ndim > OGB_MAX_NDIM || dtype_size(in.dtype) == 0)
+    if (!in.name || (!in.data && in.on_device != 2 && !empty) || in.ndim < 1 || in.ndim > OGB_MAX_NDIM || dtype_size(in.dtype) == 0)
       return bail(fail(OGB_ERR_INVALID, "field %d: bad descriptor", i));
+    if (empty && in.data) return bail(fail(OGB_ERR_INVALID, "field '%s': an empty dataset takes no data", in.name));
     size = std::max<int64_t>(size, in.shape[0]);  // get_size: the longest leaf (datasets.py:11-14)
   }
   for (int i = 0; i < n_fields; ++i)
@@ -924,7 +1036,7 @@ int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device
       return bail(fail(OGB_ERR_INVALID, "field '%s' has %lld rows, dataset size is %lld", fields[i].name,
                        (long long)fields[i].shape[0], (long long)size));
   if (size < 1 || size > (int64_t)2147483000) return bail(fail(OGB_ERR_UNSUPPORTED, "dataset size %lld out of range", (long long)size));
-  ds->size = size;
+  ds->capacity = ds->size = size;
   ds->active_rows = size;
 
   // ---- resident layout ----
@@ -1014,7 +1126,7 @@ int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device
       ds->resident_bytes += padded_bytes;
     }
     const cudaMemcpyKind kind = in.on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    if (in.on_device == 2) {  // zero-filled buffer (ReplayBuffer.create, datasets.py:101-103)
+    if (in.on_device == 2 || empty) {  // zero-filled buffer (ReplayBuffer.create, datasets.py:101-103)
       if (!f.in_record) {     // (the record table is zero-filled as a whole)
         e = cudaMemset(f.dptr, 0, padded_bytes);
         if (e != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "memset of field '%s': %s", in.name, cudaGetErrorString(e)));
@@ -1053,12 +1165,7 @@ int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device
       sh.name = "\x01next_observations";      // not a name a caller can pass
       sh.rec_off = off;
       sh.dptr = ds->record_base + off;
-      ds->shadow_next_field = (int)ds->fields.size();
-      ds->fields.push_back(sh);
-      shadow_next_kernel<<<ds->sm_count * 8, 256>>>(ds->record_base, ds->record_stride, (uint32_t)obs.rec_off, (uint32_t)off,
-                                                     (uint32_t)obs.row_bytes, size, 0, size);
-      cudaError_t e = cudaDeviceSynchronize();
-      if (e != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "shadow fill: %s", cudaGetErrorString(e)));
+      ds->fields.push_back(sh);                // (filled by build_tables)
     }
   }
   ds->terminals_field = ds->find("terminals");
@@ -1066,49 +1173,22 @@ int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device
   ds->next_obs_field = ds->find_under("next_observations");
   ds->oracle_field = ds->find("oracle_reps");
   if (ds->obs_field < 0) return bail(fail(OGB_ERR_ASSERT, "assert 'observations' in data (datasets.py:54)"));
-
-  auto host_copy_1d = [&](int fi, std::vector<uint8_t>* flags) -> int {
-    const Field& f = ds->fields[fi];
-    if (f.row_bytes != f.itemsize) return fail(OGB_ERR_UNSUPPORTED, "field '%s' must be one value per row", f.name.c_str());
-    std::vector<uint8_t> raw((size_t)size * f.row_bytes);
-    OGB_CUDA(cudaMemcpy2D(raw.data(), f.row_bytes, f.dptr, f.stride, f.row_bytes, (size_t)size, cudaMemcpyDeviceToHost));
-    flags->resize((size_t)size);
-    for (int64_t r = 0; r < size; ++r) (*flags)[(size_t)r] = positive_at(raw.data(), f.dtype, r) ? 1 : 0;
-    return 0;
-  };
-  if (ds->terminals_field >= 0) {
-    rc = host_copy_1d(ds->terminals_field, &ds->terminals_host);
-    if (rc) return bail(rc);
-  }
-  if (ds->valids_field >= 0) {  // Dataset.__init__: valid_idxs = nonzero(valids > 0)  (datasets.py:62-63)
-    std::vector<uint8_t> valid;
-    rc = host_copy_1d(ds->valids_field, &valid);
-    if (rc) return bail(rc);
-    ds->valid_host = valid;
-    std::vector<int32_t> table, gaps;
-    for (int64_t r = 0; r < size; ++r) {
-      if (valid[(size_t)r]) table.push_back((int32_t)r);
-      else gaps.push_back((int32_t)(r - (int64_t)gaps.size()));  // c[m] = (m-th invalid row) - m
-    }
-    ds->n_valid = (int64_t)table.size();
-    if (ds->n_valid == 0) return bail(fail(OGB_ERR_INVALID, "dataset has no valid rows"));
-    if ((int64_t)gaps.size() * 8 <= size) {
-      ds->valid_mode = 2;
-      ds->gap_shift = shift_for(ds->n_valid + 1, (int64_t)gaps.size());
-      std::vector<int32_t> bucket = build_buckets(gaps, ds->n_valid + 1, ds->gap_shift);
-      rc = upload_vector(gaps, &ds->d_gap_c);
-      if (!rc) rc = upload_vector(bucket, &ds->d_gap_bucket);
-      ds->gaps_host = gaps;
-      ds->resident_bytes += (gaps.size() + bucket.size()) * 4;
-    } else {
-      ds->valid_mode = 1;
-      rc = upload_vector(table, &ds->d_valid_table);
-      ds->resident_bytes += table.size() * 4;
-    }
+  if (empty) {
+    ds->sealed = false;
+    ds->active_rows = 0;
+    // the zero fill (legacy stream) must be done before ogb_dataset_write_rows writes on its non-blocking streams
+    const cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "zero fill: %s", cudaGetErrorString(e)));
+  } else {
+    rc = build_tables(ds);
     if (rc) return bail(rc);
   }
   *out = ds;
   return 0;
+}
+
+int ogb_dataset_create(const ogb_field* fields, int32_t n_fields, int32_t device, ogb_dataset** out) try {
+  return create_dataset(fields, n_fields, device, false, out);
 } OGB_CATCH_ALL
 
 int ogb_dataset_size(const ogb_dataset* ds, int64_t* out) try {
@@ -1118,6 +1198,7 @@ int ogb_dataset_size(const ogb_dataset* ds, int64_t* out) try {
 } OGB_CATCH_ALL
 int ogb_dataset_set_active_rows(ogb_dataset* ds, int64_t n) try {
   if (!ds) return fail(OGB_ERR_INVALID, "null dataset");
+  if (ds->parent) return fail(OGB_ERR_INVALID, "a view has no active rows of its own");
   if (n < 0 || n > ds->size) return fail(OGB_ERR_INVALID, "active rows must be in [0, %lld]", (long long)ds->size);
   ds->active_rows = n;
   // a buffer that is still filling up clamps idx + 1 at its CURRENT last row (datasets.py:82 with ReplayBuffer.size), which
@@ -1141,12 +1222,151 @@ int ogb_dataset_destroy(ogb_dataset* ds) try {
   return 0;
 } OGB_CATCH_ALL
 
+int ogb_dataset_create_empty(const ogb_field* fields, int32_t n_fields, int32_t device, ogb_dataset** out) try {
+  return create_dataset(fields, n_fields, device, true, out);
+} OGB_CATCH_ALL
+
+int ogb_dataset_write_rows(ogb_dataset* ds, int64_t row0, int64_t n_rows, const void* const* field_rows, int32_t n_fields) try {
+  if (!ds || !field_rows) return fail(OGB_ERR_INVALID, "ogb_dataset_write_rows: null argument");
+  if (ds->parent) return fail(OGB_ERR_INVALID, "rows cannot be written through a view");
+  if (ds->refs.load() > 1) return fail(OGB_ERR_INVALID, "the dataset is held by a sampler or a view: its rows cannot change under it");
+  if (n_fields != (int32_t)ds->n_public) return fail(OGB_ERR_INVALID, "expected %zu field pointers", ds->n_public);
+  if (row0 < 0 || n_rows < 0 || row0 + n_rows > ds->capacity)
+    return fail(OGB_ERR_INDEX, "rows [%lld, %lld) exceed the capacity of %lld rows", (long long)row0, (long long)(row0 + n_rows),
+                (long long)ds->capacity);
+  DeviceGuard device_guard(ds->device);
+  OGB_CUDA(device_guard.status);
+  ds->sealed = false;             // the shadow and the tables no longer describe the rows
+  if (n_rows == 0) return 0;
+  if (!ds->stage) {
+    constexpr size_t kStageBytes = (size_t)8 << 20;
+    size_t bytes = kStageBytes;
+    for (size_t i = 0; i < ds->n_public; ++i) bytes = std::max(bytes, ds->fields[i].row_bytes);
+    std::unique_ptr<WriteStage> st(new WriteStage());
+    st->bytes = bytes;
+    for (int b = 0; b < 2; ++b) {
+      OGB_CUDA(cudaHostAlloc((void**)&st->host[b], bytes, cudaHostAllocDefault));
+      OGB_CUDA(cudaMalloc((void**)&st->dev[b], bytes));
+      OGB_CUDA(cudaEventCreateWithFlags(&st->copied[b], cudaEventDisableTiming));
+      OGB_CUDA(cudaEventCreateWithFlags(&st->packed[b], cudaEventDisableTiming));
+    }
+    OGB_CUDA(cudaStreamCreateWithFlags(&st->copy, cudaStreamNonBlocking));
+    OGB_CUDA(cudaStreamCreateWithFlags(&st->pack, cudaStreamNonBlocking));
+    ds->stage = std::move(st);
+  }
+  WriteStage& st = *ds->stage;
+  for (size_t i = 0; i < ds->n_public; ++i) {
+    if (!field_rows[i]) continue;
+    const Field& f = ds->fields[i];
+    const size_t row = f.row_bytes;
+    const int64_t block_rows = (int64_t)(st.bytes / row);
+    const uint8_t* src = (const uint8_t*)field_rows[i];
+    const int v = std::min(2, largest_vec_log2(row, 16));
+    for (int64_t r = 0; r < n_rows; r += block_rows) {
+      const int64_t n = std::min(block_rows, n_rows - r);
+      const int b = (int)(st.block++ & 1);
+      OGB_CUDA(cudaEventSynchronize(st.copied[b]));     // the pinned buffer is free once its previous copy has finished
+      memcpy(st.host[b], src + (size_t)r * row, (size_t)n * row);
+      uint8_t* dst = f.dptr + (size_t)(row0 + r) * f.stride;
+      if (f.stride == row) {                             // dense rows: straight into place
+        OGB_CUDA(cudaMemcpyAsync(dst, st.host[b], (size_t)n * row, cudaMemcpyHostToDevice, st.copy));
+        OGB_CUDA(cudaEventRecord(st.copied[b], st.copy));
+      } else {                                           // padded rows: the copy of the next block runs under this repad
+        OGB_CUDA(cudaStreamWaitEvent(st.copy, st.packed[b], 0));
+        OGB_CUDA(cudaMemcpyAsync(st.dev[b], st.host[b], (size_t)n * row, cudaMemcpyHostToDevice, st.copy));
+        OGB_CUDA(cudaEventRecord(st.copied[b], st.copy));
+        OGB_CUDA(cudaStreamWaitEvent(st.pack, st.copied[b], 0));
+        repad_rows_kernel<<<ds->sm_count * 8, 256, 0, st.pack>>>(st.dev[b], dst, n, (uint32_t)row, (uint32_t)f.stride, v);
+        OGB_CUDA(cudaGetLastError());
+        OGB_CUDA(cudaEventRecord(st.packed[b], st.pack));
+      }
+    }
+  }
+  OGB_CUDA(cudaStreamSynchronize(st.copy));
+  OGB_CUDA(cudaStreamSynchronize(st.pack));
+  return 0;
+} OGB_CATCH_ALL
+
+int ogb_dataset_seal(ogb_dataset* ds, int64_t n_rows) try {
+  if (!ds) return fail(OGB_ERR_INVALID, "null dataset");
+  if (ds->parent) return fail(OGB_ERR_INVALID, "a view is not sealed: its parent is");
+  if (ds->refs.load() > 1) return fail(OGB_ERR_INVALID, "the dataset is held by a sampler or a view: it cannot be sealed again");
+  if (n_rows < 1 || n_rows > ds->capacity)
+    return fail(OGB_ERR_INVALID, "%lld rows do not fit the capacity of %lld rows", (long long)n_rows, (long long)ds->capacity);
+  DeviceGuard device_guard(ds->device);
+  OGB_CUDA(device_guard.status);
+  ds->stage.reset();
+  ds->sealed = false;
+  ds->size = ds->active_rows = n_rows;
+  OGB_TRY(build_tables(ds));
+  ds->sealed = true;
+  return 0;
+} OGB_CATCH_ALL
+
+int ogb_dataset_view(ogb_dataset* parent, int64_t row0, int64_t n_rows, ogb_dataset** out) try {
+  if (!parent || !out) return fail(OGB_ERR_INVALID, "ogb_dataset_view: null argument");
+  if (!parent->sealed) return fail(OGB_ERR_INVALID, "a view needs a sealed dataset");
+  if (parent->active_rows != parent->size) return fail(OGB_ERR_INVALID, "a view needs a dataset whose rows are all written");
+  if (row0 < 0 || n_rows < 1 || row0 + n_rows > parent->size)
+    return fail(OGB_ERR_INVALID, "view rows [%lld, %lld) are outside the dataset's %lld rows", (long long)row0, (long long)(row0 + n_rows),
+                (long long)parent->size);
+  // The kernels assume of a field's base pointer what cudaMalloc gives and the layout keeps at every row of the full
+  // table: 16-byte span, group and cp.async sources in the records and in padded arrays (also the TMA global address),
+  // 32 bytes for the single 256-bit load of a 32-byte record (point-maze kernel), and the row's own power-of-two
+  // alignment for the whole-row loads of dense rows of at most 16 bytes.
+  auto misaligned = [&](const uint8_t* base, size_t stride, size_t need) {
+    return ((uintptr_t)(base + (size_t)row0 * stride) % need) != 0;
+  };
+  if (parent->record_base && misaligned(parent->record_base, parent->record_stride, parent->record_stride == 32 ? 32 : 16))
+    return fail(OGB_ERR_UNSUPPORTED, "view at row %lld: the record table would lose its alignment", (long long)row0);
+  for (size_t i = 0; i < parent->n_public; ++i) {
+    const Field& f = parent->fields[i];
+    if (f.in_record) continue;    // (offsets inside a record whose base is aligned)
+    const size_t need = f.row_bytes > 16 ? 16 : ((size_t)1 << largest_vec_log2(f.row_bytes, f.row_bytes));
+    if (misaligned(f.dptr, f.stride, need))
+      return fail(OGB_ERR_UNSUPPORTED, "view at row %lld: field '%s' would lose its %zu-byte alignment", (long long)row0, f.name.c_str(), need);
+  }
+  DeviceGuard device_guard(parent->device);
+  OGB_CUDA(device_guard.status);
+  ogb_dataset* v = new ogb_dataset();
+  v->device = parent->device;
+  v->sm_count = parent->sm_count;
+  v->capacity = v->size = v->active_rows = n_rows;
+  v->fields = parent->fields;
+  for (Field& f : v->fields) f.dptr += (size_t)row0 * f.stride;
+  v->n_public = parent->n_public;
+  v->record_used = parent->record_used;
+  v->record_stride = parent->record_stride;
+  if (parent->record_base) v->record_base = parent->record_base + (size_t)row0 * parent->record_stride;
+  v->obs_field = parent->obs_field;
+  v->obs_extra = parent->obs_extra;
+  v->terminals_field = parent->terminals_field;
+  v->valids_field = parent->valids_field;
+  v->next_obs_field = parent->next_obs_field;
+  v->oracle_field = parent->oracle_field;
+  // The parent's shadow of row r is observations[r + 1]: at a view's last row that is the next view's first observation,
+  // not the clamp min(r + 1, n_rows - 1) of the view.  Only the view that ends where the parent ends keeps the shadow; the
+  // others gather next_observations by row.
+  v->shadow_next_field = row0 + n_rows == parent->size ? parent->shadow_next_field : -1;
+  if (!parent->terminals_host.empty())
+    v->terminals_host.assign(parent->terminals_host.begin() + row0, parent->terminals_host.begin() + row0 + n_rows);
+  if (!parent->valid_host.empty())
+    v->valid_host.assign(parent->valid_host.begin() + row0, parent->valid_host.begin() + row0 + n_rows);
+  v->parent = parent;
+  parent->refs.fetch_add(1);
+  const int rc = build_valid_tables(v);
+  if (rc) { dataset_unref(v); return rc; }
+  *out = v;
+  return 0;
+} OGB_CATCH_ALL
+
 int ogb_sampler_create(ogb_dataset* ds, const ogb_config* cfg, int32_t kind, uint64_t seed, uint32_t stream_id, ogb_sampler** out) try {
   if (!ds || !cfg || !out) return fail(OGB_ERR_INVALID, "ogb_sampler_create: null argument");
   if (kind < OGB_KIND_GC || kind > OGB_KIND_ATC) return fail(OGB_ERR_INVALID, "unknown sampler kind %d", kind);
   if (stream_id >= (1u << 24)) return fail(OGB_ERR_INVALID, "stream_id must be < 2^24");
   // a row's crop shift is stored as int8 (dy, dx) with -128 meaning "not augmented"
   if (cfg->crop_padding < 0 || cfg->crop_padding > 127) return fail(OGB_ERR_INVALID, "crop padding %d out of [0, 127]", cfg->crop_padding);
+  if (!ds->sealed) return fail(OGB_ERR_INVALID, "the dataset is not sealed: its rows are still being written (ogb_dataset_seal)");
   DeviceGuard device_guard(ds->device);
   OGB_CUDA(device_guard.status);
   if (kind == OGB_KIND_ATC) {
@@ -1275,6 +1495,7 @@ int ogb_sampler_num_choices(const ogb_sampler* s, int64_t* out) try {
 int ogb_sampler_write_row(ogb_sampler* s, int64_t row, const void* const* field_rows, int32_t n_fields) try {
   if (!s || !field_rows) return fail(OGB_ERR_INVALID, "null argument");
   ogb_dataset* ds = s->ds;
+  if (ds->parent) return fail(OGB_ERR_INVALID, "rows cannot be written through a view");
   if (row < 0 || row >= ds->size) return fail(OGB_ERR_INDEX, "row %lld out of range", (long long)row);
   if (n_fields != (int32_t)ds->n_public) return fail(OGB_ERR_INVALID, "expected %zu field pointers", ds->n_public);
   DeviceGuard device_guard(ds->device);

@@ -124,6 +124,33 @@ class _NativeDataset:
         self.ptr = out
         self.device = device
 
+    @classmethod
+    def empty(cls, fields: Mapping[str, '_ZeroField'], device: int) -> '_NativeDataset':
+        """ogb_dataset_create_empty: the layout of `fields` (shape[0] = capacity), rows written later, tables built at seal."""
+        _native.require_device()
+        keepalive: list = []
+        descs = (_native.Field * len(fields))(*[_describe_field(k, v, keepalive) for k, v in fields.items()])
+        out = C.c_void_p()
+        _native.check(_native.lib().ogb_dataset_create_empty(descs, len(fields), device, C.byref(out)))
+        return cls._adopt(out, device)
+
+    def view(self, row0: int, n_rows: int) -> '_NativeDataset':
+        """ogb_dataset_view: rows [row0, row0 + n_rows) of this (sealed) dataset as a dataset of their own."""
+        out = C.c_void_p()
+        _native.check(_native.lib().ogb_dataset_view(self.ptr, int(row0), int(n_rows), C.byref(out)))
+        return self._adopt(out, self.device)
+
+    @classmethod
+    def _adopt(cls, ptr, device) -> '_NativeDataset':
+        self = cls.__new__(cls)
+        self.ptr, self.device = ptr, device
+        return self
+
+    def size(self) -> int:
+        n = C.c_int64()
+        _native.check(_native.lib().ogb_dataset_size(self.ptr, C.byref(n)))
+        return n.value
+
     def resident_bytes(self) -> int:
         n = C.c_size_t()
         _native.check(_native.lib().ogb_dataset_resident_bytes(self.ptr, C.byref(n)))
@@ -214,6 +241,55 @@ class Dataset(Mapping):
         """Return the rows `idxs` of every field plus next_observations (datasets.py:78-83)."""
         idxs = np.asarray(idxs, dtype=np.int64)
         return self._plain_sampler().sample(len(idxs), idxs)
+
+
+class ResidentDataset(Dataset):
+    """A Dataset whose fields live only in HBM (built by loader.ResidentShards): a whole directory of shards, or the view
+    of one shard inside it.
+
+    The host side keeps what it needs and no copy of the fields: `size`, one byte per row of `valids` (get_random_idxs
+    under rng='numpy') and the field names.  Indexing a field raises, as for ReplayBuffer.  Samplers are created on the
+    device the table lives on; any other device is refused.
+    """
+
+    def __init__(self, nds: _NativeDataset, keys, nested: bool, valids):
+        self._dict = {}
+        self._keys = list(keys)
+        self._nested = nested
+        self.device = nds.device
+        self.size = nds.size()
+        self._valids = valids               # uint8 [size] (valids > 0), or None when the dataset has no 'valids'
+        self._valid_idxs = None
+        self._native = {nds.device: nds}
+        self._plain = {}
+
+    @property
+    def valid_idxs(self):
+        if self._valids is None:
+            raise AttributeError('valid_idxs')
+        if self._valid_idxs is None:
+            self._valid_idxs = np.flatnonzero(self._valids)
+        return self._valid_idxs
+
+    def __getitem__(self, key):
+        raise NotImplementedError(f'field {key!r}: a resident dataset keeps no host copy of its fields')
+
+    def __iter__(self):
+        return iter(self._keys)
+
+    def __len__(self):
+        return len(self._keys)
+
+    def copy(self, add_or_replace=None):
+        raise NotImplementedError('a resident dataset keeps no host copy of its fields to copy')
+
+    def native(self, device: int = 0) -> _NativeDataset:
+        if device not in self._native:
+            raise ValueError(f'the dataset is resident on device {self.device}; a sampler on device {device} cannot read it')
+        return self._native[device]
+
+    def _plain_sampler(self, device=None) -> '_Sampler':
+        return super()._plain_sampler(self.device if device is None else device)
 
 
 class ReplayBuffer(Dataset):

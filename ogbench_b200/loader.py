@@ -6,19 +6,25 @@ arrays in the regular or the compact layout.  It is I/O (np.load, decompression)
 `load_gc_dataset` uploads the fields once and returns a device sampler, and `ShardCycler` reproduces the
 directory-of-shards mode of impls/main.py:81-93,185-199 with the *next* shard loaded and uploaded by a background
 thread while the current one is being sampled, so the swap every `dataset_replace_interval` steps costs nothing.
+`ResidentShards` removes the reload altogether: every shard of a directory is uploaded once into one HBM table, each
+shard is a view of it (the dataset the shard's file would give) and the whole table is the concatenated dataset.
 """
 
 from __future__ import annotations
 
 import atexit
+import ctypes as C
 import glob
 import threading
 import weakref
+import zipfile
+from collections.abc import Mapping
 from typing import Any, Callable, List, Optional
 
 import numpy as np
 
-from .datasets import Dataset, GCDataset
+from . import _native
+from .datasets import Dataset, GCDataset, ResidentDataset, _flatten, _NativeDataset, _ZeroField
 
 
 def load_dataset(dataset_path, ob_dtype=np.float32, action_dtype=np.float32, compact_dataset=False, add_info=False):
@@ -287,3 +293,108 @@ class ShardCycler:
         if self._thread is not None:
             self._thread.join()
             self._thread = None
+
+
+def shard_rows(path) -> int:
+    """Rows of an `.npz` file as its `terminals` header declares them, read from the zip member's `.npy` header without
+    decompressing the data (np.savez and np.savez_compressed files alike)."""
+    with zipfile.ZipFile(path) as zf, zf.open('terminals.npy') as f:
+        version = np.lib.format.read_magic(f)
+        read_header = np.lib.format.read_array_header_1_0 if version == (1, 0) else np.lib.format.read_array_header_2_0
+        shape, _, _ = read_header(f)
+    return int(shape[0])
+
+
+class ResidentShards:
+    """Every shard of a dataset directory, uploaded once into one HBM table.
+
+        shards = ResidentShards(list_shards(path))
+        shards.dataset            # Dataset over every row, shards in path order: the concatenated dataset
+        shards[i], shards[path]   # Dataset of one shard: a view of the table, equal to Dataset.create(**load(path))
+        shards.bounds             # [(row0, n_rows)] per shard
+
+    `load` is the per-file host loader (default: load_dataset(p, compact_dataset=True); `lambda p: make_datasets(name,
+    dataset_path=p)[0]` for '-oraclerep-' and 'singletask' names).  The capacity comes from the files' headers; then the
+    shards are loaded, written and freed one at a time, so host memory peaks at one shard plus a pinned staging buffer.
+    Every shard must load with shard 0's fields, dtypes and row shapes.
+
+    A view keeps the reference's shard-local semantics (goals, trajectory ends and next observations stay inside the
+    shard) and a swap costs no upload; sampling `dataset` draws across every shard instead.  Shards end on trajectory
+    boundaries, so each rank of a multi-GPU run can build its own ResidentShards over its subset of the paths.
+    """
+
+    def __init__(self, paths, load: Optional[Callable[[str], dict]] = None, device: int = 0):
+        self.paths = [str(p) for p in paths]
+        lib = _native.lib()
+        nds, keys, nested, valids, self.bounds = None, None, False, [], []
+        for shard in iter_shards(self.paths, load):
+            if nds is None:
+                keys, nested = shard.keys, shard.nested
+                nds = _NativeDataset.empty({k: _ZeroField((shard.capacity, *s), d) for k, (d, s) in shard.schema.items()}, device)
+            arrays = [np.ascontiguousarray(shard.fields[k]) for k in shard.schema]
+            ptrs = (C.c_void_p * len(arrays))(*[a.ctypes.data for a in arrays])
+            _native.check(lib.ogb_dataset_write_rows(nds.ptr, shard.row0, shard.n_rows, ptrs, len(arrays)))
+            if 'valids' in shard.fields:
+                valids.append((shard.fields['valids'] > 0).astype(np.uint8))
+            self.bounds.append((shard.row0, shard.n_rows))
+            del arrays, ptrs, shard                   # this shard's host arrays go before the next one is loaded
+        n_rows = sum(n for _, n in self.bounds)
+        _native.check(lib.ogb_dataset_seal(nds.ptr, n_rows))
+        flags = np.concatenate(valids) if valids else None
+        self.dataset = ResidentDataset(nds, keys, nested, flags)
+        self._views = [ResidentDataset(nds.view(r0, n), keys, nested, flags[r0:r0 + n] if flags is not None else None)
+                       for r0, n in self.bounds]
+
+    def __len__(self):
+        return len(self.paths)
+
+    def __getitem__(self, key) -> ResidentDataset:
+        """The shard `key` (its index, or its path as given) as a dataset of its own."""
+        if isinstance(key, str):
+            if key not in self.paths:
+                raise KeyError(key)
+            key = self.paths.index(key)
+        return self._views[key]
+
+
+class _Shard:
+    __slots__ = ('path', 'row0', 'n_rows', 'capacity', 'keys', 'nested', 'schema', 'fields')
+
+
+def iter_shards(paths, load: Optional[Callable[[str], dict]] = None):
+    """The host half of ResidentShards: load the shards one at a time, in order, and yield each as a record with its
+    first row in the concatenation (`row0`), its row count, its flattened fields and the schema -- {name: (dtype, row
+    shape)} -- that shard 0 fixed; `capacity` is the rows the files' headers declare in all.  A shard whose fields, dtypes
+    or row shapes differ from shard 0's, or that loads more rows than its header declares, raises ValueError naming it."""
+    paths = [str(p) for p in paths]
+    if not paths:
+        raise ValueError('no shards given')
+    if load is None:
+        load = lambda p: load_dataset(p, compact_dataset=True)  # noqa: E731
+    declared = [shard_rows(p) for p in paths]
+    schema, row0 = None, 0
+    for path, cap in zip(paths, declared):
+        tree = load(path)
+        fields = _flatten(tree)
+        shape = {k: (np.asarray(v).dtype, np.asarray(v).shape[1:]) for k, v in fields.items()}
+        if schema is None:
+            schema, keys, nested = shape, list(tree), any(isinstance(v, Mapping) for v in tree.values())
+        elif shape != schema:
+            raise ValueError(f'{path}: fields {_describe(shape)} differ from those of {paths[0]}: {_describe(schema)}')
+        lengths = {len(v) for v in fields.values()}
+        if len(lengths) != 1:
+            raise ValueError(f'{path}: fields of different lengths {sorted(lengths)}')
+        n = lengths.pop()
+        if n > cap:
+            raise ValueError(f'{path}: {n} rows loaded, the file declares {cap}')
+        shard = _Shard()
+        shard.path, shard.row0, shard.n_rows, shard.capacity = path, row0, n, sum(declared)
+        shard.keys, shard.nested, shard.schema, shard.fields = keys, nested, schema, fields
+        del tree, fields
+        yield shard
+        del shard                                     # (the caller's reference is the last one before the next load)
+        row0 += n
+
+
+def _describe(schema) -> str:
+    return ', '.join(f'{k}: {d}{tuple(s)}' for k, (d, s) in schema.items())
