@@ -168,6 +168,18 @@ int ogb_sampler_num_terminals(const ogb_sampler* s, int64_t* out);
 /* ReplayBuffer.add_transition (datasets.py:134-142): write one row of every field (host pointers in field order,
  * NULL = leave untouched), stream-ordered between the sampler's sample() calls. */
 int ogb_sampler_write_row(ogb_sampler* s, int64_t row, const void* const* field_rows, int32_t n_fields);
+/* ReplayBuffer.add_transition called for n transitions (datasets.py:134-142) in one stream-ordered launch: source row i of
+ * every field goes to row (row0 + i) mod size, for i in [skip, n).  field_rows[f] is a C-contiguous [n, row] array (NULL =
+ * leave the field untouched): host memory where on_device[f] == 0 (on_device NULL: every field), else device memory on the
+ * dataset's device.  n - skip must not exceed the size, so that every row is written once (pass skip = n - size when n is
+ * larger: only the last `size` transitions survive).  Host rows go through a pinned stage; the call returns once the
+ * caller's host memory may be reused.  Device rows are read after the work already issued on producer_stream (NULL: no
+ * wait; 1 / 2: the legacy / per-thread default stream) and after the call returns: *out_ticket numbers this call, and
+ * every call numbered <= *out_retired has finished reading its sources (their memory may be reused).  Refused on views. */
+int ogb_sampler_write_ring(ogb_sampler* s, int64_t row0, int64_t n, int64_t skip, const void* const* field_rows, int32_t n_fields,
+                           const int32_t* on_device, void* producer_stream, uint64_t* out_ticket, uint64_t* out_retired);
+/* The CUDA stream the sampler launches on (a DLPack producer orders its writes before it: __dlpack__(stream=...)). */
+int ogb_sampler_get_stream(const ogb_sampler* s, void** out);
 int ogb_sampler_copy_bounds(const ogb_sampler* s, int64_t* terminal_locs, int64_t* initial_locs); /* host out */
 int ogb_sampler_get_counter(const ogb_sampler* s, uint64_t* out); /* checkpointable RNG position */
 int ogb_sampler_set_counter(ogb_sampler* s, uint64_t counter);

@@ -94,6 +94,9 @@ SIGNATURES = [
     ('ogb_sampler_num_choices', C.c_int, [_P, C.POINTER(C.c_int64)]),
     ('ogb_sampler_num_terminals', C.c_int, [_P, C.POINTER(C.c_int64)]),
     ('ogb_sampler_write_row', C.c_int, [_P, C.c_int64, C.POINTER(C.c_void_p), C.c_int32]),
+    ('ogb_sampler_write_ring', C.c_int, [_P, C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_void_p), C.c_int32,
+                                         C.POINTER(C.c_int32), _P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    ('ogb_sampler_get_stream', C.c_int, [_P, C.POINTER(_P)]),
     ('ogb_sampler_copy_bounds', C.c_int, [_P, _P, _P]),
     ('ogb_sampler_get_counter', C.c_int, [_P, C.POINTER(C.c_uint64)]),
     ('ogb_sampler_set_counter', C.c_int, [_P, C.c_uint64]),

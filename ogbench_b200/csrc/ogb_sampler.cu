@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <deque>
 #include <functional>
 #include <map>
 #include <memory>
@@ -267,6 +268,56 @@ __global__ void repad_rows_kernel(const uint8_t* __restrict__ dense, uint8_t* __
   }
 }
 
+// ogb_sampler_write_ring: dense source rows [0, n_rows) of every field to rows (dst0 + i) mod ring_rows of the dataset's
+// layout.  The host picks each field's access width (2^vec_log2 bytes, up to 16) so that the source, the destination base,
+// the destination stride and the row length are all multiples of it.  n_rows <= ring_rows: every row is written once.
+constexpr int kRingMaxFields = 64;
+struct RingField {
+  const uint8_t* src;
+  uint8_t* dst;
+  uint64_t stride;
+  uint32_t row_bytes;
+  uint32_t vec_log2;
+};
+struct RingParams {
+  RingField f[kRingMaxFields];
+  int n_fields;
+};
+
+template <typename T>
+__device__ __forceinline__ void ring_copy_rows(const RingField& f, int64_t n_rows, int64_t dst0, int64_t ring_rows) {
+  const uint32_t upr = f.row_bytes / (uint32_t)sizeof(T);
+  const int64_t total = n_rows * upr;
+  const T* src = reinterpret_cast<const T*>(f.src);
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    int64_t r;
+    uint32_t c;
+    if (total <= 0x7fffffff) {               // (32-bit division for every launch short of 2^31 accesses per field)
+      r = (uint32_t)e / upr;
+      c = (uint32_t)e - (uint32_t)r * upr;
+    } else {
+      r = e / upr;
+      c = (uint32_t)(e - r * upr);
+    }
+    int64_t d = dst0 + r;
+    if (d >= ring_rows) d -= ring_rows;
+    reinterpret_cast<T*>(f.dst + (size_t)d * f.stride)[c] = src[e];
+  }
+}
+
+__global__ void ring_scatter_kernel(const __grid_constant__ RingParams p, int64_t n_rows, int64_t dst0, int64_t ring_rows) {
+  for (int i = 0; i < p.n_fields; ++i) {
+    const RingField& f = p.f[i];
+    switch (f.vec_log2) {
+      case 4: ring_copy_rows<uint4>(f, n_rows, dst0, ring_rows); break;
+      case 3: ring_copy_rows<uint2>(f, n_rows, dst0, ring_rows); break;
+      case 2: ring_copy_rows<uint32_t>(f, n_rows, dst0, ring_rows); break;
+      case 1: ring_copy_rows<uint16_t>(f, n_rows, dst0, ring_rows); break;
+      default: ring_copy_rows<uint8_t>(f, n_rows, dst0, ring_rows); break;
+    }
+  }
+}
+
 __global__ void searchsorted_warp_kernel(const int64_t* __restrict__ table, int64_t n, const int64_t* __restrict__ keys, int64_t m,
                                          int side_right, int64_t* __restrict__ out) {
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -354,6 +405,25 @@ struct WriteStage {
     if (pack) cudaStreamDestroy(pack);
   }
 };
+
+namespace {
+// Two pinned host blocks and two device blocks of `bytes` each, their events, and a copy stream (and a pack stream when the
+// blocks are unpacked on one of the stage's own).
+int make_write_stage(size_t bytes, bool with_pack, std::unique_ptr<WriteStage>* out) {
+  std::unique_ptr<WriteStage> st(new WriteStage());
+  st->bytes = bytes;
+  for (int b = 0; b < 2; ++b) {
+    OGB_CUDA(cudaHostAlloc((void**)&st->host[b], bytes, cudaHostAllocDefault));
+    OGB_CUDA(cudaMalloc((void**)&st->dev[b], bytes));
+    OGB_CUDA(cudaEventCreateWithFlags(&st->copied[b], cudaEventDisableTiming));
+    OGB_CUDA(cudaEventCreateWithFlags(&st->packed[b], cudaEventDisableTiming));
+  }
+  OGB_CUDA(cudaStreamCreateWithFlags(&st->copy, cudaStreamNonBlocking));
+  if (with_pack) OGB_CUDA(cudaStreamCreateWithFlags(&st->pack, cudaStreamNonBlocking));
+  *out = std::move(st);
+  return 0;
+}
+}  // namespace
 
 struct ogb_dataset {
   std::atomic<int> refs{1};
@@ -481,6 +551,12 @@ struct ogb_sampler {
   };
   std::vector<CachedBlock> block_cache;
   size_t cache_bytes = 0;
+  // ogb_sampler_write_ring: the pinned stage of host rows (host[b] -> dev[b] on the stage's copy stream, `packed[b]` =
+  // the scatter that read dev[b] has finished), and the calls whose device sources may still be read
+  std::unique_ptr<WriteStage> ring_stage;
+  uint64_t ring_ticket = 0, ring_retired = 0;
+  std::deque<std::pair<uint64_t, cudaEvent_t>> ring_in_flight;
+  std::vector<cudaEvent_t> ring_spare_events;
 };
 
 struct ogb_batch {
@@ -701,6 +777,9 @@ void sampler_unref(ogb_sampler* s) {
   if (s->h_flags) cudaFreeHost(s->h_flags);
   if (s->d_neg_lut) cudaFree(s->d_neg_lut);
   if (s->d_pow_lut) cudaFree(s->d_pow_lut);
+  s->ring_stage.reset();
+  for (auto& t : s->ring_in_flight) cudaEventDestroy(t.second);
+  for (cudaEvent_t ev : s->ring_spare_events) cudaEventDestroy(ev);
   dataset_unref(s->ds);
   delete s;
 }
@@ -1242,17 +1321,7 @@ int ogb_dataset_write_rows(ogb_dataset* ds, int64_t row0, int64_t n_rows, const 
     constexpr size_t kStageBytes = (size_t)8 << 20;
     size_t bytes = kStageBytes;
     for (size_t i = 0; i < ds->n_public; ++i) bytes = std::max(bytes, ds->fields[i].row_bytes);
-    std::unique_ptr<WriteStage> st(new WriteStage());
-    st->bytes = bytes;
-    for (int b = 0; b < 2; ++b) {
-      OGB_CUDA(cudaHostAlloc((void**)&st->host[b], bytes, cudaHostAllocDefault));
-      OGB_CUDA(cudaMalloc((void**)&st->dev[b], bytes));
-      OGB_CUDA(cudaEventCreateWithFlags(&st->copied[b], cudaEventDisableTiming));
-      OGB_CUDA(cudaEventCreateWithFlags(&st->packed[b], cudaEventDisableTiming));
-    }
-    OGB_CUDA(cudaStreamCreateWithFlags(&st->copy, cudaStreamNonBlocking));
-    OGB_CUDA(cudaStreamCreateWithFlags(&st->pack, cudaStreamNonBlocking));
-    ds->stage = std::move(st);
+    OGB_TRY(make_write_stage(bytes, true, &ds->stage));
   }
   WriteStage& st = *ds->stage;
   for (size_t i = 0; i < ds->n_public; ++i) {
@@ -1525,6 +1594,167 @@ int ogb_sampler_write_row(ogb_sampler* s, int64_t row, const void* const* field_
   }
   return 0;
 } OGB_CATCH_ALL
+
+int ogb_sampler_get_stream(const ogb_sampler* s, void** out) try {
+  if (!s || !out) return fail(OGB_ERR_INVALID, "null argument");
+  *out = (void*)s->stream;
+  return 0;
+} OGB_CATCH_ALL
+
+// ReplayBuffer.add_transition for n transitions at once (datasets.py:134-142): source row i -> row (row0 + i) mod size for
+// i in [skip, n), every field in one ring_scatter_kernel launch per stage block, ordered on the sampler's stream like
+// ogb_sampler_write_row.  Host rows are packed into the pinned stage (block k + 1 is packed and copied while block k is
+// scattered); device rows are read in place.
+int ogb_sampler_write_ring(ogb_sampler* s, int64_t row0, int64_t n, int64_t skip, const void* const* field_rows, int32_t n_fields,
+                           const int32_t* on_device, void* producer_stream, uint64_t* out_ticket, uint64_t* out_retired) try {
+  if (!s || !field_rows || !out_ticket || !out_retired) return fail(OGB_ERR_INVALID, "null argument");
+  ogb_dataset* ds = s->ds;
+  if (ds->parent) return fail(OGB_ERR_INVALID, "rows cannot be written through a view");
+  const int64_t ring = ds->size;
+  if (row0 < 0 || row0 >= ring) return fail(OGB_ERR_INDEX, "row0 %lld out of [0, %lld)", (long long)row0, (long long)ring);
+  if (n < 0 || skip < 0 || skip > n) return fail(OGB_ERR_INVALID, "need 0 <= skip <= n (got n = %lld, skip = %lld)", (long long)n, (long long)skip);
+  if (n - skip > ring)
+    return fail(OGB_ERR_INVALID, "%lld rows exceed the %lld-row ring: only the last %lld can survive (skip = n - size)",
+                (long long)(n - skip), (long long)ring, (long long)ring);
+  if (n_fields != (int32_t)ds->n_public) return fail(OGB_ERR_INVALID, "expected %zu field pointers", ds->n_public);
+  DeviceGuard device_guard(ds->device);
+  OGB_CUDA(device_guard.status);
+  const int64_t rows = n - skip;
+  std::vector<int> write;                 // fields with a source
+  size_t host_row_bytes = 0;              // bytes of one row of every host source
+  bool any_device = false;
+  for (size_t i = 0; i < ds->n_public; ++i) {
+    if (!field_rows[i]) continue;
+    write.push_back((int)i);
+    if (!on_device || !on_device[i]) {
+      host_row_bytes += ds->fields[i].row_bytes;
+      continue;
+    }
+    cudaPointerAttributes attr{};
+    if (cudaPointerGetAttributes(&attr, field_rows[i]) != cudaSuccess) {
+      cudaGetLastError();
+      attr.type = cudaMemoryTypeUnregistered;
+    }
+    if ((attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) || attr.device != ds->device)
+      return fail(OGB_ERR_INVALID, "field '%s': the source is not device memory of device %d", ds->fields[i].name.c_str(), ds->device);
+    any_device = true;
+  }
+  std::lock_guard<std::mutex> lock(s->mu);
+  while (!s->ring_in_flight.empty()) {    // calls whose scatter has finished no longer read their device sources
+    const cudaError_t q = cudaEventQuery(s->ring_in_flight.front().second);
+    if (q == cudaErrorNotReady) break;
+    if (q != cudaSuccess) return fail(OGB_ERR_CUDA, "ring write event: %s", cudaGetErrorString(q));
+    s->ring_spare_events.push_back(s->ring_in_flight.front().second);
+    s->ring_in_flight.pop_front();
+  }
+  auto take_event = [&](cudaEvent_t* ev) -> int {
+    if (!s->ring_spare_events.empty()) {
+      *ev = s->ring_spare_events.back();
+      s->ring_spare_events.pop_back();
+      return 0;
+    }
+    OGB_CUDA(cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
+    return 0;
+  };
+  const uint64_t ticket = ++s->ring_ticket;
+  if (rows > 0) {
+    if (s->aux_stream) {  // index kernels of big launches read tiny fields on the auxiliary stream
+      cudaEvent_t ev = s->chunk_events[s->next_event];
+      s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
+      OGB_CUDA(cudaEventRecord(ev, s->aux_stream));
+      OGB_CUDA(cudaStreamWaitEvent(s->stream, ev, 0));
+    }
+    if (any_device && producer_stream && producer_stream != (void*)s->stream) {
+      cudaEvent_t ev;
+      OGB_TRY(take_event(&ev));
+      s->ring_spare_events.push_back(ev);   // (a wait takes the event's state when it is issued: free again right away)
+      OGB_CUDA(cudaEventRecord(ev, (cudaStream_t)producer_stream));
+      OGB_CUDA(cudaStreamWaitEvent(s->stream, ev, 0));
+    }
+    WriteStage* st = nullptr;
+    int64_t block_rows = rows;
+    if (host_row_bytes > 0) {
+      if (!s->ring_stage) {
+        size_t all = 0;
+        for (size_t i = 0; i < ds->n_public; ++i) all += round_up(ds->fields[i].row_bytes, 16);
+        OGB_TRY(make_write_stage(std::max<size_t>((size_t)8 << 20, all), false, &s->ring_stage));
+      }
+      st = s->ring_stage.get();
+      block_rows = std::max<int64_t>(1, (int64_t)((st->bytes - 16 * write.size()) / host_row_bytes));
+    }
+    std::vector<size_t> stage_off(ds->n_public, 0);
+    for (int64_t r = 0; r < rows; r += block_rows) {
+      const int64_t k = std::min(block_rows, rows - r);
+      int b = 0;
+      if (st) {
+        b = (int)(st->block++ & 1);
+        OGB_CUDA(cudaEventSynchronize(st->copied[b]));     // host[b] is free once its previous copy has finished
+        size_t off = 0;
+        for (int i : write) {
+          if (on_device && on_device[i]) continue;
+          const size_t row = ds->fields[(size_t)i].row_bytes;
+          memcpy(st->host[b] + off, (const uint8_t*)field_rows[i] + (size_t)(skip + r) * row, (size_t)k * row);
+          stage_off[(size_t)i] = off;
+          off = round_up(off + (size_t)k * row, 16);
+        }
+        OGB_CUDA(cudaStreamWaitEvent(st->copy, st->packed[b], 0));   // dev[b] is free once the scatter that read it has run
+        OGB_CUDA(cudaMemcpyAsync(st->dev[b], st->host[b], off, cudaMemcpyHostToDevice, st->copy));
+        OGB_CUDA(cudaEventRecord(st->copied[b], st->copy));
+        OGB_CUDA(cudaStreamWaitEvent(s->stream, st->copied[b], 0));
+      }
+      for (size_t g = 0; g < write.size(); g += kRingMaxFields) {
+        RingParams p{};
+        p.n_fields = (int)std::min<size_t>(kRingMaxFields, write.size() - g);
+        int64_t max_units = 1;
+        for (int j = 0; j < p.n_fields; ++j) {
+          const int i = write[g + (size_t)j];
+          const Field& f = ds->fields[(size_t)i];
+          const bool dev = on_device && on_device[i];
+          const uint8_t* src = dev ? (const uint8_t*)field_rows[i] + (size_t)(skip + r) * f.row_bytes : st->dev[b] + stage_off[(size_t)i];
+          int v = 4;     // the widest access that divides the row, both bases and the destination stride
+          const uint64_t bits = (uint64_t)f.row_bytes | (uint64_t)f.stride | (uint64_t)(uintptr_t)f.dptr | (uint64_t)(uintptr_t)src;
+          while (v > 0 && (bits & ((1ull << v) - 1)) != 0) --v;
+          p.f[j] = RingField{src, f.dptr, (uint64_t)f.stride, (uint32_t)f.row_bytes, (uint32_t)v};
+          max_units = std::max<int64_t>(max_units, k * (int64_t)(f.row_bytes >> v));
+        }
+        const int grid = (int)std::min<int64_t>((int64_t)ds->sm_count * 8, (max_units + 255) / 256);
+        ring_scatter_kernel<<<grid, 256, 0, s->stream>>>(p, k, (row0 + skip + r) % ring, ring);
+        OGB_CUDA(cudaGetLastError());
+      }
+      if (st) OGB_CUDA(cudaEventRecord(st->packed[b], s->stream));
+    }
+    if (any_device) {
+      cudaEvent_t ev;
+      OGB_TRY(take_event(&ev));
+      OGB_CUDA(cudaEventRecord(ev, s->stream));
+      s->ring_in_flight.emplace_back(ticket, ev);
+    }
+    if (ds->shadow_next_field >= 0 && field_rows[ds->obs_field]) {
+      // row r shadows row r + 1, so the written rows' predecessors change, and the last row shadows itself.  Not fused into
+      // the scatter: row r's shadow reads row r + 1, which another CTA may still be writing.
+      const Field& sh = ds->fields[(size_t)ds->shadow_next_field];
+      const Field& obs = ds->fields[(size_t)ds->obs_field];
+      const int64_t dst0 = (row0 + skip) % ring, end = dst0 + rows;
+      int64_t seg[2][2] = {{0, ring}, {0, 0}};
+      if (rows < ring) {
+        seg[0][0] = std::max<int64_t>(dst0 - 1, 0);
+        seg[0][1] = std::min(end, ring);
+        if (end > ring) seg[1][1] = end - ring;
+      }
+      for (auto& sg : seg) {
+        if (sg[1] <= sg[0]) continue;
+        const int grid = (int)std::min<int64_t>((int64_t)ds->sm_count * 8, ((sg[1] - sg[0]) * (int64_t)obs.row_bytes + 255) / 256);
+        shadow_next_kernel<<<grid, 256, 0, s->stream>>>(ds->record_base, ds->record_stride, (uint32_t)obs.rec_off, (uint32_t)sh.rec_off,
+                                                         (uint32_t)obs.row_bytes, ds->size, sg[0], sg[1]);
+        OGB_CUDA(cudaGetLastError());
+      }
+    }
+  }
+  *out_ticket = ticket;
+  *out_retired = s->ring_in_flight.empty() ? ticket : s->ring_in_flight.front().first - 1;
+  return 0;
+} OGB_CATCH_ALL
+
 int ogb_sampler_num_terminals(const ogb_sampler* s, int64_t* out) try {
   if (!s || !out) return fail(OGB_ERR_INVALID, "null argument");
   *out = (int64_t)s->term_host.size();

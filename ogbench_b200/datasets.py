@@ -15,6 +15,7 @@ reference call sites working unchanged.  There is no CPU implementation behind t
 
 from __future__ import annotations
 
+import collections
 import ctypes as C
 import weakref
 from typing import Any, Dict, Mapping
@@ -62,6 +63,81 @@ def get_size(data) -> int:
 
 def _is_device_array(x) -> bool:
     return not isinstance(x, np.ndarray) and (hasattr(x, '__cuda_array_interface__') or hasattr(x, 'data_ptr'))
+
+
+def ring_plan(pointer: int, size: int, max_size: int, n: int):
+    """(row0, skip, pointer, size) of n add_transition calls on a ring of max_size rows (datasets.py:134-142): rows
+    (row0 + i) % max_size for i in [skip, n) are written (only the last max_size transitions survive), and pointer and size
+    end where n single calls leave them -- size = max(pointer, size) after every call, so it never reaches max_size
+    through a wrap (:141-142)."""
+    if n == 0:
+        return pointer, 0, pointer, size
+    end = pointer + n
+    if end < max_size:                       # no wrap: the largest pointer visited is the last one
+        top = end
+    elif pointer <= max_size - 2:            # the pointer passes max_size - 1 before it wraps to 0
+        top = max_size - 1
+    else:                                    # it starts at max_size - 1: 0, 1, ..., n - 1 after that
+        top = min(n - 1, max_size - 1)
+    return pointer, max(0, n - max_size), end % max_size, max(size, top)
+
+
+_KDL_CUDA = 2
+_DL_DTYPES = {(0, 8): np.int8, (0, 16): np.int16, (0, 32): np.int32, (0, 64): np.int64, (1, 8): np.uint8, (1, 16): np.uint16,
+              (1, 32): np.uint32, (1, 64): np.uint64, (2, 16): np.float16, (2, 32): np.float32, (2, 64): np.float64,
+              (6, 8): np.bool_}
+
+
+def _is_device_leaf(x) -> bool:
+    """A CUDA array (DLPack device kDLCUDA, or __cuda_array_interface__ without DLPack); CPU tensors are host leaves."""
+    if isinstance(x, np.ndarray):
+        return False
+    if hasattr(x, '__dlpack_device__') and hasattr(x, '__dlpack__'):
+        return x.__dlpack_device__()[0] == _KDL_CUDA
+    return hasattr(type(x), '__cuda_array_interface__')   # (on the type: evaluating the property may synchronise)
+
+
+def _c_contiguous(shape, strides, itemsize) -> bool:
+    """strides in bytes; dimensions of length 1 may carry any stride."""
+    step = itemsize
+    for n, st in zip(reversed(shape), reversed(strides)):
+        if n != 1 and st != step:
+            return False
+        step *= n
+    return True
+
+
+def _device_source(name, leaf, dtype, shape, device, stream):
+    """(pointer, keepalive, producer stream or None) of a device leaf, which must already have the field's dtype, the row
+    shape `shape` and be C-contiguous (no cast on the device).  DLPack leaves are exported with `stream` as the consumer,
+    so the producer orders its writes before the sampler's stream reads them."""
+    from .device_array import _DLManagedTensorHead, _PyCapsule_GetPointer
+
+    if hasattr(leaf, '__dlpack__'):
+        dev_type, dev_id = leaf.__dlpack_device__()
+        if dev_id != device:
+            raise ValueError(f'field {name!r}: the leaf lives on cuda:{dev_id}, the buffer on cuda:{device}')
+        capsule = leaf.__dlpack__(stream=stream)
+        head = _DLManagedTensorHead.from_address(_PyCapsule_GetPointer(capsule, b'dltensor'))
+        got_dtype = _DL_DTYPES.get((head.code, head.bits)) if head.lanes == 1 else None
+        got_shape = tuple(C.cast(head.shape, C.POINTER(C.c_int64))[d] for d in range(head.ndim))
+        itemsize = head.bits // 8
+        strides = (None if not head.strides else
+                   tuple(C.cast(head.strides, C.POINTER(C.c_int64))[d] * itemsize for d in range(head.ndim)))
+        ptr, keep, producer = (head.data or 0) + head.byte_offset, capsule, None
+    else:
+        cai = leaf.__cuda_array_interface__
+        got_dtype, got_shape = np.dtype(cai['typestr']), tuple(cai['shape'])
+        strides = None if cai.get('strides') is None else tuple(cai['strides'])
+        ptr, keep, producer = cai['data'][0], leaf, cai.get('stream')
+    if got_dtype is None or np.dtype(got_dtype) != dtype:
+        raise ValueError(f'field {name!r}: device leaves must already have the dtype {dtype} (got {got_dtype}); '
+                         'there is no cast on the device')
+    if got_shape != tuple(shape):
+        raise ValueError(f'field {name!r}: expected a device leaf of shape {tuple(shape)}, got {got_shape}')
+    if strides is not None and not _c_contiguous(got_shape, strides, dtype.itemsize):
+        raise ValueError(f'field {name!r}: device leaves must be C-contiguous')
+    return ptr, keep, producer
 
 
 class _ZeroField:
@@ -360,10 +436,92 @@ class ReplayBuffer(Dataset):
         _native.check(_native.lib().ogb_sampler_write_row(sampler.ptr, int(row), ptrs, len(self._names)))
 
     def add_transition(self, transition):
-        """Add a transition to the replay buffer (datasets.py:134-142)."""
+        """Add a transition to the replay buffer (datasets.py:134-142).  Leaves on the buffer's GPU (torch, JAX, CuPy) are
+        read in place, with the rules of add_transitions."""
+        if any(_is_device_leaf(v) for _, v in _leaves(transition)):
+            self._write_ring(transition, single=True)
+            return
         self._write(self.pointer, transition)
         self.pointer = (self.pointer + 1) % self.max_size
         self.size = max(self.pointer, self.size)
+        self._sync_size()
+
+    def add_transitions(self, transitions):
+        """Add n transitions at once: `transitions` is a dict (or pytree) like add_transition's whose leaves carry a
+        leading axis of length n.  Same effect as `for i in range(n): add_transition({k: v[i] ...})` -- rows, `pointer` and
+        `size` included -- in one stream-ordered launch.
+
+        numpy leaves are cast to the field's dtype as add_transition casts them.  Leaves on the buffer's GPU (anything with
+        `__dlpack__` or `__cuda_array_interface__`: torch, JAX, CuPy) are read in place, after the work their producer has
+        issued so far; they must already have the field's dtype and row shape and be C-contiguous (ValueError otherwise:
+        there is no cast on the device).  Host and device leaves may be mixed.  The call does not wait for the GPU: the
+        library keeps device leaves referenced until the write has read them."""
+        self._write_ring(transitions, single=False)
+
+    def _write_ring(self, transitions, single):
+        sampler = self._plain_sampler(self._device)
+        if self._nested:
+            transitions = _flatten(transitions)
+        leaves = [transitions[name] for name in self._names]          # a missing key is a KeyError, as in tree_map
+        lengths, hosts, devices = {}, {}, {}
+        for name, leaf in zip(self._names, leaves):
+            zf = self._dict[name]
+            if _is_device_leaf(leaf):
+                devices[name] = leaf
+                continue
+            arr = np.asarray(leaf)
+            if single:
+                arr = arr.reshape(1, *zf.shape[1:])
+            elif arr.ndim == 0:
+                raise ValueError(f'field {name!r}: add_transitions needs a leading axis of transitions')
+            try:
+                hosts[name] = np.ascontiguousarray(arr, dtype=zf.dtype).reshape(len(arr), *zf.shape[1:])
+            except ValueError as exc:
+                raise ValueError(f'field {name!r}: rows of shape {zf.shape[1:]} expected ({exc})') from None
+            lengths[name] = len(arr)
+        stream, keep, producers = None, [], set()
+        ptrs = (C.c_void_p * len(self._names))()
+        on_device = (C.c_int32 * len(self._names))()
+        for i, name in enumerate(self._names):
+            if name in hosts:
+                ptrs[i] = hosts[name].ctypes.data
+                continue
+            leaf, zf = devices[name], self._dict[name]
+            if single:
+                rows = zf.shape[1:]
+            else:
+                shape = tuple(getattr(leaf, 'shape', ()))
+                if not shape:
+                    raise ValueError(f'field {name!r}: add_transitions needs a leading axis of transitions')
+                rows = (shape[0], *zf.shape[1:])
+            if stream is None:
+                handle = C.c_void_p()
+                _native.check(_native.lib().ogb_sampler_get_stream(sampler.ptr, C.byref(handle)))
+                stream = handle.value or 1                             # (DLPack's name for the legacy default stream)
+            ptrs[i], src, producer = _device_source(name, leaf, zf.dtype, rows, self._device, stream)
+            on_device[i] = 1
+            keep.append(src)
+            if producer is not None:
+                producers.add(producer)
+            lengths[name] = 1 if single else rows[0]
+        if len(set(lengths.values())) > 1:
+            raise ValueError(f'the leaves hold different numbers of transitions: {lengths}')
+        if len(producers) > 1:
+            raise ValueError('device leaves produced on different streams (__cuda_array_interface__ "stream"): pass them in separate calls')
+        n = next(iter(lengths.values())) if lengths else 0
+        if n == 0:
+            return
+        row0, skip, pointer, size = ring_plan(self.pointer, self.size, self.max_size, n)
+        ticket, retired = C.c_uint64(), C.c_uint64()
+        _native.check(_native.lib().ogb_sampler_write_ring(
+            sampler.ptr, row0, n, skip, ptrs, len(self._names), on_device, C.c_void_p(producers.pop() if producers else None),
+            C.byref(ticket), C.byref(retired)))
+        in_flight = sampler._in_flight
+        if keep:
+            in_flight.append((ticket.value, keep))
+        while in_flight and in_flight[0][0] <= retired.value:
+            in_flight.popleft()
+        self.pointer, self.size = pointer, size
         self._sync_size()
 
     def clear(self):
@@ -434,6 +592,11 @@ class _PinnedBlock:
 _PINNED = _PinnedPool()
 
 
+def _destroy_sampler(ptr, in_flight):
+    _native.lib().ogb_sampler_destroy(ptr)      # (waits for the sampler's stream)
+    in_flight.clear()
+
+
 class _Sampler:
     """Thin owner of an ogb_sampler handle; builds the C config from the reference's config mapping."""
 
@@ -493,7 +656,10 @@ class _Sampler:
         out = C.c_void_p()
         _native.check(_native.lib().ogb_sampler_create(self._nds.ptr, C.byref(cfg), kind, seed, stream_id, C.byref(out)))
         self.ptr = out
-        self._finalizer = weakref.finalize(self, _native.lib().ogb_sampler_destroy, out)
+        # (ticket, sources) of ogb_sampler_write_ring calls whose device sources the stream may still read: released once the
+        # library reports the call retired, or after the sampler (and with it its stream) is gone
+        self._in_flight = collections.deque()
+        self._finalizer = weakref.finalize(self, _destroy_sampler, out, self._in_flight)
         if output == 'numpy':  # the batch is read on the host anyway: let the kernel range-check given idxs (IndexError at the copy)
             _native.check(_native.lib().ogb_sampler_set_deferred_index_check(out, 1))
         self._layouts: Dict[Any, Any] = {}
