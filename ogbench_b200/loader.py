@@ -8,13 +8,18 @@ directory-of-shards mode of impls/main.py:81-93,185-199 with the *next* shard lo
 thread while the current one is being sampled, so the swap every `dataset_replace_interval` steps costs nothing.
 `ResidentShards` removes the reload altogether: every shard of a directory is uploaded once into one HBM table, each
 shard is a view of it (the dataset the shard's file would give) and the whole table is the concatenated dataset.
+`upload_dataset` gives load_dataset's result in HBM without the host copy: the file is inflated, cast, laid out and
+written a block at a time, which is also how ResidentShards reads its files with the default loader.
 """
 
 from __future__ import annotations
 
+import ast
 import atexit
+import contextlib
 import ctypes as C
 import glob
+import queue
 import threading
 import weakref
 import zipfile
@@ -298,11 +303,245 @@ class ShardCycler:
 def shard_rows(path) -> int:
     """Rows of an `.npz` file as its `terminals` header declares them, read from the zip member's `.npy` header without
     decompressing the data (np.savez and np.savez_compressed files alike)."""
-    with zipfile.ZipFile(path) as zf, zf.open('terminals.npy') as f:
-        version = np.lib.format.read_magic(f)
-        read_header = np.lib.format.read_array_header_1_0 if version == (1, 0) else np.lib.format.read_array_header_2_0
-        shape, _, _ = read_header(f)
+    with zipfile.ZipFile(path) as zf, _open_member(zf, path, 'terminals') as f:
+        shape, _, _ = _read_npy_header(f, path, 'terminals')
     return int(shape[0])
+
+
+# ------------------------------------------ streaming .npz members into HBM ------------------------------------------
+_BLOCK_BYTES = 8 << 20          # one block of ogb_dataset_write_rows's pinned stage
+_MAX_HEADER_BYTES = 10000       # np.load's default limit on a .npy header
+_INFO_KEYS = ('qpos', 'qvel', 'button_states')
+
+
+def _open_member(zf: zipfile.ZipFile, path, key):
+    try:
+        return zf.open(f'{key}.npy')
+    except KeyError:
+        raise KeyError(f'{key} is not a file in the archive {path}') from None
+
+
+def _read_npy_header(f, path, key):
+    """(shape, dtype, fortran_order) from the `.npy` header at the start of `f` (format versions 1.0, 2.0 and 3.0), which
+    is left at the first byte of the array data."""
+    magic = f.read(8)
+    if len(magic) != 8 or magic[:6] != b'\x93NUMPY' or magic[6] not in (1, 2, 3) or magic[7] != 0:
+        raise ValueError(f'{path}: member {key!r} is not a .npy array of format version 1.0, 2.0 or 3.0')
+    length = int.from_bytes(f.read(2 if magic[6] == 1 else 4), 'little')
+    text = f.read(length) if length <= _MAX_HEADER_BYTES else b''
+    try:
+        header = ast.literal_eval(text.decode('utf8' if magic[6] == 3 else 'latin1'))
+        shape, fortran = tuple(int(n) for n in header['shape']), bool(header['fortran_order'])
+        dtype = np.lib.format.descr_to_dtype(header['descr'])
+    except Exception as exc:
+        raise ValueError(f'{path}: member {key!r} has an unreadable .npy header') from exc
+    return shape, dtype, fortran
+
+
+def read_member_blocks(path, key, block_rows: Optional[int] = None):
+    """The array `key` of the `.npz` file at `path` (what `np.load(path)[key]` gives), yielded as consecutive blocks of
+    `block_rows` rows, by default about 8 MB of them.  Stored (np.savez) and deflated (np.savez_compressed) members alike,
+    ZIP64 members included; only the current block is held in host memory.  A member that cannot be sliced into rows
+    (Fortran order, object dtype, a 0-d or empty array) is read whole by np.load and yielded as one block.  A member
+    that ends before the row count of its header raises ValueError; a missing member raises KeyError."""
+    with zipfile.ZipFile(path) as zf, _open_member(zf, path, key) as f:
+        shape, dtype, fortran = _read_npy_header(f, path, key)
+        row_bytes = dtype.itemsize * int(np.prod(shape[1:], dtype=np.int64))
+        streamable = not fortran and not dtype.hasobject and len(shape) >= 1 and shape[0] > 0 and row_bytes > 0
+        if streamable:
+            n = shape[0]
+            rows = block_rows or max(1, _BLOCK_BYTES // row_bytes)
+            for r0 in range(0, n, rows):
+                m = min(rows, n - r0)
+                data = f.read(m * row_bytes)
+                if len(data) != m * row_bytes:
+                    raise ValueError(f'{path}: member {key!r} ends after {r0 + len(data) // row_bytes} of the {n} rows '
+                                     'its header declares')
+                yield np.frombuffer(data, dtype).reshape(m, *shape[1:])
+    if not streamable:
+        with np.load(path) as z:
+            yield z[key]
+
+
+def _read_member(path, key) -> np.ndarray:
+    blocks = list(read_member_blocks(path, key))
+    return np.concatenate(blocks) if len(blocks) > 1 else blocks[0]
+
+
+def _terminal_rows(terminals, r0, r1):
+    """load_dataset's float32 `terminals` and `follows_terminal` (the next row's terminal, 1.0 after the file's last row)
+    at the file rows [r0, r1), with its own expressions: every element equals the one of the whole-file arrays."""
+    t = terminals[r0:r1].astype(np.float32)
+    follows = np.concatenate([terminals[r0 + 1:r1 + 1].astype(np.float32), [1.0] if r1 == len(terminals) else []])
+    return t, follows
+
+
+class _FileStream:
+    """`load_dataset(path, ...)` of one `.npz` file as row writes computed a block at a time.
+
+    `fields` is the result's layout, {name: (dtype, shape)} in load_dataset's key order, known from the members' headers
+    and the file's `terminals`, which is read whole (one byte per row in OGBench files).  `producers(block_rows)` gives one
+    generator per member (and one for the terminal fields); each yields (first row, {field: rows}) writes that together
+    cover every row of every field once.  Compact layout: rows stay where they are.  Regular layout: the kept rows of a
+    block go to `i - (terminals before i)`, and the same cast observation block, shifted by one row, gives the block's
+    `next_observations`.  With the compact layout `flags` holds one byte of `valids > 0` per row once the terminal
+    producer has run.
+    """
+
+    def __init__(self, path, ob_dtype=np.float32, action_dtype=np.float32, compact_dataset=False, add_info=False):
+        self.path, self.compact = str(path), compact_dataset
+        with zipfile.ZipFile(self.path) as zf:
+            present = set(zf.namelist())
+            keys = ['observations', 'actions', 'terminals'] + [k for k in _INFO_KEYS if add_info and f'{k}.npy' in present]
+            heads = {}
+            for k in keys:
+                with _open_member(zf, self.path, k) as f:
+                    heads[k] = _read_npy_header(f, self.path, k)
+        self.terminals = _read_member(self.path, 'terminals')
+        n = len(self.terminals)
+        for k, (shape, _, _) in heads.items():
+            if len(shape) < 1 or shape[0] != n:
+                raise ValueError(f'{self.path}: member {k!r} of shape {shape} does not have the {n} rows of terminals')
+        self.casts = {'observations': np.dtype(ob_dtype), 'actions': np.dtype(action_dtype)}
+        self.members = [k for k in keys if k != 'terminals']
+        obs_row = heads['observations'][0][1:]
+        if compact_dataset:
+            self.keep, rows, next_rows = None, n, None
+            self.flags = np.zeros(n, np.uint8)
+        else:
+            self.keep = (1.0 - self.terminals.astype(np.float32)).astype(bool)      # load_dataset's ob_mask
+            rows, next_rows = int(np.count_nonzero(self.keep)), int(np.count_nonzero(self.keep[:-1]))
+            self.flags = None
+        self.fields = {'observations': (self.casts['observations'], (rows, *obs_row)),
+                       'actions': (self.casts['actions'], (rows, *heads['actions'][0][1:])),
+                       'terminals': (np.dtype(np.float32), (rows,))}
+        self.fields.update({k: (heads[k][1], (rows, *heads[k][0][1:])) for k in keys[3:]})
+        if compact_dataset:
+            self.fields['valids'] = (np.dtype(np.float32), (rows,))
+        else:
+            self.fields['next_observations'] = (self.casts['observations'], (next_rows, *obs_row))
+
+    def producers(self, block_rows: Optional[int] = None):
+        return [self._member_writes(k, block_rows) for k in self.members] + [self._terminal_writes(block_rows)]
+
+    def _member_writes(self, key, block_rows):
+        cast = self.casts.get(key)
+        r0 = dest = 0
+        for block in read_member_blocks(self.path, key, block_rows):
+            r1 = r0 + len(block)
+            if cast is not None:
+                block = block.astype(cast, copy=False)
+            if self.compact:
+                yield r0, {key: block}
+            else:
+                keep = self.keep[r0:r1]
+                yield dest, {key: block[keep]}
+                if key == 'observations':
+                    # next_observations = observations[next_ob_mask], next_ob_mask[j] = ob_mask[j - 1] (False at j = 0)
+                    follows_kept = self.keep[max(r0 - 1, 0):r1 - 1]
+                    if r0 == 0:
+                        follows_kept = np.concatenate([[False], follows_kept])
+                    yield dest - int(r0 > 0 and self.keep[r0 - 1]), {'next_observations': block[follows_kept]}
+                dest += int(np.count_nonzero(keep))
+            r0 = r1
+
+    def _terminal_writes(self, block_rows):
+        n = len(self.terminals)
+        rows = block_rows or _BLOCK_BYTES // 32       # (float64 temporaries of load_dataset's expressions)
+        dest = 0
+        for r0 in range(0, n, rows):
+            r1 = min(n, r0 + rows)
+            t, follows = _terminal_rows(self.terminals, r0, r1)
+            if self.compact:
+                valids = 1.0 - t
+                self.flags[r0:r1] = valids > 0
+                yield r0, {'terminals': np.minimum(t + follows, 1.0).astype(np.float32), 'valids': valids}
+            else:
+                keep = self.keep[r0:r1]
+                yield dest, {'terminals': follows[keep].astype(np.float32)}
+                dest += int(np.count_nonzero(keep))
+
+    def write(self, nds: _NativeDataset, row0: int, names) -> None:
+        """Run the producers, one thread each, and write their rows from this thread to rows `row0 + r` of `nds`, whose
+        fields are `names` in order (ogb_dataset_write_rows is synchronous and takes one caller at a time)."""
+        _pump(self.producers(), lambda r, arrays: _write_rows(nds, names, row0 + r, arrays))
+
+
+def _write_rows(nds: _NativeDataset, names, row0: int, arrays) -> None:
+    """ogb_dataset_write_rows of `arrays` ({field: rows}, some of the table's fields `names`, in any order) at rows
+    [row0, row0 + n); the other fields are left as they are."""
+    n = len(next(iter(arrays.values())))
+    if n == 0:
+        return
+    arrays = {k: np.ascontiguousarray(a) for k, a in arrays.items()}
+    ptrs = (C.c_void_p * len(names))()
+    for i, k in enumerate(names):
+        if k in arrays:
+            ptrs[i] = arrays[k].ctypes.data
+    _native.check(_native.lib().ogb_dataset_write_rows(nds.ptr, row0, n, ptrs, len(names)))
+
+
+def _pump(producers, consume):
+    """Run each generator on a thread of its own and call consume(*item) for every item on this thread, in arrival order.
+    A bounded queue of two items per producer sits between them; an exception on either side stops every thread and is
+    raised here."""
+    q: queue.Queue = queue.Queue(maxsize=2 * len(producers))
+    stop = threading.Event()
+    done = object()
+
+    def put(item) -> bool:
+        while not stop.is_set():
+            try:
+                q.put(item, timeout=0.1)
+                return True
+            except queue.Full:
+                pass
+        return False
+
+    def work(gen):
+        try:
+            with contextlib.closing(gen):
+                for item in gen:
+                    if not put(item):
+                        return
+            put(done)
+        except BaseException as exc:  # raised on the consuming thread
+            put(exc)
+
+    threads = [threading.Thread(target=work, args=(g,), daemon=True) for g in producers]
+    for t in threads:
+        t.start()
+    try:
+        finished = 0
+        while finished < len(threads):
+            item = q.get()
+            if item is done:
+                finished += 1
+            elif isinstance(item, BaseException):
+                raise item
+            else:
+                consume(*item)
+    finally:
+        stop.set()
+        for t in threads:
+            t.join()
+
+
+def upload_dataset(dataset_path, ob_dtype=np.float32, action_dtype=np.float32, compact_dataset=False, add_info=False,
+                   device: int = 0) -> ResidentDataset:
+    """`Dataset.create(**load_dataset(dataset_path, ...))`, streamed: the file's members are inflated a block at a time, one
+    thread per member, cast and laid out per block, and written into HBM, so host memory holds a few blocks per member
+    and a few bytes per row instead of the whole file.  The dataset samples byte for byte what the host-loaded one does;
+    it keeps no host copy of its fields (ResidentDataset)."""
+    stream = _FileStream(dataset_path, ob_dtype, action_dtype, compact_dataset, add_info)
+    rows = {k: shape[0] for k, (_, shape) in stream.fields.items()}
+    if len(set(rows.values())) != 1:      # a regular layout whose last row is not terminal: Dataset.create refuses it too
+        raise ValueError(f'{dataset_path}: fields of different lengths {rows}')
+    nds = _NativeDataset.empty({k: _ZeroField(shape, dtype) for k, (dtype, shape) in stream.fields.items()}, device)
+    stream.write(nds, 0, list(stream.fields))
+    n = rows['terminals']
+    _native.check(_native.lib().ogb_dataset_seal(nds.ptr, n))
+    return ResidentDataset(nds, list(stream.fields), False, stream.flags)
 
 
 class ResidentShards:
@@ -313,10 +552,12 @@ class ResidentShards:
         shards[i], shards[path]   # Dataset of one shard: a view of the table, equal to Dataset.create(**load(path))
         shards.bounds             # [(row0, n_rows)] per shard
 
-    `load` is the per-file host loader (default: load_dataset(p, compact_dataset=True); `lambda p: make_datasets(name,
-    dataset_path=p)[0]` for '-oraclerep-' and 'singletask' names).  The capacity comes from the files' headers; then the
-    shards are loaded, written and freed one at a time, so host memory peaks at one shard plus a pinned staging buffer.
-    Every shard must load with shard 0's fields, dtypes and row shapes.
+    `load` is the per-file host loader.  By default each file is streamed into the table block by block as upload_dataset
+    does, with the result of load_dataset(p, compact_dataset=True), so host memory holds a few 8 MB blocks per member and
+    a few bytes per row.  A given `load` (`lambda p: make_datasets(name, dataset_path=p)[0]` for '-oraclerep-' and
+    'singletask' names, whose relabelling works on whole arrays) is called on one shard at a time, and each shard is
+    written and freed before the next is loaded, so host memory peaks at one shard plus a pinned staging buffer.  The
+    capacity comes from the files' headers.  Every shard must load with shard 0's fields, dtypes and row shapes.
 
     A view keeps the reference's shard-local semantics (goals, trajectory ends and next observations stay inside the
     shard) and a swap costs no upload; sampling `dataset` draws across every shard instead.  Shards end on trajectory
@@ -331,13 +572,15 @@ class ResidentShards:
             if nds is None:
                 keys, nested = shard.keys, shard.nested
                 nds = _NativeDataset.empty({k: _ZeroField((shard.capacity, *s), d) for k, (d, s) in shard.schema.items()}, device)
-            arrays = [np.ascontiguousarray(shard.fields[k]) for k in shard.schema]
-            ptrs = (C.c_void_p * len(arrays))(*[a.ctypes.data for a in arrays])
-            _native.check(lib.ogb_dataset_write_rows(nds.ptr, shard.row0, shard.n_rows, ptrs, len(arrays)))
-            if 'valids' in shard.fields:
-                valids.append((shard.fields['valids'] > 0).astype(np.uint8))
+            if shard.stream is not None:
+                shard.stream.write(nds, shard.row0, list(shard.schema))
+                valids.append(shard.stream.flags)
+            else:
+                _write_rows(nds, list(shard.schema), shard.row0, shard.fields)
+                if 'valids' in shard.fields:
+                    valids.append((shard.fields['valids'] > 0).astype(np.uint8))
             self.bounds.append((shard.row0, shard.n_rows))
-            del arrays, ptrs, shard                   # this shard's host arrays go before the next one is loaded
+            del shard                                 # this shard's host arrays go before the next one is loaded
         n_rows = sum(n for _, n in self.bounds)
         _native.check(lib.ogb_dataset_seal(nds.ptr, n_rows))
         flags = np.concatenate(valids) if valids else None
@@ -358,30 +601,38 @@ class ResidentShards:
 
 
 class _Shard:
-    __slots__ = ('path', 'row0', 'n_rows', 'capacity', 'keys', 'nested', 'schema', 'fields')
+    __slots__ = ('path', 'row0', 'n_rows', 'capacity', 'keys', 'nested', 'schema', 'fields', 'stream')
 
 
 def iter_shards(paths, load: Optional[Callable[[str], dict]] = None):
     """The host half of ResidentShards: load the shards one at a time, in order, and yield each as a record with its
     first row in the concatenation (`row0`), its row count, its flattened fields and the schema -- {name: (dtype, row
-    shape)} -- that shard 0 fixed; `capacity` is the rows the files' headers declare in all.  A shard whose fields, dtypes
-    or row shapes differ from shard 0's, or that loads more rows than its header declares, raises ValueError naming it."""
+    shape)} -- that shard 0 fixed; `capacity` is the rows the files' headers declare in all.  Without `load`, a record
+    holds no fields (`fields` is None) but the stream that writes load_dataset(path, compact_dataset=True) block by
+    block (`stream`, None when `load` is given).  A shard whose fields, dtypes or row shapes differ from shard 0's, or
+    that loads more rows than its header declares, raises ValueError naming it."""
     paths = [str(p) for p in paths]
     if not paths:
         raise ValueError('no shards given')
-    if load is None:
-        load = lambda p: load_dataset(p, compact_dataset=True)  # noqa: E731
     declared = [shard_rows(p) for p in paths]
     schema, row0 = None, 0
     for path, cap in zip(paths, declared):
-        tree = load(path)
-        fields = _flatten(tree)
-        shape = {k: (np.asarray(v).dtype, np.asarray(v).shape[1:]) for k, v in fields.items()}
+        if load is None:
+            stream, fields = _FileStream(path, compact_dataset=True), None
+            shape = {k: (d, s[1:]) for k, (d, s) in stream.fields.items()}
+            names, is_nested = list(stream.fields), False
+            lengths = {s[0] for _, s in stream.fields.values()}
+        else:
+            stream, tree = None, load(path)
+            fields = _flatten(tree)
+            shape = {k: (np.asarray(v).dtype, np.asarray(v).shape[1:]) for k, v in fields.items()}
+            names, is_nested = list(tree), any(isinstance(v, Mapping) for v in tree.values())
+            lengths = {len(v) for v in fields.values()}
+            del tree
         if schema is None:
-            schema, keys, nested = shape, list(tree), any(isinstance(v, Mapping) for v in tree.values())
+            schema, keys, nested = shape, names, is_nested
         elif shape != schema:
             raise ValueError(f'{path}: fields {_describe(shape)} differ from those of {paths[0]}: {_describe(schema)}')
-        lengths = {len(v) for v in fields.values()}
         if len(lengths) != 1:
             raise ValueError(f'{path}: fields of different lengths {sorted(lengths)}')
         n = lengths.pop()
@@ -389,8 +640,8 @@ def iter_shards(paths, load: Optional[Callable[[str], dict]] = None):
             raise ValueError(f'{path}: {n} rows loaded, the file declares {cap}')
         shard = _Shard()
         shard.path, shard.row0, shard.n_rows, shard.capacity = path, row0, n, sum(declared)
-        shard.keys, shard.nested, shard.schema, shard.fields = keys, nested, schema, fields
-        del tree, fields
+        shard.keys, shard.nested, shard.schema, shard.fields, shard.stream = keys, nested, schema, fields, stream
+        del fields, stream
         yield shard
         del shard                                     # (the caller's reference is the last one before the next load)
         row0 += n
