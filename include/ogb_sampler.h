@@ -153,9 +153,9 @@ int ogb_sampler_create(ogb_dataset* ds, const ogb_config* cfg, int32_t kind, uin
                        ogb_sampler** out);
 int ogb_sampler_set_stream(ogb_sampler* s, void* cuda_stream);    /* launch on the caller's stream instead */
 int ogb_sampler_set_debug(ogb_sampler* s, int32_t flags);         /* bit 0: keep the index vectors readable; bit 1: canary fill;
-                                                                     bit 2: warp-specialised fused kernel (index warps + queue);
                                                                      bit 3: row gathers walk their tiles with a fixed stride instead
-                                                                     of taking them from the ticket counter */
+                                                                     of taking them from the ticket counter; any other bit:
+                                                                     OGB_ERR_INVALID */
 int ogb_sampler_set_host_chunks(ogb_sampler* s, int32_t n_chunks); /* batches headed for host memory (ogb_batch_copy_to_host): issue
                                                                      big launches in up to n_chunks row chunks and copy each
                                                                      chunk out while the next is computed */

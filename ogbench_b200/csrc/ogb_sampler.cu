@@ -30,60 +30,28 @@ namespace {
 
 thread_local std::string g_error;
 
-// Measurement switches, read once from the environment.  None of them is needed in production: each forces one of the
-// alternatives DESIGN.md's "measured alternatives" table compares, so that the A/B can be repeated on a box with
-// scratch/ab.sh without rebuilding.  Results are identical under every setting: they choose between kernels the parity tests cover.
+// Switches read once from the environment.  None of them is needed in production: each forces, for every input, a path
+// that some real inputs take anyway, so that the tests can reach it with any dataset (test_gpu_rows.py runs each one in
+// a process of its own against the default's batches).  Results are identical under every setting.
 struct AbSwitches {
-  bool no_segments;      // OGB_NO_SEGMENTS     general bucketed searches instead of the segment table
   bool no_records;       // OGB_NO_RECORDS      one array per field instead of the packed record table
-  int record_align;      // OGB_RECORD_ALIGN=n  record stride rounded to n bytes instead of 128
-  int band_rows;         // OGB_BAND_ROWS=n     first band height tried by the frame kernel instead of 32
-  bool no_overlap;       // OGB_NO_OVERLAP      index kernel on the main stream, never under the previous gather
-  bool no_fuse;          // OGB_NO_FUSE         never fuse the index algebra into the gather kernel
   int fuse;              // OGB_FUSE=0|1        force the fused kernel off / on (-1: the built-in policy)
   bool gather_lsu;       // OGB_GATHER=lsu      register-staged gather kernel instead of the cp.async rings
   bool no_tiny_groups;   // OGB_NO_TINY_GROUPS  small fields copied one by one instead of grouped record loads
-  bool no_smem_tables;   // OGB_NO_SMEM_TABLES  index kernel never keeps the segment table in shared memory
-  bool smem_tables;      // OGB_SMEM_TABLES     ... and keeps it there on the main stream too
-  int stage_bytes;       // OGB_STAGE_BYTES=n   per-warp stage budget instead of 4096 / 6144
-  int ws;                // OGB_WS=0|1          warp-specialised fused kernel off / on (-1: ogb_sampler_set_debug decides)
   bool timeline;         // OGB_TIMELINE        record an event per phase for ogb_debug_timeline
-  int gather_shape;      // OGB_GATHER_SHAPE=SWW  stages * 100 + warps per CTA of the row-gather kernels (default: 220 for the fused GCDataset launch, 310 / 308 otherwise; also 208, 216, 316)
-  bool no_shadow;        // OGB_NO_SHADOW       no shadow copy of the next row's observation inside the records
-  int index_grid;        // OGB_INDEX_GRID=n    index kernel grid capped at n CTAs per SM instead of 16
-  bool no_point;         // OGB_NO_POINT        point-maze records go through the generic tiny-field walk of the index kernel
-  bool static_tiles;     // OGB_STATIC_TILES    row gathers walk their tiles with a fixed stride instead of taking tickets
-  bool no_wide_record;   // OGB_NO_WIDE_RECORD  point-maze kernel: two 128-bit loads of the record instead of one 256-bit load
-  int claim_pairs;       // OGB_CLAIM_PAIRS=n   a tile's ticket is taken n (tile, job) pairs before it is needed (default: 1 fused, 3 un-fused)
 };
 
 const AbSwitches& ab() {
   static const AbSwitches sw = [] {
     auto flag = [](const char* name) { return getenv(name) != nullptr; };
-    auto number = [](const char* name, int absent) { const char* v = getenv(name); return v ? atoi(v) : absent; };
     const char* gather = getenv("OGB_GATHER");
+    const char* fuse = getenv("OGB_FUSE");
     AbSwitches a;
-    a.no_segments = flag("OGB_NO_SEGMENTS");
     a.no_records = flag("OGB_NO_RECORDS");
-    a.record_align = number("OGB_RECORD_ALIGN", 0);
-    a.band_rows = number("OGB_BAND_ROWS", 0);
-    a.no_overlap = flag("OGB_NO_OVERLAP");
-    a.no_fuse = flag("OGB_NO_FUSE");
-    a.fuse = number("OGB_FUSE", -1);
+    a.fuse = fuse ? atoi(fuse) : -1;
     a.gather_lsu = gather != nullptr && strcmp(gather, "lsu") == 0;
     a.no_tiny_groups = flag("OGB_NO_TINY_GROUPS");
-    a.no_smem_tables = flag("OGB_NO_SMEM_TABLES");
-    a.smem_tables = flag("OGB_SMEM_TABLES");
-    a.stage_bytes = number("OGB_STAGE_BYTES", 0);
-    a.ws = number("OGB_WS", -1);
     a.timeline = flag("OGB_TIMELINE");
-    a.gather_shape = number("OGB_GATHER_SHAPE", 0);
-    a.no_shadow = flag("OGB_NO_SHADOW");
-    a.index_grid = number("OGB_INDEX_GRID", 0);
-    a.no_point = flag("OGB_NO_POINT");
-    a.static_tiles = flag("OGB_STATIC_TILES");
-    a.claim_pairs = number("OGB_CLAIM_PAIRS", 0);
-    a.no_wide_record = flag("OGB_NO_WIDE_RECORD");
     return a;
   }();
   return sw;
@@ -175,10 +143,9 @@ size_t rows_per_item(size_t pitch, size_t budget) {
 
 // Stage budget of a row-gather launch whose widest span is max_pitch bytes: 4 KB stages (2 CTAs per SM) for rows up to
 // 256 bytes, 6 KB (16-row items, 1 CTA per SM) beyond -- C3's 384/288-byte spans run 15 % faster with 16-row items than
-// with 8-row ones.  OGB_STAGE_BYTES overrides the default.
+// with 8-row ones.
 size_t stage_budget(size_t max_pitch) {
-  const int env = ab().stage_bytes;
-  return std::max<size_t>(env ? (size_t)env : (max_pitch > 256 ? 6144 : 4096), max_pitch);
+  return std::max<size_t>(max_pitch > 256 ? 6144 : 4096, max_pitch);
 }
 
 bool positive_at(const void* data, int dtype, int64_t i) {
@@ -498,8 +465,7 @@ struct ogb_sampler {
   bool debug = false;
   bool defer_index_check = false;        // host-output mode: given indices are range-checked by the kernel, the error
                                          // surfaces at ogb_batch_copy_to_host / ogb_batch_sync instead of at sample()
-  bool prefer_ws = false;                // debug bit 2: use the warp-specialised fused kernel
-  bool static_tiles = false;             // debug bit 3: row gathers walk their tiles with a fixed stride (no ticket counter)
+  bool static_tiles = false;             // debug bit 3: row gathers walk their tiles with a fixed stride (no tickets)
   bool canary = false;                   // debug: fill every batch block with 0xA5 first, so that tests can verify that
                                          // no kernel wrote outside the keys (ogb_batch_check_gaps)
   bool profile = false;                  // record timing events around the dominant kernel of every call
@@ -540,7 +506,7 @@ struct ogb_sampler {
   static constexpr int kSchedSlots = 64;
   uint32_t* d_sched = nullptr;
   uint32_t sched_seq = 0;
-  uint32_t* next_sched() { return d_sched ? d_sched + 32 * (size_t)(sched_seq++ % kSchedSlots) : nullptr; }
+  uint32_t* next_sched() { return d_sched + 32 * (size_t)(sched_seq++ % kSchedSlots); }
   std::vector<cudaEvent_t> chunk_events;       // ring of join events (index kernel -> gathers)
   int next_event = 0;
   std::mutex cache_mu;
@@ -823,7 +789,7 @@ void batch_unref(ogb_batch* b) {
 // general searches.
 int build_segment_table(ogb_sampler* s) {
   const ogb_dataset* ds = s->ds;
-  if (ds->valid_mode != 2 || ds->gaps_host.empty() || ab().no_segments) return 0;
+  if (ds->valid_mode != 2 || ds->gaps_host.empty()) return 0;
   const std::vector<int32_t>& c = ds->gaps_host;
   const size_t n_gaps = c.size();
   int64_t min_gap = ds->n_valid;
@@ -1044,7 +1010,7 @@ bool tma_eligible(const Field& f, const ogb_config& cfg, int fs) {
 }
 
 int band_rows_for(int64_t H, int pad) {
-  for (int rb = ab().band_rows > 0 ? ab().band_rows : 32; rb > pad; --rb)
+  for (int rb = 32; rb > pad; --rb)
     if (H % rb == 0) return rb;
   return 0;
 }
@@ -1178,9 +1144,8 @@ static int create_dataset(const ogb_field* fields, int32_t n_fields, int32_t dev
       // 32- and 64-byte records stay sector / granule sized; longer ones are padded to whole 128-byte L2 lines, so that a
       // goal row (a prefix of the record) never straddles a line (measured on the 156-byte C2 record: stride 256 is
       // 8 % faster than 160 or 192 and 3 % faster than separate arrays)
-      const int env_align = ab().record_align;
       ds->record_used = cursor;
-      ds->record_stride = cursor <= 32 ? 32 : cursor <= 64 ? 64 : round_up(cursor, env_align >= 32 ? (size_t)env_align : 128);
+      ds->record_stride = cursor <= 32 ? 32 : cursor <= 64 ? 64 : round_up(cursor, 128);
       const size_t bytes = (size_t)size * ds->record_stride;
       cudaError_t e = cudaMalloc((void**)&ds->record_base, bytes);
       if (e == cudaSuccess) e = cudaMemset(ds->record_base, 0, bytes);
@@ -1234,7 +1199,7 @@ static int create_dataset(const ogb_field* fields, int32_t n_fields, int32_t dev
   ds->obs_field = ds->find_under("observations");
   for (size_t i = 0; i < ds->n_public; ++i)
     if ((int)i != ds->obs_field && ogb_dataset::under(ds->fields[i].name, "observations")) ds->obs_extra.push_back((int)i);
-  if (ds->obs_field >= 0 && ds->obs_extra.empty() && ds->find_under("next_observations") < 0 && !ab().no_shadow) {
+  if (ds->obs_field >= 0 && ds->obs_extra.empty() && ds->find_under("next_observations") < 0) {
     const Field obs = ds->fields[(size_t)ds->obs_field];
     size_t a = 16;
     while (obs.row_bytes % a != 0) a >>= 1;
@@ -1507,11 +1472,10 @@ int ogb_sampler_create(ogb_dataset* ds, const ogb_config* cfg, int32_t kind, uin
   s->n_slots = kind == OGB_KIND_GC ? (cfg->trl ? ogb::GC_TRL_NUM_SLOTS : ogb::GC_NUM_SLOTS) : (kind == OGB_KIND_HGC ? ogb::HGC_NUM_SLOTS : 2);
   s->plan[0] = build_plan(s, false);
   s->plan[1] = build_plan(s, true);
-  if (!ab().static_tiles) {   // ticket counters of the row gathers, zeroed once: every launch leaves its pair at zero
-    if (cudaMalloc((void**)&s->d_sched, (size_t)ogb_sampler::kSchedSlots * 128) != cudaSuccess ||
-        cudaMemset(s->d_sched, 0, (size_t)ogb_sampler::kSchedSlots * 128) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess)
-      return bail(fail(OGB_ERR_CUDA, "ticket counters: %s", cudaGetErrorString(cudaGetLastError())));
-  }
+  // ticket counters of the row gathers, zeroed once: every launch leaves its pair at zero
+  if (cudaMalloc((void**)&s->d_sched, (size_t)ogb_sampler::kSchedSlots * 128) != cudaSuccess ||
+      cudaMemset(s->d_sched, 0, (size_t)ogb_sampler::kSchedSlots * 128) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess)
+    return bail(fail(OGB_ERR_CUDA, "ticket counters: %s", cudaGetErrorString(cudaGetLastError())));
   *out = s;
   return 0;
 } OGB_CATCH_ALL
@@ -1546,9 +1510,9 @@ int ogb_sampler_set_profile(ogb_sampler* s, int32_t on) try {
 } OGB_CATCH_ALL
 int ogb_sampler_set_debug(ogb_sampler* s, int32_t keep) try {
   if (!s) return fail(OGB_ERR_INVALID, "null sampler");
+  if (keep & ~11) return fail(OGB_ERR_INVALID, "debug flags 0x%x: only bits 0, 1 and 3 are defined", (unsigned)keep);
   s->debug = (keep & 1) != 0;
   s->canary = (keep & 2) != 0;
-  s->prefer_ws = (keep & 4) != 0;
   s->static_tiles = (keep & 8) != 0;
   return 0;
 } OGB_CATCH_ALL
@@ -1945,7 +1909,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   // Phase-one work (uploads of validation draws, the index kernel) goes to `first`: for big launches that is the
   // auxiliary stream, so that the index kernel of this call overlaps the gathers of the previous call, which are
   // still running on the main stream.  The recycled block only has to wait for its own previous owner.
-  const bool no_overlap = ab().no_overlap, no_fuse = ab().no_fuse, gather_lsu = ab().gather_lsu;
+  const bool gather_lsu = ab().gather_lsu;
   auto takes_async_path = [&](const Field& f) {
     return f.row_bytes > 16 && f.stride <= (size_t)ogb::kAsyncMaxStride && (size_t)ds->size * f.stride < ((size_t)1 << 36) &&
            !gather_lsu;
@@ -1958,7 +1922,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   // previous call's frame gathers).  OGB_FUSE=0/1 forces either.
   const int fuse_env = ab().fuse;
   bool fuse = false;
-  if (!no_fuse && (fuse_env >= 0 ? fuse_env != 0 : (!any_frames && (total < kOverlapMinRows || spec.kind != OGB_KIND_HGC))))
+  if (fuse_env >= 0 ? fuse_env != 0 : (!any_frames && (total < kOverlapMinRows || spec.kind != OGB_KIND_HGC)))
     for (const KeyPlan& k : plan)
       if (k.route == ROUTE_ROW && k.alias_of < 0 && takes_async_path(ds->fields[(size_t)k.field])) fuse = true;
   // Image batches are few rows with long gathers: their (latency-bound) index kernel always goes to the auxiliary
@@ -1966,7 +1930,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   bool any_gather = any_frames;            // is there a gather launch for the index kernel to hide under?
   for (const KeyPlan& k : plan)
     if (k.route == ROUTE_ROW && k.alias_of < 0 && ds->fields[(size_t)k.field].row_bytes > 16) any_gather = true;
-  const bool use_aux = !fuse && !no_overlap && any_gather && (total >= kOverlapMinRows || any_frames);
+  const bool use_aux = !fuse && any_gather && (total >= kOverlapMinRows || any_frames);
   if (use_aux) {
     int rc = ensure_aux(s);
     if (rc) return bail(rc);
@@ -2262,7 +2226,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   // nothing else to gather.  The index kernel then runs with these copies compiled in.
   // (the kernel also compiles out what such a launch cannot need: index vectors in memory -- no later kernel, debug off --,
   // frame-stack rows, the SLOT_NEXT row, the TRL branch, and every valid-row form but the segment table)
-  bool point_record = !ab().no_point && spec.kind == OGB_KIND_GC && !spec.trl && !any_async && lsu_keys.empty() && !any_frames &&
+  bool point_record = spec.kind == OGB_KIND_GC && !spec.trl && !any_async && lsu_keys.empty() && !any_frames &&
                       !s->debug && p.valid_mode == 3 && p.vec_init == nullptr &&
                       p.n_tiny_groups == 1 && p.n_tiny_fields == 5 && p.n_tiny == 2 && p.n_tiny_fast == 2 &&
                       p.tiny_groups[0].slot == SLOT_IDX && p.tiny_groups[0].n_vec == 2 &&
@@ -2280,7 +2244,6 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
   typedef std::function<int(int64_t, int64_t, cudaStream_t)> LaunchFn;
   std::vector<LaunchFn> gather_launches;
   LaunchFn fused_launch;
-  const char* fused_name = "relabel_gather_kernel";
   bool fused_writes_vecs = false;
 
   LaunchFn index_launch = [&, p](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
@@ -2290,13 +2253,11 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     const int flavour = p.kind == OGB_KIND_GC ? FLAVOUR_GC : (p.kind == OGB_KIND_HGC ? FLAVOUR_HGC : FLAVOUR_PLAIN);
     const bool inject = draws != nullptr;
     // Big launches over a dataset whose segment table is small: persistent CTAs keep the table in shared memory.
-    const bool no_smem_tables = ab().no_smem_tables;
     const size_t table_bytes = (size_t)p.n_seg_table * 16 + (size_t)p.n_seg_bucket * 4;
     // Used when the index kernel runs on the auxiliary stream under another call's gather: the persistent form with few
     // CTAs disturbs the gather less (C3 0.716 vs 0.730 ms); alone on its stream the plain grid is faster (C1 0.047 vs 0.049).
-    const bool force_smem_tables = ab().smem_tables;
-    const bool smem_tables = !no_smem_tables && (st != s->stream || force_smem_tables) && p.valid_mode == 3 && table_bytes > 0 &&
-                             table_bytes <= 48 * 1024 && end - begin >= 65536;
+    const bool smem_tables = st != s->stream && p.valid_mode == 3 && table_bytes > 0 && table_bytes <= 48 * 1024 &&
+                             end - begin >= 65536;
     const void* fn = nullptr;
 #define OGB_PICK_INDEX_KERNEL(INJ, SM)                                                                                  \
     fn = flavour == FLAVOUR_GC ? (const void*)relabel_index_kernel<INJ, FLAVOUR_GC, SM>                                   \
@@ -2313,7 +2274,6 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     if (point_record && smem_tables && !inject) fn = (const void*)relabel_index_kernel<false, FLAVOUR_GC, true, true, 5>;
     b->name_index = kernel_name("relabel_index_kernel", {inject ? 1 : 0, flavour, smem_tables ? 1 : 0, point_record && !(smem_tables && inject) ? 1 : 0,
                                                         point_record && !inject ? 5 : 4});
-    p.wide_record = ab().no_wide_record ? 0 : 1;   // +1.2 % on C1 at 16M rows per launch (0.740 vs 0.731, batch r2l)
     // Grid cap: a whole number of waves of resident CTAs (a 16-per-SM grid of the five-per-SM point-maze kernel is 3.2
     // waves, and the last, fifth-full wave cost C1 5 %: 0.731 vs 0.771-0.775 of peak for 5, 10 or 32 per SM, batch r2l).
     static std::mutex occ_mu;
@@ -2329,7 +2289,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
       }
       resident_index = it->second;
     }
-    int64_t grid_cap = (int64_t)ds->sm_count * (ab().index_grid > 0 ? ab().index_grid : 2 * resident_index);
+    int64_t grid_cap = (int64_t)ds->sm_count * 2 * resident_index;
     size_t smem = 0;
     if (smem_tables) {
       smem = table_bytes;
@@ -2378,8 +2338,8 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     size_t stage = 0;
     for (size_t t = q0; t < q1; ++t) stage = std::max(stage, rows_for(span_jobs[t].bytes) * span_jobs[t].bytes);
     ap.stage_bytes = (int)round_up(stage, 128);
-    // (stages, warps per CTA): 3 x 8 built in (two CTAs per SM); the alternatives are compiled for the GCDataset fused
-    // launch and the un-fused gather only (OGB_GATHER_SHAPE=SWW overrides, measurement switch).
+    // (stages, warps per CTA): 3 x 8 (two CTAs per SM), except for the fused GCDataset launch (2 x 20, or 2 x 16 when
+    // 20 warps' rings do not fit) and the un-fused gather with stages over 4 KB (3 x 10).
     // Measured on B200 (profiles/r2_ab_shapes.txt).  Fused GCDataset launch: ONE CTA of 20 warps with two stages per warp
     // (160 KB of shared memory with 4 KB stages) -- 2 x 16 had beaten 3 x 8 x 2 CTAs by 4 % (C2) / 2 % (C5) with static
     // tiles; with ticket-scheduled tiles and ~1 ms launches 2 x 20 is another 4 % ahead on C2 (0.945-0.961 vs 0.908-0.927
@@ -2387,15 +2347,11 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     // 4-13 % (uneven warps per scheduler, and a register cap that makes the index algebra spill; 24 warps with the index
     // algebra out of line, to keep the loops under the 80-register cap, lost 25 %).  Un-fused gather: three
     // stages; with 6 KB stages (rows > 256 B: C3) ten warps in one CTA, 0.979 vs 0.964 for eight (twelve: 0.968).
-    int shape = ab().gather_shape;
-    const bool fused_gc = fuse && q0 == 0 && p.kind == OGB_KIND_GC && draws == nullptr;
-    const bool known = shape == 308 || shape == 208 || shape == 216 || shape == 316 || shape == 220 || shape == 310;
-    if (!known) {
-      if (fused_gc) shape = (size_t)20 * 2 * ap.stage_bytes <= (size_t)200 * 1024 ? 220 : 216;
-      else shape = (!(fuse && q0 == 0) && ap.stage_bytes > 4096 && (size_t)10 * 3 * ap.stage_bytes <= (size_t)200 * 1024) ? 310 : 308;
-    }
-    if (shape == 310 && fuse && q0 == 0) shape = 308;   // (un-fused only)
-    if (shape != 308 && fuse && q0 == 0 && !fused_gc) shape = 308;
+    const bool fused_here = fuse && q0 == 0;
+    const bool fused_gc = fused_here && p.kind == OGB_KIND_GC && draws == nullptr;
+    int shape = 308;
+    if (fused_gc) shape = (size_t)20 * 2 * ap.stage_bytes <= (size_t)200 * 1024 ? 220 : 216;
+    else if (!fused_here && ap.stage_bytes > 4096 && (size_t)10 * 3 * ap.stage_bytes <= (size_t)200 * 1024) shape = 310;
     const int n_stages = shape / 100, n_warps = shape % 100;
     ap.ring_bytes = n_stages * ap.stage_bytes;
     for (; q < q1; ++q) {
@@ -2457,22 +2413,22 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     // (C3 0.952 / 0.956 / 0.960 / 0.963 for 1 / 2 / 3 / all), while C5b's shape prefers <= 3 (1.021 vs 1.011) -> three.
     std::vector<int> pair_first;
     for (int k = 0; k < ap.n_items; ++k) if (ap.items[k].flags & 1u) pair_first.push_back(k);
-    const bool fused_here = fuse && q0 == 0;
-    const bool dyn_tiles = s->d_sched != nullptr && !s->static_tiles && (fused_here || pair_first.size() >= 2);
+    const bool dyn_tiles = !s->static_tiles && (fused_here || pair_first.size() >= 2);
     {
       // index (into pair_first) of the pair at whose first item the tile is needed; the fused kernel needs it one pair "later"
       const int need = (int)pair_first.size() - (fused_here ? 0 : 1);
-      const int ahead = ab().claim_pairs > 0 ? ab().claim_pairs : (fused_here ? 1 : 3);
+      const int ahead = fused_here ? 1 : 3;
       ap.claim_item = pair_first[(size_t)std::max(0, need - ahead)];
     }
     // shared memory: item table, output table, one 16-byte tile FIFO per warp, then the rings
     ap.ring_offset = (int)round_up((size_t)ap.n_items * sizeof(ItemDesc) + (size_t)ap.n_outs * sizeof(OutDesc) + (size_t)n_warps * 16, 128);
     const size_t smem = (size_t)ap.ring_offset + (size_t)n_warps * ap.ring_bytes;
-    if (smem > (size_t)225 * 1024) return bail(fail(OGB_ERR_UNSUPPORTED, "gather shape %d needs %zu bytes of shared memory", shape, smem));
+    if (smem > (size_t)225 * 1024)
+      return bail(fail(OGB_ERR_UNSUPPORTED, "internal: gather shape %d needs %zu bytes of shared memory", shape, smem));
     // persistent grid: exactly the CTAs that are resident at once (shared memory bounds them here; the fused kernels are
     // compiled for gather_min_blocks(warps) CTAs per SM, so registers allow at least that many)
     const int ctas_per_sm = (int)std::max<size_t>(1, std::min<size_t>(n_warps <= 8 ? 2 : 1, (size_t)(220 * 1024) / smem));
-    if (fuse && q0 == 0) {
+    if (fused_here) {
       // index algebra + the first (normally the only) group of row jobs in ONE launch; the launches that take the
       // remaining jobs read the index vectors this one computes
       if (q1 < span_jobs.size()) p.write_vecs = 1;
@@ -2483,17 +2439,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
       std::shared_ptr<FusedParams> keep(fp);
       const int flavour = p.kind == OGB_KIND_GC ? FLAVOUR_GC : (p.kind == OGB_KIND_HGC ? FLAVOUR_HGC : FLAVOUR_PLAIN);
       const bool inject = draws != nullptr;
-      // large launches: the warp-specialised form (index warps feed the gather warps through a shared-memory queue)
-      // Measured on B200: equal to the same-warp fusion on C2 (0.200 vs 0.203 ms) and slower on C5 (0.371 vs 0.361 ms) --
-      // the index algebra costs the SM the same whichever warp runs it -- so it is off unless asked for
-      // (OGB_WS=1 or ogb_sampler_set_debug bit 2).
-      const int ws_env = ab().ws;
-      const int n_slots_fl = flavour == FLAVOUR_GC ? GC_TRL_NUM_SLOTS : (flavour == FLAVOUR_HGC ? HGC_NUM_SLOTS : 2);
-      const size_t ws_smem = smem + (size_t)kAsyncWarps * ((size_t)kQueueDepth * n_slots_fl * 128 + 16 * kQueueDepth);
-      const bool ws = (ws_env >= 0 ? ws_env != 0 : s->prefer_ws) && ws_smem <= 113 * 1024 && shape == 308;
-      fused_name = ws ? "relabel_gather_ws_kernel" : "relabel_gather_kernel";
-      b->name_fused = ws ? kernel_name("relabel_gather_ws_kernel", {inject ? 1 : 0, flavour})
-                         : kernel_name("relabel_gather_kernel", {inject ? 1 : 0, flavour, n_stages, n_warps});
+      b->name_fused = kernel_name("relabel_gather_kernel", {inject ? 1 : 0, flavour, n_stages, n_warps});
       fused_launch = [=](int64_t begin, int64_t end, cudaStream_t st) -> int {
         FusedParams& f = *keep;
         f.relabel.row_begin = f.gather.row_begin = begin;
@@ -2501,38 +2447,27 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         const int64_t n_warp_tiles = (end - begin + 31) / 32;
         const unsigned grid = (unsigned)std::min<int64_t>((n_warp_tiles + n_warps - 1) / n_warps, (int64_t)ds->sm_count * ctas_per_sm);
         // (tickets only when there are more tiles than warps: a small launch gives every warp at most its first tile)
-        f.gather.sched = dyn_tiles && !ws && n_warp_tiles > (int64_t)grid * n_warps ? s->next_sched() : nullptr;
-        const void* fn = nullptr;
-#define OGB_PICK_FUSED(KERNEL, INJ)                                                      \
-        fn = flavour == FLAVOUR_GC ? (const void*)KERNEL<INJ, FLAVOUR_GC>                   \
-           : flavour == FLAVOUR_HGC ? (const void*)KERNEL<INJ, FLAVOUR_HGC>                 \
-                                    : (const void*)KERNEL<INJ, FLAVOUR_PLAIN>
-        if (ws && inject) { OGB_PICK_FUSED(relabel_gather_ws_kernel, true); }
-        else if (ws) { OGB_PICK_FUSED(relabel_gather_ws_kernel, false); }
-        else if (inject) { OGB_PICK_FUSED(relabel_gather_kernel, true); }
-        else { OGB_PICK_FUSED(relabel_gather_kernel, false); }
-#undef OGB_PICK_FUSED
-        if (shape == 208) fn = (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 8>;
-        else if (shape == 216) fn = (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 16>;
-        else if (shape == 316) fn = (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 3, 16>;
-        else if (shape == 220) fn = (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 20>;
-        const size_t smem_bytes = ws ? ws_smem : smem;
-        const unsigned threads = ws ? (kAsyncWarps + kIndexWarps) * 32 : (unsigned)n_warps * 32;
-        if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes) != cudaSuccess)
+        f.gather.sched = dyn_tiles && n_warp_tiles > (int64_t)grid * n_warps ? s->next_sched() : nullptr;
+        // (2 x 20 and 2 x 16 are compiled for the fused GCDataset launch with Philox draws only: fused_gc)
+        const void* fn = shape == 220 ? (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 20>
+                       : shape == 216 ? (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 16>
+                       : flavour == FLAVOUR_GC ? (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_GC>
+                                                         : (const void*)relabel_gather_kernel<false, FLAVOUR_GC>)
+                       : flavour == FLAVOUR_HGC ? (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_HGC>
+                                                          : (const void*)relabel_gather_kernel<false, FLAVOUR_HGC>)
+                                                : (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_PLAIN>
+                                                          : (const void*)relabel_gather_kernel<false, FLAVOUR_PLAIN>);
+        if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
           return fail(OGB_ERR_CUDA, "cudaFuncSetAttribute(relabel_gather_kernel) failed");
         void* args[] = {(void*)&f};
-        if (cudaLaunchKernel(fn, dim3(grid), dim3(threads), args, smem_bytes, st) != cudaSuccess)
+        if (cudaLaunchKernel(fn, dim3(grid), dim3((unsigned)n_warps * 32), args, smem, st) != cudaSuccess)
           return fail(OGB_ERR_CUDA, "relabel_gather_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         b->launches++;
         return 0;
       };
       continue;
     }
-    const void* gather_fn = shape == 208 ? (const void*)gather_rows_async_kernel<2, 8>
-                          : shape == 216 ? (const void*)gather_rows_async_kernel<2, 16>
-                          : shape == 316 ? (const void*)gather_rows_async_kernel<3, 16>
-                          : shape == 220 ? (const void*)gather_rows_async_kernel<2, 20>
-                          : shape == 310 ? (const void*)gather_rows_async_kernel<3, 10>
+    const void* gather_fn = shape == 310 ? (const void*)gather_rows_async_kernel<3, 10>
                                          : (const void*)gather_rows_async_kernel<kAsyncStages, kAsyncWarps>;
     OGB_CUDA(cudaFuncSetAttribute(gather_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (b->name_async.empty()) b->name_async = kernel_name("gather_rows_async_kernel", {n_stages, n_warps});
@@ -2706,7 +2641,7 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     phase.mark();   // prepare
     // dominant kernel = the one that moves the batch's bytes: the frame gather, else the row gather (fused or not),
     // else the index kernel itself (datasets whose rows are all <= 16 bytes)
-    b->dominant = any_frames ? (any_frames_tma ? "gather_frames_tma_kernel" : "gather_frames_generic_kernel") : fused_launch ? fused_name
+    b->dominant = any_frames ? (any_frames_tma ? "gather_frames_tma_kernel" : "gather_frames_generic_kernel") : fused_launch ? "relabel_gather_kernel"
                 : any_async ? "gather_rows_async_kernel" : !lsu_keys.empty() ? "gather_rows_kernel" : "relabel_index_kernel";
     // row chunks (multiples of 32 rows, each at least kChunkMinRows): one unless the batch is headed for host memory
     constexpr int64_t kChunkMinRows = 16384;
@@ -3115,7 +3050,7 @@ int ogb_batch_dominant_kernel(ogb_batch* b, const char** name, float* ms) try {
   {
     const std::string d = b->dominant;
     const std::string& full = d == "gather_frames_tma_kernel" ? b->name_frames
-                            : (d == "relabel_gather_kernel" || d == "relabel_gather_ws_kernel") ? b->name_fused
+                            : d == "relabel_gather_kernel" ? b->name_fused
                             : d == "gather_rows_async_kernel" ? b->name_async : d == "relabel_index_kernel" ? b->name_index : d;
     b->dominant_full = full.empty() ? d : full;
   }

@@ -6,8 +6,7 @@
 // scalar keys (masks, rewards, offsets, steps), copies the fields whose rows are <= 16 bytes, and leaves the dataset
 // row of every index-vector slot in registers.  It runs inside
 //   relabel_index_kernel      stand-alone (rows go to int32 index vectors in memory for the gather kernels),
-//   relabel_gather_kernel     fused with the row gather: sample() is one launch,
-//   relabel_gather_ws_kernel  the same launch, warp-specialised (optional).
+//   relabel_gather_kernel     fused with the row gather: sample() is one launch.
 //
 // gather_rows_async_body gathers the dataset rows those slots name (datasets.py:78-83 get_subset, :341-357
 // get_observations / get_goal_observations) into the dense output arrays: per-warp cp.async rings, span jobs over the
@@ -175,7 +174,6 @@ struct RelabelParams {
   int32_t n_tiny;              // the first n_tiny_fast of them have rows of 4, 8 or 16 bytes
   int32_t n_tiny_fast;
   int32_t write_vecs;          // 0: no later kernel needs the index vectors (everything was tiny) and debug is off
-  int32_t wide_record;         // kPoint: fetch the 32-byte record with one 256-bit load (default; OGB_NO_WIDE_RECORD: two 128-bit loads)
   TinyJob tiny[kMaxTinyJobs];
   int32_t n_tiny_groups;
   int32_t n_tiny_fields;
@@ -369,14 +367,14 @@ __device__ __forceinline__ void relabel_row(const RelabelParams& p, const SegVie
     if (kPoint ? u == 0 : (u < p.n_tiny_groups && p.tiny_groups[u].slot == SLOT_IDX)) {
       const TinyGroup& grp = p.tiny_groups[u];
       const uint4* sp = reinterpret_cast<const uint4*>(grp.src + (size_t)(uint32_t)i * grp.stride);
-      if (kPoint && p.wide_record) {
+      if (kPoint) {   // the 32-byte record in one 256-bit load: +1.2 % on C1 over two 128-bit loads (0.740 vs 0.731, batch r2l)
         asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                      : "=r"(grp_a[u].x), "=r"(grp_a[u].y), "=r"(grp_a[u].z), "=r"(grp_a[u].w), "=r"(grp_b[u].x), "=r"(grp_b[u].y),
                        "=r"(grp_b[u].z), "=r"(grp_b[u].w)
                      : "l"(sp));
       } else {
         grp_a[u] = __ldg(sp);
-        if (kPoint || grp.n_vec > 1) grp_b[u] = __ldg(sp + 1);
+        if (grp.n_vec > 1) grp_b[u] = __ldg(sp + 1);
       }
     }
   }
@@ -821,15 +819,9 @@ __device__ __forceinline__ uint4 lds128(uint32_t addr) {
 }
 
 // Output rows are written once and read by another kernel much later: store them with the streaming (evict-first)
-// policy so that they do not push dataset rows out of L2 (OGB_PLAIN_STORES at build time restores plain stores).
+// policy so that they do not push dataset rows out of L2 (+2 % on C3 over plain stores).
 // (The converse hint -- loading the rows with an L2 evict-last policy -- was measured as well: no effect on C2/C3/C5.)
-__device__ __forceinline__ void store_out(uint4* p, const uint4 v) {
-#ifdef OGB_PLAIN_STORES
-  *p = v;
-#else
-  __stcs(p, v);
-#endif
-}
+__device__ __forceinline__ void store_out(uint4* p, const uint4 v) { __stcs(p, v); }
 
 // generic element drain (rows whose size is not a multiple of 4 bytes): flat element index, coalesced stores
 template <typename V>
@@ -887,35 +879,6 @@ struct TileCursor {
 // then a single launch.
 // (A TMA variant -- one cp.async.bulk per source row instead of 16-byte LDGSTS chunks -- was measured and dropped:
 // equal on 224/288-byte rows, 17 % slower on 128-byte rows.)
-// Warp-specialised form (MODE_QUEUE): kIndexWarps extra warps per CTA run relabel_row for the tiles of the gather warps
-// and hand the rows of every slot over through a small shared-memory queue (kQueueDepth tiles per gather warp, one
-// full/empty mbarrier pair per queue slot), so the L2 lookup latency of the index algebra is taken by warps that hold
-// no cp.async ring and the gather warps never stop issuing.
-constexpr int kIndexWarps = 3;
-constexpr int kQueueDepth = 2;
-enum : int { MODE_VECTORS = 0, MODE_FUSED = 1, MODE_QUEUE = 2 };
-
-struct QueueView {          // shared-memory addresses of one gather warp's queue
-  uint32_t rows;            // int32 [kQueueDepth][kSlots][32]
-  uint32_t full;            // uint64 mbarrier [kQueueDepth]
-  uint32_t empty;           // uint64 mbarrier [kQueueDepth]
-};
-
-__device__ __forceinline__ void queue_mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void queue_mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void queue_mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "QUEUE_WAIT_LOOP:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra.uni QUEUE_WAIT_DONE;\n\t"
-      "bra.uni QUEUE_WAIT_LOOP;\n\t"
-      "QUEUE_WAIT_DONE:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
 __device__ __forceinline__ void sts32(uint32_t addr, int32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
 
 // every CTA copies the launch's item / output tables from the constant bank into shared memory once
@@ -928,9 +891,8 @@ __device__ __forceinline__ void stage_tables(const AsyncGatherParams& p, uint8_t
   for (int i = threadIdx.x; i < n_out_vecs; i += blockDim.x) outs_s[i] = reinterpret_cast<const uint4*>(p.outs)[i];
 }
 
-template <int kMode, bool kInject, int kFlavour, int kStages = kAsyncStages, int kWarps = kAsyncWarps>
-__device__ __forceinline__ void gather_rows_async_body(const AsyncGatherParams& p, const RelabelParams& rp, uint8_t* smem_dyn,
-                                                       const QueueView qv) {
+template <bool kFused, bool kInject, int kFlavour, int kStages = kAsyncStages, int kWarps = kAsyncWarps>
+__device__ __forceinline__ void gather_rows_async_body(const AsyncGatherParams& p, const RelabelParams& rp, uint8_t* smem_dyn) {
   constexpr int kSlots = FlavourSlots<kFlavour>::value;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int32_t n_warps_global = (int32_t)gridDim.x * kWarps;
@@ -951,7 +913,7 @@ __device__ __forceinline__ void gather_rows_async_body(const AsyncGatherParams& 
   // those pairs' issue loops.  The tail cursor drains the same tile sequence a few items
   // later: the warp keeps its claimed tiles in a four-entry FIFO in shared memory (the head is at most kStages - 1 tile
   // boundaries ahead of the tail, plus the tile it has resolved but not entered).
-  const bool dyn = kMode != MODE_QUEUE && p.sched != nullptr;
+  const bool dyn = p.sched != nullptr;
   const int32_t dyn_base = (int32_t)(p.row_begin >> 5) + n_warps_global;            // ticket t names tile dyn_base + t
   const uint32_t fifo_u32 = (uint32_t)__cvta_generic_to_shared(smem_dyn) + (uint32_t)p.ring_offset - 16u * (uint32_t)(kWarps - warp);
   uint32_t ticket = 0;                   // lane 0: the ticket in flight
@@ -997,27 +959,15 @@ __device__ __forceinline__ void gather_rows_async_body(const AsyncGatherParams& 
     return __ldg(p.vec_rows + (int64_t)slot * p.total_rows + ((int64_t)tile << 5) + min(lane, n - 1));
   };
   int32_t pref_rows = 0;
-  if (kMode == MODE_VECTORS) pref_rows = load_rows(first_tile, items_s[1].w);
-  uint32_t queue_k = 0;                  // MODE_QUEUE: ordinal of the next tile this warp takes from its queue
+  if (!kFused) pref_rows = load_rows(first_tile, items_s[1].w);
   auto issue = [&](const TileCursor& c, const uint32_t stage_u32) {
     if (c.tile < n_tiles) {
       const uint4* it = items_s + c.k * (int)(sizeof(ItemDesc) / 16);
       const uint4 d0 = it[0], d1 = it[1], d2 = it[2];
       if (dyn && c.k == p.claim_item && lane == 0) ticket = atomicAdd(p.sched, 1u);
       if (d2.z & 1u) {                                           // entering the next (tile, job) pair
-        if (kMode == MODE_FUSED) {
+        if (kFused) {
           if (c.k == 0 && lane < c.n) relabel_row<kInject, kFlavour>(rp, SegView{rp.seg_bucket, rp.seg_table}, ((int64_t)c.tile << 5) + lane, sr);
-          issue_rows = pick_slot<kSlots>(sr, (int)d1.w);
-        } else if (kMode == MODE_QUEUE) {
-          if (c.k == 0) {                                        // take this tile's rows from the index warps
-            const uint32_t qs = queue_k % kQueueDepth;
-            queue_mbar_wait(qv.full + 8u * qs, (queue_k / kQueueDepth) & 1u);
-#pragma unroll
-            for (int v = 0; v < kSlots; ++v) sr[v] = (int32_t)lds32(qv.rows + ((qs * kSlots + (uint32_t)v) * 32u + (uint32_t)lane) * 4u);
-            __syncwarp();
-            if (lane == 0) queue_mbar_arrive(qv.empty + 8u * qs);
-            ++queue_k;
-          }
           issue_rows = pick_slot<kSlots>(sr, (int)d1.w);
         } else {
           issue_rows = pref_rows;
@@ -1131,7 +1081,7 @@ __global__ void __launch_bounds__(kWarps * 32, gather_min_blocks(kWarps)) gather
   extern __shared__ __align__(128) uint8_t smem_dyn[];
   stage_tables(p, smem_dyn);
   __syncthreads();
-  gather_rows_async_body<MODE_VECTORS, false, FLAVOUR_PLAIN, kStages, kWarps>(p, *reinterpret_cast<const RelabelParams*>(&p), smem_dyn, QueueView{0, 0, 0});
+  gather_rows_async_body<false, false, FLAVOUR_PLAIN, kStages, kWarps>(p, *reinterpret_cast<const RelabelParams*>(&p), smem_dyn);
   sched_release(p.sched);
 }
 
@@ -1146,63 +1096,8 @@ __global__ void __launch_bounds__(kWarps * 32, gather_min_blocks(kWarps)) relabe
   extern __shared__ __align__(128) uint8_t smem_dyn[];
   stage_tables(p.gather, smem_dyn);
   __syncthreads();
-  gather_rows_async_body<MODE_FUSED, kInject, kFlavour, kStages, kWarps>(p.gather, p.relabel, smem_dyn, QueueView{0, 0, 0});
+  gather_rows_async_body<true, kInject, kFlavour, kStages, kWarps>(p.gather, p.relabel, smem_dyn);
   sched_release(p.gather.sched);
-}
-
-// sample() in one launch, warp-specialised: warps [0, kAsyncWarps) gather, warps [kAsyncWarps, +kIndexWarps) run the
-// index algebra ahead of them.  Dynamic shared memory: the tables, the rings, then the row queues, then the mbarriers.
-template <bool kInject, int kFlavour>
-__global__ void __launch_bounds__((kAsyncWarps + kIndexWarps) * 32) relabel_gather_ws_kernel(const __grid_constant__ FusedParams p) {
-  constexpr int kSlots = FlavourSlots<kFlavour>::value;
-  extern __shared__ __align__(128) uint8_t smem_dyn[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  stage_tables(p.gather, smem_dyn);
-  const uint32_t rings_end = (uint32_t)p.gather.ring_offset + (uint32_t)kAsyncWarps * (uint32_t)p.gather.ring_bytes;
-  const uint32_t queue_u32 = (uint32_t)__cvta_generic_to_shared(smem_dyn) + rings_end;
-  constexpr uint32_t kQueueBytesPerWarp = kQueueDepth * kSlots * 32 * 4;
-  const uint32_t bars_u32 = queue_u32 + (uint32_t)kAsyncWarps * kQueueBytesPerWarp;
-  auto view_of = [&](int w) { return QueueView{queue_u32 + (uint32_t)w * kQueueBytesPerWarp, bars_u32 + (uint32_t)w * (16u * kQueueDepth),
-                                               bars_u32 + (uint32_t)w * (16u * kQueueDepth) + 8u * kQueueDepth}; };
-  if (threadIdx.x < kAsyncWarps * kQueueDepth * 2) queue_mbar_init(bars_u32 + 8u * threadIdx.x, 1);
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  __syncthreads();
-
-  if (warp < kAsyncWarps) {
-    gather_rows_async_body<MODE_QUEUE, kInject, kFlavour>(p.gather, p.relabel, smem_dyn, view_of(warp));
-    return;
-  }
-  // ---- index warps ----
-  const RelabelParams& rp = p.relabel;
-  const int ix = warp - kAsyncWarps;
-  const int32_t n_warps_global = (int32_t)gridDim.x * kAsyncWarps;
-  const int32_t n_warp_tiles = (int32_t)((p.gather.row_end + 31) >> 5);
-  const int32_t last_n = (int32_t)(p.gather.row_end - ((int64_t)(n_warp_tiles - 1) << 5));
-  const int32_t tile0 = (int32_t)(p.gather.row_begin >> 5) + (int32_t)blockIdx.x * kAsyncWarps;
-  const SegView seg{rp.seg_bucket, rp.seg_table};
-#pragma unroll 1
-  for (uint32_t k = 0;; ++k) {
-    bool any = false;
-#pragma unroll 1
-    for (int w = ix; w < kAsyncWarps; w += kIndexWarps) {
-      const int64_t tile = (int64_t)tile0 + w + (int64_t)k * n_warps_global;
-      if (tile >= n_warp_tiles) continue;
-      any = true;
-      const QueueView qv = view_of(w);
-      const uint32_t qs = k % kQueueDepth;
-      queue_mbar_wait(qv.empty + 8u * qs, ((k / kQueueDepth) & 1u) ^ 1u);     // first round: passes at once
-      const int n = tile == n_warp_tiles - 1 ? last_n : 32;
-      int32_t sr[kMaxSlots];
-#pragma unroll
-      for (int v = 0; v < kMaxSlots; ++v) sr[v] = 0;
-      if (lane < n) relabel_row<kInject, kFlavour>(rp, seg, (tile << 5) + lane, sr);
-#pragma unroll
-      for (int v = 0; v < kSlots; ++v) sts32(qv.rows + ((qs * kSlots + (uint32_t)v) * 32u + (uint32_t)lane) * 4u, sr[v]);
-      __syncwarp();
-      if (lane == 0) queue_mbar_arrive(qv.full + 8u * qs);
-    }
-    if (!any) break;
-  }
 }
 
 }  // namespace ogb

@@ -681,8 +681,8 @@ class _Sampler:
         _native.check(_native.lib().ogb_sampler_set_stream(self.ptr, C.c_void_p(cuda_stream)))
 
     def set_debug(self, on=True):
-        """bit 0 (True / 1): keep the index vectors readable; bit 1 (2): canary-fill every batch block first; bit 2 (4): the
-        warp-specialised fused kernel; bit 3 (8): statically strided tiles in the row gathers instead of ticket scheduling."""
+        """bit 0 (True / 1): keep the index vectors readable; bit 1 (2): canary-fill every batch block first; bit 3 (8):
+        statically strided tiles in the row gathers instead of ticket scheduling.  Any other bit raises ValueError."""
         _native.check(_native.lib().ogb_sampler_set_debug(self.ptr, int(on)))
 
     @property

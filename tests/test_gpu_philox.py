@@ -88,20 +88,21 @@ def test_philox_mode_is_the_oracle_on_philox_draws(case):
             assert np.array_equal(got[k][ok], want[k][ok]), (k, call)
 
 
-def test_warp_specialised_kernel_equals_default():
-    """The optional warp-specialised fused kernel (index warps feeding gather warps through a shared-memory queue with
-    mbarriers) must produce the very same batches as the default kernels, small and large launches, ragged tail."""
-    lengths = ragged(21, 300, 30, 200)
-    fields = toy_fields(21, lengths, (29,), 8, np.float32)
-    config = cfg()
-    a = device_sampler(fields, config, 'gc', seed=5)
-    b = device_sampler(fields, config, 'gc', seed=5)
-    b._sampler.set_debug(4)
-    for K, B in ((1, 1000), (40, 1024), (3, 77)):
-        x, y = to_host(a.sample_many(K, B)), to_host(b.sample_many(K, B))
-        assert set(x) == set(y)
-        for k in x:
-            assert np.array_equal(x[k], y[k]), (k, K, B)
+def test_undefined_debug_bits_are_refused():
+    """ogb_sampler_set_debug defines bits 0, 1 and 3; any other bit (bit 2 selected a kernel that no longer exists) is
+    refused with OGB_ERR_INVALID (ValueError) instead of being ignored, and the sampler keeps sampling."""
+    fields = toy_fields(21, ragged(21, 30, 5, 60), (29,), 8, np.float32)
+    a = device_sampler(fields, cfg(), 'gc', seed=5)
+    b = device_sampler(fields, cfg(), 'gc', seed=5)
+    b._sampler.set_debug(1 | 2 | 8)
+    for bad in (4, 4 | 8, 16, -1):
+        with pytest.raises(ValueError, match='debug flags'):
+            b._sampler.set_debug(bad)
+    b._sampler.set_debug(0)
+    x, y = to_host(a.sample(100)), to_host(b.sample(100))
+    assert set(x) == set(y)
+    for k in x:
+        assert np.array_equal(x[k], y[k]), k
 
 
 def torch_from(x):

@@ -65,8 +65,8 @@ def rows_per_item(pitch, budget):
     return r
 
 
-def stage_budget(max_pitch, env):
-    return max(int(env.get('OGB_STAGE_BYTES', 0)) or (6144 if max_pitch > 256 else 4096), max_pitch)
+def stage_budget(max_pitch):
+    return max(6144 if max_pitch > 256 else 4096, max_pitch)
 
 
 def under(name, prefix):
@@ -220,9 +220,9 @@ class RowPlan:
         n = self.fl[0].n
         takes_async = lambda f: f.row > 16 and f.stride <= ASYNC_MAX_STRIDE and n * f.stride < 1 << 36 and not lsu_env
         rows = [k for k in self.keys if not k.alias]
-        # fused: vector keys on the cp.async path, and not a big HGC launch (OGB_NO_FUSE / OGB_FUSE override)
+        # fused: vector keys on the cp.async path, and not a big HGC launch (OGB_FUSE=0|1 overrides)
         fuse_env = env.get('OGB_FUSE')
-        fuse = ('OGB_NO_FUSE' not in env and (fuse_env == '1' if fuse_env is not None else (total < OVERLAP_MIN_ROWS or kind != 'hgc'))
+        fuse = ((fuse_env == '1' if fuse_env is not None else (total < OVERLAP_MIN_ROWS or kind != 'hgc'))
                 and any(takes_async(k.field) for k in rows))
         self.n_tiny, self.n_tiny_groups, self.n_tiny_fields = 0, 0, 0
         spans, self.lsu = [], []
@@ -255,7 +255,7 @@ class RowPlan:
                     if fn.rec_off > hi + 32:
                         break
                     pitch = round_up(max(hi, fn.rec_off + fn.row) - lo, 16)
-                    if 32 // rows_per_item(pitch, stage_budget(pitch, env)) * (k1 - k0 + 1) > MAX_ITEM_OUTS:
+                    if 32 // rows_per_item(pitch, stage_budget(pitch)) * (k1 - k0 + 1) > MAX_ITEM_OUTS:
                         break
                     hi, has_long, k1 = max(hi, fn.rec_off + fn.row), has_long or fn.row > 16, k1 + 1
                 if has_long:
@@ -291,7 +291,7 @@ class RowPlan:
             q1 = min(len(spans), q + MAX_ROW_JOBS)
             reason = 'jobs' if q1 < len(spans) else None
             while True:
-                budget = stage_budget(max(s.bytes for s in spans[q:q1]), env)
+                budget = stage_budget(max(s.bytes for s in spans[q:q1]))
                 items = sum(32 // rows_per_item(s.bytes, budget) for s in spans[q:q1])
                 outs = sum(32 // rows_per_item(s.bytes, budget) * len(s.outs) for s in spans[q:q1])
                 if (items <= MAX_ITEMS and outs <= MAX_ITEM_OUTS) or q1 == q + 1:
@@ -313,7 +313,7 @@ class RowPlan:
                     for k, soff in s.outs:
                         self.drains.add(self.drain(k.field.row, soff, s.bytes, sub))
             self.launches.append(dict(first=q, items=items, outs=outs, stage=stage,
-                                      shape=self.shape(env, kind, q == 0 and self.fused, philox, stage)))
+                                      shape=self.shape(kind, q == 0 and self.fused, philox, stage)))
             q = q1
         # register-staged keys: one launch per element width and 24 keys
         self.lsu_vecs = [vec_log2(k.field.row, k.field.stride) for k in self.lsu]
@@ -331,19 +331,11 @@ class RowPlan:
             return WORDS if sub * row % 16 == 0 else WORDS_UNALIGNED
         return ELEMS_U16 if row % 2 == 0 and soff % 2 == 0 else ELEMS_U8
 
-    def shape(self, env, kind, fused_here, philox, stage):
-        shape = int(env.get('OGB_GATHER_SHAPE', 0))
-        fused_gc = fused_here and kind in ('gc', 'trl') and philox
-        if shape not in (308, 208, 216, 316, 220, 310):
-            if fused_gc:
-                shape = 220 if 20 * 2 * stage <= 200 * 1024 else 216
-            else:
-                shape = 310 if not fused_here and stage > 4096 and 10 * 3 * stage <= 200 * 1024 else 308
-        if shape == 310 and fused_here:
-            shape = 308
-        if shape != 308 and fused_here and not fused_gc:
-            shape = 308
-        return shape
+    @staticmethod
+    def shape(kind, fused_here, philox, stage):
+        if fused_here and kind in ('gc', 'trl') and philox:
+            return 220 if 20 * 2 * stage <= 200 * 1024 else 216
+        return 310 if not fused_here and stage > 4096 and 10 * 3 * stage <= 200 * 1024 else 308
 
     def smem(self, launch):
         """Shared memory of one row-gather launch: item and output tables, a tile FIFO per warp, the rings."""
@@ -623,11 +615,6 @@ def test_split_fused_launches_against_the_oracle(case):
         if philox:
             handle = philox_leg(case, fields, debug)
             check_path(handle, plan_of(case, case_total(case)), case['name'])
-        # the warp-specialised fused kernel needs the 3 x 8 shape with <= 4 KB stages: not these launches
-        sampler = sampler_for(case, fields, seed=2)
-        sampler._sampler.set_debug(4)
-        _, kernel = batch_info(sampler._sampler.sample_native(case['B']))
-        assert not kernel.startswith('relabel_gather_ws_kernel'), kernel
 
 
 @pytest.mark.gpu
@@ -686,10 +673,9 @@ def test_eight_leaf_pytree_samples():
     assert to_host(sampler.sample(7))['actions'].shape == (7, 4)
 
 
-# ------------------------------------------------ measurement switches ------------------------------------------------
-SWITCHES = [{'OGB_GATHER': 'lsu'}, {'OGB_NO_RECORDS': '1'}, {'OGB_NO_FUSE': '1'}, {'OGB_FUSE': '1'}, {'OGB_NO_TINY_GROUPS': '1'},
-            {'OGB_STATIC_TILES': '1'}, {'OGB_GATHER_SHAPE': '208'}, {'OGB_GATHER_SHAPE': '216'}, {'OGB_GATHER_SHAPE': '316'},
-            {'OGB_GATHER_SHAPE': '310'}, {'OGB_STAGE_BYTES': '8192'}]
+# ------------------------------------------------ switches ------------------------------------------------
+# each forces, for every input, a path that some real inputs take anyway
+SWITCHES = [{'OGB_GATHER': 'lsu'}, {'OGB_NO_RECORDS': '1'}, {'OGB_FUSE': '0'}, {'OGB_FUSE': '1'}, {'OGB_NO_TINY_GROUPS': '1'}]
 # one split GC case, one C3-like HGC case (384-byte spans, un-fused at >= 32,768 rows), one LSU case
 SWITCH_CASES = [SPLIT_CASES[0], C_('c3-like', 'hgc', ((96,), F32), 51, B=1024, K=33, traj=(300, 20, 300)), BIG_CASES[5]]
 
@@ -724,26 +710,19 @@ def run_switch(env):
 
 @pytest.mark.gpu
 def test_measurement_switches_give_identical_batches():
-    """Every measurement switch (read once per process, so one process each) returns the default process's batches byte
-    for byte, or -- a gather shape whose shared memory does not fit -- refuses with NotImplementedError, after which the
-    process keeps sampling the other cases."""
+    """Every switch (read once per process, so one process each) returns the default process's batches byte for byte,
+    with the launch count the restated planner predicts for it."""
     default = run_switch({})
     for case in SWITCH_CASES:
         assert 'refused' not in default[case['name']], default[case['name']]
-    refusals = 0
     for env in SWITCHES:
         got = run_switch(env)
         for case in SWITCH_CASES:
             plan = plan_of(case, case_total(case), env=env)
             name = case['name']
-            if plan.refused_smem:
-                assert 'shared memory' in got[name].get('refused', ''), (env, name, got[name])
-                refusals += 1
-                continue
             assert 'refused' not in got[name], (env, name, got[name])
             assert got[name]['launches'] == plan.n_launches, (env, name, got[name]['launches'], plan.n_launches)
             assert got[name]['keys'] == default[name]['keys'], (env, name)
-    assert refusals >= 1
 
 
 # ------------------------------------------------ no GPU ------------------------------------------------
@@ -771,6 +750,9 @@ def test_case_plan_reaches_every_path():
     assert plans['split-jobs'].split_reasons == {'jobs'}
     assert not plans['big-hgc-unfused'].fused and not plans['big-hgc-unfused-nodedup'].fused and plans['hgc-fused'].fused
     assert plans['big-gc-fused/philox'].launches[0]['shape'] == 220 and plans['split-items-gc/philox'].launches[0]['shape'] == 220
+    # every compiled gather shape is planned by some case: 2 x 16 for a fused GCDataset launch of 6 KB stages, 3 x 10 for an
+    # un-fused gather of 6 KB stages
+    assert {la['shape'] for p in plans.values() for la in p.launches} == {220, 216, 308, 310}
     # tiny observations drained inside the span of the transition's record
     for name in ('obs1-u8', 'obs6-u8', 'obs12-f32'):
         p = plans[name]
@@ -782,8 +764,12 @@ def test_case_plan_reaches_every_path():
     assert {k.field.row for k in plans['lsu'].lsu} == {4097, 4098, 4100, 4104, 4112}
     # the eight-leaf pytree: no observation span holds all eight leaves any more
     assert all(len(s.outs) < 8 for s in plans['pytree-8x100'].spans if s.slot != SLOT_IDX)
-    # the switch matrix: every switch launches or is refused for its shared memory, and at least one is refused
-    refused = [(tuple(env.items()), c['name']) for env in SWITCHES for c in SWITCH_CASES if plan_of(c, case_total(c), env=env).refused_smem]
-    assert refused and all(dict(e).get('OGB_GATHER_SHAPE') == '316' for e, _ in refused), refused
+    # no case, by default or under any switch, plans a launch over the shared-memory limit (that refusal is internal)
+    refused = [name for name, p in plans.items() if p.refused_smem]
+    for c in ALL_CASES + SWITCH_CASES:
+        fields, config = make_fields(c), make_config(c)
+        refused += [(c['name'], tuple(env.items())) for env in SWITCHES
+                    if RowPlan(fields, c['kind'], config, case_total(c), c.get('dedup', True), env).refused_smem]
+    assert not refused, refused
     assert time.time() - t0 < 10
 
