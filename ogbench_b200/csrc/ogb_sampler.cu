@@ -545,9 +545,8 @@ struct ogb_batch {
   std::vector<cudaEvent_t> chunk_done;                     // ... are complete once chunk_done[c] has fired
   int32_t* idx_error = nullptr;                            // device flag of the deferred index check (inside the block)
   cudaEvent_t prof_begin = nullptr, prof_end = nullptr;   // profile mode: brackets of the dominant kernel
-  const char* dominant = "";                               // its name ...
-  std::string dominant_full;                               // ... with the template arguments ncu prints, e.g. "relabel_gather_kernel<0, 0, 2, 20>"
-  std::string name_fused, name_async, name_frames, name_index;   // (as chosen by the launches of this batch)
+  const char* dominant = "";                               // its name, with the template arguments ncu prints, e.g.
+                                                           // "relabel_gather_kernel<0, 0, 2, 20>" (static storage)
   cudaEvent_t ready = nullptr;
   cudaEvent_t copied = nullptr;                            // ogb_batch_copy_to_host_begin: the D2H copy of the block has finished
   volatile int32_t* h_idx_flag = nullptr;                  // ... and where the deferred index flag lands (pinned, sampler-owned)
@@ -612,6 +611,21 @@ int ensure_aux(ogb_sampler* s) {
   s->chunk_events.resize(1 + kMaxChunks + 1);
   for (auto& ev : s->chunk_events) OGB_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
   return 0;
+}
+
+// Orders `to` behind the work issued so far on `from`, through the next event of the sampler's join ring.
+int join_streams(ogb_sampler* s, cudaStream_t from, cudaStream_t to) {
+  cudaEvent_t ev = s->chunk_events[s->next_event];
+  s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
+  OGB_CUDA(cudaEventRecord(ev, from));
+  OGB_CUDA(cudaStreamWaitEvent(to, ev, 0));
+  return 0;
+}
+
+// Rows a start index is drawn from: those of `table` (TRL rows, ATC anchors) when there is one, else the valid rows
+// (every row that holds data when the dataset has no 'valids').
+int64_t n_choices_for(const ogb_dataset* ds, const int32_t* table, int64_t table_rows) {
+  return table ? table_rows : (ds->valid_mode == 0 ? ds->active_rows : ds->n_valid);
 }
 
 void block_give(ogb_sampler* s, uint8_t* block, size_t bytes, std::vector<cudaEvent_t>&& free_after) {
@@ -1032,14 +1046,6 @@ int get_tmap(ogb_sampler* s, int field, int band_rows, CUtensorMap* out) {
   if (r != CUDA_SUCCESS) return fail(OGB_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
   s->tmaps[{field, band_rows}] = tm;
   *out = tm;
-  return 0;
-}
-
-template <int FS>
-int launch_frames_tma(const CUtensorMap& tm, const ogb::FramesParams& fp, int64_t n_items, size_t smem, cudaStream_t st) {
-  OGB_CUDA(cudaFuncSetAttribute(ogb::gather_frames_tma_kernel<FS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  ogb::gather_frames_tma_kernel<FS><<<(unsigned)n_items, ogb::kFramesThreads, smem, st>>>(tm, fp);
-  OGB_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -1518,8 +1524,7 @@ int ogb_sampler_set_debug(ogb_sampler* s, int32_t keep) try {
 } OGB_CATCH_ALL
 int ogb_sampler_num_choices(const ogb_sampler* s, int64_t* out) try {
   if (!s || !out) return fail(OGB_ERR_INVALID, "null argument");
-  if (s->trl_rows.dev) *out = (int64_t)s->trl_rows.host.size();
-  else *out = s->ds->valid_mode == 0 ? s->ds->active_rows : s->ds->n_valid;
+  *out = n_choices_for(s->ds, s->trl_rows.dev, (int64_t)s->trl_rows.host.size());
   return 0;
 } OGB_CATCH_ALL
 
@@ -1534,12 +1539,8 @@ int ogb_sampler_write_row(ogb_sampler* s, int64_t row, const void* const* field_
   DeviceGuard device_guard(ds->device);
   OGB_CUDA(device_guard.status);
   std::lock_guard<std::mutex> lock(s->mu);
-  if (s->aux_stream) {  // index kernels of big launches read tiny fields on the auxiliary stream
-    cudaEvent_t ev = s->chunk_events[s->next_event];
-    s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
-    OGB_CUDA(cudaEventRecord(ev, s->aux_stream));
-    OGB_CUDA(cudaStreamWaitEvent(s->stream, ev, 0));
-  }
+  // index kernels of big launches read tiny fields on the auxiliary stream
+  if (s->aux_stream) OGB_TRY(join_streams(s, s->aux_stream, s->stream));
   for (size_t i = 0; i < ds->n_public; ++i) {
     if (!field_rows[i]) continue;
     const Field& f = ds->fields[i];
@@ -1622,12 +1623,8 @@ int ogb_sampler_write_ring(ogb_sampler* s, int64_t row0, int64_t n, int64_t skip
   };
   const uint64_t ticket = ++s->ring_ticket;
   if (rows > 0) {
-    if (s->aux_stream) {  // index kernels of big launches read tiny fields on the auxiliary stream
-      cudaEvent_t ev = s->chunk_events[s->next_event];
-      s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
-      OGB_CUDA(cudaEventRecord(ev, s->aux_stream));
-      OGB_CUDA(cudaStreamWaitEvent(s->stream, ev, 0));
-    }
+    // index kernels of big launches read tiny fields on the auxiliary stream
+    if (s->aux_stream) OGB_TRY(join_streams(s, s->aux_stream, s->stream));
     if (any_device && producer_stream && producer_stream != (void*)s->stream) {
       cudaEvent_t ev;
       OGB_TRY(take_event(&ev));
@@ -1771,6 +1768,68 @@ std::string kernel_name(const char* base, std::initializer_list<int> args) {
   return out + ">";
 }
 
+// A kernel and the name ogb_batch_dominant_kernel reports for it (the one ncu prints, which bench.py looks up in
+// profiles/traffic.json), both taken from the same template arguments.
+struct KernelChoice {
+  const void* fn;
+  const char* name;
+  int resident = 0;   // index kernels: CTAs resident per SM without dynamic shared memory (4 if the query fails)
+};
+
+template <bool kInject, int kFlavour, bool kSmemTables, bool kPoint = false, int kMinBlocks = 4>
+KernelChoice index_instance() {
+  static const std::string name = kernel_name("relabel_index_kernel", {kInject, kFlavour, kSmemTables, kPoint, kMinBlocks});
+  const void* fn = (const void*)ogb::relabel_index_kernel<kInject, kFlavour, kSmemTables, kPoint, kMinBlocks>;
+  static const int resident = [fn] {
+    int n = 0;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, fn, ogb::kRelabelThreads, 0) == cudaSuccess && n >= 1 ? n : 4;
+  }();
+  return {fn, name.c_str(), resident};
+}
+template <int kFlavour>
+KernelChoice index_flavour(bool inject, bool smem_tables) {
+  return inject ? (smem_tables ? index_instance<true, kFlavour, true>() : index_instance<true, kFlavour, false>())
+                : (smem_tables ? index_instance<false, kFlavour, true>() : index_instance<false, kFlavour, false>());
+}
+// relabel_index_kernel for injected or Philox draws, the flavour, the segment table in shared memory or not, and the
+// point-maze record (always a GCDataset launch)
+KernelChoice choose_index_kernel(bool inject, int flavour, bool smem_tables, bool point_record) {
+  using namespace ogb;
+  // 48 registers, five CTAs per SM: 0.556 vs 0.541 of peak with four (six spill: 0.541), profiles/r2_ab_shapes.txt
+  if (point_record && !inject)
+    return smem_tables ? index_instance<false, FLAVOUR_GC, true, true, 5>() : index_instance<false, FLAVOUR_GC, false, true, 5>();
+  if (point_record && !smem_tables) return index_instance<true, FLAVOUR_GC, false, true>();
+  return flavour == FLAVOUR_GC ? index_flavour<FLAVOUR_GC>(inject, smem_tables)
+       : flavour == FLAVOUR_HGC ? index_flavour<FLAVOUR_HGC>(inject, smem_tables) : index_flavour<FLAVOUR_PLAIN>(inject, smem_tables);
+}
+
+template <bool kInject, int kFlavour, int kStages = ogb::kAsyncStages, int kWarps = ogb::kAsyncWarps>
+KernelChoice fused_instance() {
+  static const std::string name = kernel_name("relabel_gather_kernel", {kInject, kFlavour, kStages, kWarps});
+  return {(const void*)ogb::relabel_gather_kernel<kInject, kFlavour, kStages, kWarps>, name.c_str()};
+}
+// relabel_gather_kernel in a shape of split_span_jobs (2 x 20 and 2 x 16 are compiled for the fused GCDataset launch with
+// Philox draws only)
+KernelChoice choose_fused_kernel(bool inject, int flavour, int shape) {
+  using namespace ogb;
+  if (shape == 220 || shape == 216) return shape == 220 ? fused_instance<false, FLAVOUR_GC, 2, 20>() : fused_instance<false, FLAVOUR_GC, 2, 16>();
+  if (flavour == FLAVOUR_GC) return inject ? fused_instance<true, FLAVOUR_GC>() : fused_instance<false, FLAVOUR_GC>();
+  if (flavour == FLAVOUR_HGC) return inject ? fused_instance<true, FLAVOUR_HGC>() : fused_instance<false, FLAVOUR_HGC>();
+  return inject ? fused_instance<true, FLAVOUR_PLAIN>() : fused_instance<false, FLAVOUR_PLAIN>();
+}
+
+template <int kStages, int kWarps>
+KernelChoice async_instance() {
+  static const std::string name = kernel_name("gather_rows_async_kernel", {kStages, kWarps});
+  return {(const void*)ogb::gather_rows_async_kernel<kStages, kWarps>, name.c_str()};
+}
+
+template <int FS>
+KernelChoice frames_instance() {
+  static const std::string name = kernel_name("gather_frames_tma_kernel", {FS});
+  return {(const void*)ogb::gather_frames_tma_kernel<FS>, name.c_str()};
+}
+
 // OGB_HOST_PHASES=1 (measurement switch): host time of run_sample by phase, summed over all calls, printed at exit.
 struct HostPhases {
   static constexpr int kN = 7;
@@ -1798,526 +1857,212 @@ struct PhaseClock {
   }
 };
 
-int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t n_batches, const int64_t* idxs, int32_t evaluation,
-               const ogb_draws* draws, ogb_batch** out) {
-  using namespace ogb;
-  PhaseClock phase;
-  if (!s || !out) return fail(OGB_ERR_INVALID, "ogb_sampler_sample: null argument");
-  if (batch_size < 0 || n_batches < 1) return fail(OGB_ERR_INVALID, "batch_size must be >= 0 and n_batches >= 1");
-  if (draws && n_batches != 1) return fail(OGB_ERR_INVALID, "validation draws need n_batches == 1");
+// The start-row tables of `p`: `table` (TRL rows, ATC anchors) when there is one, else the dataset's valid rows --
+// through the sampler's one-probe segment table when it has one --, and the trajectory tables.
+void set_row_tables(const ogb_sampler* s, const int32_t* table, int64_t n_choices, ogb::RelabelParams* p) {
   const ogb_dataset* ds = s->ds;
-  const ogb_config& cfg = s->cfg;
-  const int64_t total = batch_size * (int64_t)n_batches;
-  if (total > (int64_t)1 << 31) return fail(OGB_ERR_UNSUPPORTED, "more than 2^31 rows in one launch");
-  const bool stacked_next = (cfg.frame_stack > 0 && spec.kind != OGB_KIND_PLAIN) || spec.kind == OGB_KIND_ATC;
-  const int64_t idx_last = (stacked_next ? ds->size - spec.next_offset : ds->size) - 1;
-  const bool defer_check = idxs && s->defer_index_check;
-  if (idxs && !defer_check) {  // numpy fancy indexing would raise IndexError (negative wrap-around is not supported here)
-    // branch-free scan (vectorises): idx < 0 or idx > last sets the sign bit of idx | (last - idx)
-    const int64_t last = idx_last;
-    int64_t bad = 0;
-    for (int64_t r = 0; r < total; ++r) bad |= idxs[r] | (last - idxs[r]);
-    if (bad < 0)
-      for (int64_t r = 0; r < total; ++r)
-        if (idxs[r] < 0 || idxs[r] > last)
-          return fail(OGB_ERR_INDEX, "index %lld is out of bounds for axis 0 with size %lld", (long long)idxs[r], (long long)ds->size);
+  p->term = s->d_term;
+  p->term_bucket = s->d_term_bucket;
+  p->term_shift = s->term_shift;
+  p->valid_table = table ? table : ds->d_valid_table;
+  p->gap_c = ds->d_gap_c;
+  p->gap_bucket = ds->d_gap_bucket;
+  p->gap_shift = ds->gap_shift;
+  p->valid_mode = table ? 1 : ds->valid_mode;
+  if (!table && s->seg_shift >= 0) {
+    p->valid_mode = 3;
+    p->seg_table = s->d_seg_table;
+    p->seg_bucket = s->d_seg_bucket;
+    p->seg_shift = s->seg_shift;
+    p->n_seg_table = s->n_seg_table;
+    p->n_seg_bucket = s->n_seg_bucket;
   }
-  if (idxs && spec.trl) {
-    // datasets.py:255-256: `assert (idxs != final_state_idxs).all()` -- a given index that is a trajectory's final state
-    // (a terminal row) has no midpoint span, and its idx + 1 belongs to the next trajectory (or lies past the table)
-    for (int64_t r = 0; r < total; ++r)
-      if (idxs[r] >= 0 && idxs[r] < ds->size && !ds->terminals_host.empty() && ds->terminals_host[(size_t)idxs[r]])
-        return fail(OGB_ERR_ASSERT, "assert (idxs != final_state_idxs).all() (datasets.py:256): index %lld is a final state", (long long)idxs[r]);
-  }
-  const int64_t n_choices = spec.n_choices >= 0 ? spec.n_choices : (ds->valid_mode == 0 ? ds->active_rows : ds->n_valid);
-  if (n_choices < 1) return fail(OGB_ERR_INVALID, "nothing to sample from: the dataset holds no rows yet");
-  const bool forced_crop = spec.crop_padding >= 0;
-  const bool aug_mode = forced_crop || (cfg.has_p_aug && !evaluation && spec.kind != OGB_KIND_PLAIN);
-  const double p_aug_eff = forced_crop ? 1.0 : cfg.p_aug;
-  const int crop_pad_eff = forced_crop ? spec.crop_padding : cfg.crop_padding;
-  const int n_goal_sets = (spec.kind == OGB_KIND_GC || spec.kind == OGB_KIND_HGC) ? 3 : 0;
-  const bool geom[3] = {cfg.value_geom_sample != 0, true, cfg.actor_geom_sample != 0};
-  const bool cur_only[3] = {cfg.value_p_curgoal == 1.0, cfg.value_p_curgoal == 1.0, cfg.actor_p_curgoal == 1.0};
-  const bool goal_used[3] = {true, spec.kind == OGB_KIND_HGC && cfg.has_low_discount, true};
-  if (draws) {
-    if (!idxs && !draws->idx_pos) return fail(OGB_ERR_INVALID, "validation mode needs idx_pos or idxs");
-    for (int gs = 0; gs < n_goal_sets; ++gs) {
-      if (!goal_used[gs]) continue;
-      const ogb_goal_draws& d = draws->goals[gs];
-      if (!d.rand_pos || (geom[gs] ? !d.offset : !d.dist) || (!cur_only[gs] && (!d.u_traj || !d.u_cur)))
-        return fail(OGB_ERR_INVALID, "validation mode: goal set %d is missing draws", gs);
-      for (int64_t r = 0; r < batch_size; ++r)
-        if (d.rand_pos[r] < 0 || d.rand_pos[r] >= n_choices) return fail(OGB_ERR_INDEX, "rand_pos out of range");
-    }
-    if (draws->idx_pos && !idxs)
-      for (int64_t r = 0; r < batch_size; ++r)
-        if (draws->idx_pos[r] < 0 || draws->idx_pos[r] >= n_choices) return fail(OGB_ERR_INDEX, "idx_pos out of range");
-    if (aug_mode && !draws->has_aug_coin) return fail(OGB_ERR_INVALID, "validation mode: the augmentation coin is missing");
-    if (aug_mode && draws->aug_coin < p_aug_eff && !draws->crop) return fail(OGB_ERR_INVALID, "validation mode: crop draws are missing");
-  }
-  DeviceGuard device_guard(ds->device);
-  OGB_CUDA(device_guard.status);
-  std::lock_guard<std::mutex> lock(s->mu);
-  phase.mark();   // checks
+  p->n_choices = n_choices;
+}
 
-  const std::vector<KeyPlan>& plan = *spec.plan;
-  bool any_frames = false;
-  for (const KeyPlan& k : plan) any_frames |= (k.route == ROUTE_FRAMES && k.alias_of < 0);
-  const bool want_crop = any_frames;
-  const bool want_init = any_frames && cfg.frame_stack > 1;
-
-  // ---- lay out the single device block: keys first (so one D2H copy takes the whole batch), then scratch ----
-  ogb_batch* b = new ogb_batch();
-  b->sampler = s;
-  s->refs.fetch_add(1);
-  b->batch = batch_size;
-  b->n_batches = n_batches;
-  b->total_rows = total;
-  b->keys = plan;
-  b->offsets.assign(plan.size(), 0);
-  b->n_slots = spec.n_slots;
-  size_t cursor = 0;
-  for (size_t i = 0; i < plan.size(); ++i) {
-    if (plan[i].alias_of >= 0) continue;
-    b->offsets[i] = cursor;
-    cursor = round_up(cursor + (size_t)total * plan[i].row_bytes, 256);
-  }
-  for (size_t i = 0; i < plan.size(); ++i)
-    if (plan[i].alias_of >= 0) b->offsets[i] = b->offsets[(size_t)plan[i].alias_of];
-  b->keys_bytes = cursor;
-  auto carve = [&](size_t bytes) { size_t off = cursor; cursor = round_up(cursor + bytes, 256); return off; };
-  size_t off_trl_mid = 0;
-  size_t off_rows = 0, off_init = 0, off_crop = 0, off_idxs = 0, off_draw_i64[1 + 3 * 2 + 1] = {0}, off_draw_f64[3 * 3] = {0};
-  off_rows = carve((size_t)spec.n_slots * total * 4);
-  if (want_init) off_init = carve((size_t)spec.n_slots * total * 4);
-  if (want_crop) off_crop = carve((size_t)total * 2);
-  if (idxs) off_idxs = carve((size_t)total * 8);
-  size_t off_idx_error = 0;
-  if (defer_check) off_idx_error = carve(4);
-  if (draws) {
-    off_draw_i64[0] = carve((size_t)batch_size * 8);
-    for (int gs = 0; gs < 3; ++gs) {
-      off_draw_i64[1 + 2 * gs] = carve((size_t)batch_size * 8);
-      off_draw_i64[2 + 2 * gs] = carve((size_t)batch_size * 8);
-      for (int q = 0; q < 3; ++q) off_draw_f64[3 * gs + q] = carve((size_t)batch_size * 8);
-    }
-    off_draw_i64[7] = carve((size_t)batch_size * 16);
-    if (spec.trl) off_trl_mid = carve((size_t)batch_size * 8);
-  }
-  b->block_bytes = std::max<size_t>(cursor, 256);
-  auto bail = [&](int code) { batch_unref(b); return code; };
-  // Phase-one work (uploads of validation draws, the index kernel) goes to `first`: for big launches that is the
-  // auxiliary stream, so that the index kernel of this call overlaps the gathers of the previous call, which are
-  // still running on the main stream.  The recycled block only has to wait for its own previous owner.
-  const bool gather_lsu = ab().gather_lsu;
-  auto takes_async_path = [&](const Field& f) {
-    return f.row_bytes > 16 && f.stride <= (size_t)ogb::kAsyncMaxStride && (size_t)ds->size * f.stride < ((size_t)1 << 36) &&
-           !gather_lsu;
-  };
-  // When some key goes through the cp.async row gather, the index algebra is fused into that launch (one kernel per
-  // sample() for vector observations); otherwise the index kernel runs on its own.
-  // Measured on B200 with ~1M-row launches: fused wins for GCDataset shapes (C2 0.201 vs 0.216 ms, C5 0.356 vs 0.372)
-  // and loses for the heavier HGC algebra with its 16-row items (C3 0.757 vs 0.730 ms), so big HGC launches stay split;
-  // small launches always fuse (one kernel launch less).  Image batches keep the index kernel apart (it overlaps the
-  // previous call's frame gathers).  OGB_FUSE=0/1 forces either.
-  const int fuse_env = ab().fuse;
-  bool fuse = false;
-  if (fuse_env >= 0 ? fuse_env != 0 : (!any_frames && (total < kOverlapMinRows || spec.kind != OGB_KIND_HGC)))
-    for (const KeyPlan& k : plan)
-      if (k.route == ROUTE_ROW && k.alias_of < 0 && takes_async_path(ds->fields[(size_t)k.field])) fuse = true;
-  // Image batches are few rows with long gathers: their (latency-bound) index kernel always goes to the auxiliary
-  // stream, where it runs under the frame gathers of the previous call.
-  bool any_gather = any_frames;            // is there a gather launch for the index kernel to hide under?
-  for (const KeyPlan& k : plan)
-    if (k.route == ROUTE_ROW && k.alias_of < 0 && ds->fields[(size_t)k.field].row_bytes > 16) any_gather = true;
-  const bool use_aux = !fuse && any_gather && (total >= kOverlapMinRows || any_frames);
-  if (use_aux) {
-    int rc = ensure_aux(s);
-    if (rc) return bail(rc);
-  }
-  cudaStream_t first = use_aux ? s->aux_stream : s->stream;
-  phase.mark();   // batch + layout
-  {
-    std::vector<cudaEvent_t> free_after;
-    int rc = block_take(s, b->block_bytes, &b->block, &b->block_bytes, &free_after);
-    for (cudaEvent_t ev : free_after) {
-      cudaStreamWaitEvent(first, ev, 0);
-      if (first != s->stream) cudaStreamWaitEvent(s->stream, ev, 0);
-      cudaEventDestroy(ev);
-    }
-    if (rc) return bail(rc);
-  }
-  uint8_t* base = b->block;
-  phase.mark();   // block
-  if (s->canary) {
-    cudaMemsetAsync(base, 0xA5, b->block_bytes, first);
-    if (first != s->stream) {   // the gathers on the main stream must not start before the fill has finished
-      cudaEvent_t ev = s->chunk_events[s->next_event];
-      s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
-      cudaEventRecord(ev, first);
-      cudaStreamWaitEvent(s->stream, ev, 0);
-    }
-  }
-  b->vec_rows = (int32_t*)(base + off_rows);
-  if (want_crop) b->crop = (int8_t*)(base + off_crop);
-  if (want_init) b->vec_init = (int32_t*)(base + off_init);
-  if (total == 0) {   // an empty batch is legal (np.random.randint(n, size=0) in the reference): every key with zero rows, no launch
-    if (cudaEventCreateWithFlags(&b->ready, cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(b->ready, s->stream) != cudaSuccess)
-      return bail(fail(OGB_ERR_CUDA, "ready event failed"));
-    if (!draws) s->counter += (uint64_t)n_batches;
-    *out = b;
-    return 0;
-  }
-
-  // ---- parameters of the fused index + row-gather kernel ----
-  RelabelParams p;
-  memset(&p, 0, sizeof(p));
-  p.term = s->d_term;
-  p.term_bucket = s->d_term_bucket;
-  p.term_shift = s->term_shift;
-  p.valid_table = spec.choice_table ? spec.choice_table : ds->d_valid_table;
-  p.gap_c = ds->d_gap_c;
-  p.gap_bucket = ds->d_gap_bucket;
-  p.gap_shift = ds->gap_shift;
-  p.valid_mode = spec.choice_table ? 1 : ds->valid_mode;
-  if (!spec.choice_table && s->seg_shift >= 0) {
-    p.valid_mode = 3;
-    p.seg_table = s->d_seg_table;
-    p.seg_bucket = s->d_seg_bucket;
-    p.seg_shift = s->seg_shift;
-    p.n_seg_table = s->n_seg_table;
-    p.n_seg_bucket = s->n_seg_bucket;
-  }
-  p.next_offset = (int32_t)spec.next_offset;
-  p.trl = spec.trl ? 1 : 0;
-  p.n_choices = n_choices;
-  // (a ReplayBuffer that is still filling up clamps idx + 1 at its current size, datasets.py:82 with self.size = fill)
-  p.n_rows_ds = (int32_t)(spec.kind == OGB_KIND_PLAIN && ds->active_rows > 0 ? ds->active_rows : ds->size);
-  const double p_cur[3] = {cfg.value_p_curgoal, cfg.value_p_curgoal, cfg.actor_p_curgoal};
-  const double p_traj[3] = {cfg.value_p_trajgoal, cfg.value_p_trajgoal, cfg.actor_p_trajgoal};
-  const double disc[3] = {cfg.discount, cfg.has_low_discount ? cfg.low_discount : cfg.discount, cfg.discount};
+// How one goal set draws its goals (datasets.py:296-327).
+ogb::GoalSpec goal_spec(double p_cur, double p_traj, bool geom, double discount) {
   auto word_threshold = [](double prob, uint32_t* thr, uint8_t* always) {
     // (w * 2^-32 < prob) <=> (w < ceil(prob * 2^32)) for 32-bit words w; the scaling by 2^32 is exact in float64
     const double t = std::ceil(prob * 4294967296.0);
     *always = t >= 4294967296.0 ? 1 : 0;
     *thr = t <= 0.0 ? 0u : (t >= 4294967296.0 ? 0xFFFFFFFFu : (uint32_t)t);
   };
-  for (int gs = 0; gs < 3; ++gs) {
-    GoalSpec& spec = p.goal[gs];
-    spec.geom = geom[gs];
-    spec.cur_only = cur_only[gs];
-    spec.p_cur = p_cur[gs];
-    spec.thr_traj = cur_only[gs] ? 0.0 : p_traj[gs] / (1.0 - p_cur[gs]);
-    spec.log_1mp = std::log(1.0 - (1.0 - disc[gs]));
-    spec.geo_abs_margin = (float)(1.5e-8 / std::fabs(spec.log_1mp));
-    word_threshold(spec.thr_traj, &spec.thr_traj32, &spec.traj_always);
-    word_threshold(spec.p_cur, &spec.thr_cur32, &spec.cur_always);
-  }
-  {  // the actor coins are only drawn when they can change the outcome
-    const GoalSpec& a = p.goal[2];
-    const bool cur_fixed = a.cur_only || a.cur_always || a.thr_cur32 == 0;
-    const bool traj_fixed = a.traj_always || a.thr_traj32 == 0;
-    p.actor_mix = (a.cur_only || (cur_fixed && traj_fixed)) ? 0 : 1;
-  }
-  p.neg_lut = s->d_neg_lut;
-  p.pow_lut = s->d_pow_lut;
-  p.kind = spec.kind;
-  p.has_low_goal = goal_used[1];
-  p.k_val = cfg.value_subgoal_steps;
-  p.k_act = cfg.actor_subgoal_steps;
-  p.k_lo = cfg.low_subgoal_steps;
-  p.gc_negative = cfg.gc_negative;
-  p.stacked_next = stacked_next;
-  p.aug_mode = aug_mode;
-  p.crop_pad = crop_pad_eff;
-  p.p_aug = p_aug_eff;
-  p.key = make_rng_key(s->seed, s->stream_id);
-  p.batch0 = s->counter;
-  p.batch = batch_size;
-  p.batch_magic = batch_size > 1 && batch_size < ((int64_t)1 << 32) ? (uint64_t)(~(uint64_t)0 / (uint64_t)batch_size) + 1 : 0;
-  p.total_rows = total;
-  p.n_slots = spec.n_slots;
-  p.narrow = cfg.jax_compat ? 1 : 0;
-  p.vec_rows = b->vec_rows;
-  p.vec_init = b->vec_init;
-  p.crop_out = b->crop;
+  ogb::GoalSpec g{};
+  g.geom = geom;
+  g.cur_only = p_cur == 1.0;
+  g.p_cur = p_cur;
+  g.thr_traj = g.cur_only ? 0.0 : p_traj / (1.0 - p_cur);
+  g.log_1mp = std::log(1.0 - (1.0 - discount));
+  g.geo_abs_margin = (float)(1.5e-8 / std::fabs(g.log_1mp));
+  word_threshold(g.thr_traj, &g.thr_traj32, &g.traj_always);
+  word_threshold(g.p_cur, &g.thr_cur32, &g.cur_always);
+  return g;
+}
 
-  auto h2d = [&](size_t off, const void* src, size_t bytes) -> cudaError_t {
-    return cudaMemcpyAsync(base + off, src, bytes, cudaMemcpyHostToDevice, first);
-  };
-  if (idxs) {
-    if (h2d(off_idxs, idxs, (size_t)total * 8) != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "H2D of idxs failed"));
-    p.given_idxs = (const int64_t*)(base + off_idxs);
-    if (defer_check) {
-      b->idx_error = (int32_t*)(base + off_idx_error);
-      if (cudaMemsetAsync(b->idx_error, 0, 4, first) != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "memset of the index flag failed"));
-      p.idx_error = b->idx_error;
-      p.idx_last = idx_last;
-    }
-  }
-  if (draws) {
-    cudaError_t e = cudaSuccess;
-    if (draws->idx_pos && !idxs) { e = h2d(off_draw_i64[0], draws->idx_pos, (size_t)batch_size * 8); p.in_idx_pos = (const int64_t*)(base + off_draw_i64[0]); }
-    for (int gs = 0; gs < n_goal_sets && e == cudaSuccess; ++gs) {
-      if (!goal_used[gs]) continue;
-      const ogb_goal_draws& d = draws->goals[gs];
-      e = h2d(off_draw_i64[1 + 2 * gs], d.rand_pos, (size_t)batch_size * 8);
-      p.in_goal[gs].rand_pos = (const int64_t*)(base + off_draw_i64[1 + 2 * gs]);
-      if (d.offset && e == cudaSuccess) { e = h2d(off_draw_i64[2 + 2 * gs], d.offset, (size_t)batch_size * 8); p.in_goal[gs].offset = (const int64_t*)(base + off_draw_i64[2 + 2 * gs]); }
-      if (d.dist && e == cudaSuccess) { e = h2d(off_draw_f64[3 * gs], d.dist, (size_t)batch_size * 8); p.in_goal[gs].dist = (const double*)(base + off_draw_f64[3 * gs]); }
-      if (d.u_traj && e == cudaSuccess) { e = h2d(off_draw_f64[3 * gs + 1], d.u_traj, (size_t)batch_size * 8); p.in_goal[gs].u_traj = (const double*)(base + off_draw_f64[3 * gs + 1]); }
-      if (d.u_cur && e == cudaSuccess) { e = h2d(off_draw_f64[3 * gs + 2], d.u_cur, (size_t)batch_size * 8); p.in_goal[gs].u_cur = (const double*)(base + off_draw_f64[3 * gs + 2]); }
-    }
-    if (draws->crop && e == cudaSuccess) { e = h2d(off_draw_i64[7], draws->crop, (size_t)batch_size * 16); p.in_crop = (const int64_t*)(base + off_draw_i64[7]); }
-    if (spec.trl && e == cudaSuccess) {
-      if (!draws->trl_midpoints) return bail(fail(OGB_ERR_INVALID, "validation mode: TRL midpoint draws are missing"));
-      e = h2d(off_trl_mid, draws->trl_midpoints, (size_t)batch_size * 8);
-      p.in_trl_mid = (const int64_t*)(base + off_trl_mid);
-    }
-    p.in_coin = draws->has_aug_coin ? draws->aug_coin : 2.0;
-    if (p.aug_mode && !(p.in_coin < p.p_aug)) p.in_crop = nullptr;
-    if (e != cudaSuccess) return bail(fail(OGB_ERR_CUDA, "H2D of validation draws failed: %s", cudaGetErrorString(e)));
-  }
-  for (size_t i = 0; i < plan.size(); ++i) {
-    if (plan[i].route != ROUTE_SCALAR) continue;
-    void* ptr = base + b->offsets[i];
-    switch (plan[i].scalar) {
-      case SC_MASKS: p.masks = (double*)ptr; break;
-      case SC_REWARDS: p.rewards = (double*)ptr; break;
-      case SC_HV_OFFSETS: p.hv_offsets = (int64_t*)ptr; break;
-      case SC_HV_STEPS: p.hv_steps = (int64_t*)ptr; break;
-      case SC_HV_MASKS: p.hv_masks = (double*)ptr; break;
-      case SC_HV_REWARDS: p.hv_rewards = (double*)ptr; break;
-      case SC_LV_STEPS: p.lv_steps = (int64_t*)ptr; break;
-      case SC_LV_MASKS: p.lv_masks = (double*)ptr; break;
-      case SC_LV_REWARDS: p.lv_rewards = (double*)ptr; break;
-      case SC_TRL_OFFSETS: p.trl_offsets = (int64_t*)ptr; break;
-      case SC_TRL_MID_OFFSETS: p.trl_mid_offsets = (int64_t*)ptr; break;
-      default: break;
-    }
-  }
-  phase.mark();   // params
-  // ---- classify the vector-valued keys: tiny rows ride along in the index kernel, the rest go to a gather launch ----
-  // A span job loads one contiguous piece of the source rows named by one index vector and feeds one output per key.
+// Can the cp.async row gather read field f: rows at most kAsyncMaxStride apart, the whole field below 64 GiB, and the
+// register-staged gather not forced (OGB_GATHER=lsu)?
+bool async_reachable(const ogb_dataset* ds, const Field& f) {
+  return f.stride <= (size_t)ogb::kAsyncMaxStride && (size_t)ds->size * f.stride < ((size_t)1 << 36) && !ab().gather_lsu;
+}
+
+// A span job loads one contiguous piece of the source rows named by one index vector and feeds one output per key.
+struct SpanJob {
+  int slot;
+  const uint8_t* src;            // 16-byte aligned start of the span in row 0
+  size_t stride, bytes;          // source row stride, span length (multiple of 16)
+  std::vector<std::pair<size_t, size_t>> outs;   // (plan index, offset of the field inside the span)
+};
+
+// Sorts the row keys of a call by path: tiny rows ride along in the index kernel (the tiny jobs, groups and fields of
+// `p`), the rest go to a gather launch -- the returned span jobs of the cp.async row gather, or register-staged (LSU) keys.
+std::vector<SpanJob> classify_rows(const ogb_dataset* ds, const std::vector<KeyPlan>& plan, uint8_t* base,
+                                   const std::vector<size_t>& offsets, ogb::RelabelParams* p, std::vector<size_t>* lsu_keys) {
+  using namespace ogb;
   // Fields of the packed record table that are gathered through the same index vector and lie next to each other
   // (observations, actions, terminals, valids of the sampled transition) share ONE span.
-  struct SpanJob {
-    int slot;
-    const uint8_t* src;            // 16-byte aligned start of the span in row 0
-    size_t stride, bytes;          // source row stride, span length (multiple of 16)
-    std::vector<std::pair<size_t, size_t>> outs;   // (plan index, offset of the field inside the span)
-  };
   std::vector<SpanJob> span_jobs;
-  std::vector<size_t> lsu_keys;
-  p.n_tiny = 0;
-  {
-    auto add_tiny = [&](size_t i) -> bool {
-      const Field& f = ds->fields[(size_t)plan[i].field];
-      if (f.row_bytes > 16 || p.n_tiny >= kMaxTinyJobs) return false;
-      TinyJob& t = p.tiny[p.n_tiny++];
-      const int v = largest_vec_log2(f.row_bytes, f.row_bytes);
-      t.src = f.dptr;
-      t.dst = base + b->offsets[i];
-      t.slot = (uint8_t)plan[i].slot;
-      t.size_log2 = (uint8_t)v;
-      t.n_elem = (uint8_t)(f.row_bytes >> v);
-      t.row_bytes = (uint8_t)f.row_bytes;
-      t.stride = (uint16_t)f.stride;
-      return true;
-    };
-    std::map<int, std::vector<size_t>> record_keys;   // slot -> keys whose field lives in the record table
-    for (size_t i = 0; i < plan.size(); ++i) {
-      if (plan[i].route != ROUTE_ROW || plan[i].alias_of >= 0) continue;
-      const Field& f = ds->fields[(size_t)plan[i].field];
-      if (f.in_record && f.stride <= (size_t)kAsyncMaxStride && !gather_lsu &&
-          (size_t)ds->size * f.stride < ((size_t)1 << 36)) {
-        record_keys[plan[i].slot].push_back(i);
-      } else if (add_tiny(i)) {
-      } else if (takes_async_path(f)) {
-        span_jobs.push_back({plan[i].slot, f.dptr, f.stride, round_up(f.row_bytes, 16), {{i, 0}}});
-      } else {
-        lsu_keys.push_back(i);
-      }
-    }
-    for (auto& kv : record_keys) {
-      std::vector<size_t>& keys = kv.second;
-      std::sort(keys.begin(), keys.end(), [&](size_t a, size_t c) {
-        return ds->fields[(size_t)plan[a].field].rec_off < ds->fields[(size_t)plan[c].field].rec_off;
-      });
-      for (size_t k0 = 0; k0 < keys.size();) {
-        // extend the span while the next field starts within 32 bytes of the end of the current one, and while one
-        // gather launch still holds the span's outputs (items x fields, at the span's own stage budget: a launch's
-        // budget is never smaller, so it never has more items per span); an over-full span becomes two at a field boundary
-        const Field& f0 = ds->fields[(size_t)plan[keys[k0]].field];
-        size_t lo = f0.rec_off & ~(size_t)15, hi = f0.rec_off + f0.row_bytes, k1 = k0 + 1;
-        bool has_long = f0.row_bytes > 16;
-        while (k1 < keys.size()) {
-          const Field& fn = ds->fields[(size_t)plan[keys[k1]].field];
-          if (fn.rec_off > hi + 32) break;
-          const size_t pitch = round_up(std::max(hi, fn.rec_off + fn.row_bytes) - lo, 16);
-          if ((32 / rows_per_item(pitch, stage_budget(pitch))) * (k1 - k0 + 1) > (size_t)kMaxItemOuts) break;
-          hi = std::max(hi, fn.rec_off + fn.row_bytes);
-          has_long |= fn.row_bytes > 16;
-          ++k1;
-        }
-        if (has_long) {
-          SpanJob job{kv.first, ds->record_base + lo, ds->record_stride, round_up(hi - lo, 16), {}};
-          for (size_t k = k0; k < k1; ++k) job.outs.push_back({keys[k], ds->fields[(size_t)plan[keys[k]].field].rec_off - lo});
-          span_jobs.push_back(std::move(job));
-        } else {
-          // all tiny.  Fields of whole 4-byte words whose span fits two 16-byte loads become one group of the index
-          // kernel (one record load for all of them); whatever does not fit is copied field by field.
-          size_t k = k0;
-          const bool no_groups = ab().no_tiny_groups;
-          while (!no_groups && k < k1 && p.n_tiny_groups < kMaxTinyGroups) {
-            const Field& fa = ds->fields[(size_t)plan[keys[k]].field];
-            const size_t glo = fa.rec_off & ~(size_t)15;
-            size_t kk = k, n_f = 0;
-            int n_fields_total = 0;
-            for (int gi = 0; gi < p.n_tiny_groups; ++gi) n_fields_total += p.tiny_groups[gi].n_fields;
-            while (kk < k1) {
-              const Field& fk = ds->fields[(size_t)plan[keys[kk]].field];
-              if (fk.row_bytes % 4 != 0 || fk.rec_off % 4 != 0 || fk.rec_off + fk.row_bytes > glo + 32 ||
-                  (fk.row_bytes == 16 && (fk.rec_off - glo) % 16 != 0) || n_fields_total + (int)n_f >= kMaxTinyFields) break;
-              ++kk; ++n_f;
-            }
-            if (n_f < 2) break;                    // a single field gains nothing over a plain tiny copy
-            TinyGroup& grp = p.tiny_groups[p.n_tiny_groups++];
-            grp.src = ds->record_base + glo;
-            grp.stride = (uint16_t)ds->record_stride;
-            grp.slot = (uint8_t)kv.first;
-            grp.first_field = (uint8_t)n_fields_total;
-            grp.n_fields = (uint8_t)n_f;
-            size_t ghi = glo;
-            for (size_t t = k; t < kk; ++t) {
-              const Field& fk = ds->fields[(size_t)plan[keys[t]].field];
-              TinyField& tf = p.tiny_fields[n_fields_total++];
-              tf.dst = base + b->offsets[keys[t]];
-              tf.word = (uint8_t)((fk.rec_off - glo) / 4);
-              tf.n_words = (uint8_t)(fk.row_bytes / 4);
-              tf.group = (uint8_t)(p.n_tiny_groups - 1);
-              ghi = std::max(ghi, fk.rec_off + fk.row_bytes);
-            }
-            grp.n_vec = (uint8_t)(ghi - glo > 16 ? 2 : 1);
-            p.n_tiny_fields = n_fields_total;
-            k = kk;
-          }
-          for (; k < k1; ++k)
-            if (!add_tiny(keys[k])) {   // more tiny rows than the index kernel takes: a span of their own
-              const Field& fk = ds->fields[(size_t)plan[keys[k]].field];
-              const size_t l2 = fk.rec_off & ~(size_t)15;
-              span_jobs.push_back({kv.first, ds->record_base + l2, ds->record_stride, round_up(fk.rec_off + fk.row_bytes - l2, 16),
-                                   {{keys[k], fk.rec_off - l2}}});
-            }
-        }
-        k0 = k1;
-      }
-    }
-  }
-  {  // rows of 4, 8 or 16 bytes first: the index kernel copies those four at a time
-    auto fast = [](const TinyJob& t) { return t.row_bytes == 4 || t.row_bytes == 8 || t.row_bytes == 16; };
-    std::stable_partition(p.tiny, p.tiny + p.n_tiny, fast);
-    p.n_tiny_fast = (int32_t)std::count_if(p.tiny, p.tiny + p.n_tiny, fast);
-  }
-  const bool any_async = !span_jobs.empty();
-  fuse = fuse && any_async;
-  // The point-maze record (relabel_row<..., kPoint>): one group of the transition's own 32-byte record holding
-  // observations f32[2] | actions f32[2] | terminals | valids | shadow next observation, and the two 8-byte goal rows;
-  // nothing else to gather.  The index kernel then runs with these copies compiled in.
-  // (the kernel also compiles out what such a launch cannot need: index vectors in memory -- no later kernel, debug off --,
-  // frame-stack rows, the SLOT_NEXT row, the TRL branch, and every valid-row form but the segment table)
-  bool point_record = spec.kind == OGB_KIND_GC && !spec.trl && !any_async && lsu_keys.empty() && !any_frames &&
-                      !s->debug && p.valid_mode == 3 && p.vec_init == nullptr &&
-                      p.n_tiny_groups == 1 && p.n_tiny_fields == 5 && p.n_tiny == 2 && p.n_tiny_fast == 2 &&
-                      p.tiny_groups[0].slot == SLOT_IDX && p.tiny_groups[0].n_vec == 2 &&
-                      p.tiny[0].slot == GC_VALUE_GOAL && p.tiny[0].row_bytes == 8 && p.tiny[1].slot == GC_ACTOR_GOAL && p.tiny[1].row_bytes == 8;
-  if (point_record) {
-    static const int kWord[5] = {0, 2, 4, 5, 6}, kCount[5] = {2, 2, 1, 1, 2};
-    for (int f = 0; f < 5; ++f) point_record = point_record && p.tiny_fields[f].word == kWord[f] && p.tiny_fields[f].n_words == kCount[f];
-  }
-  // the index vectors only go to memory when a later launch (or the debug interface) reads them; a fused launch that
-  // leaves span jobs to a second row-gather launch sets it below, where the launch split is known
-  p.write_vecs = ((!fuse && any_async) || !lsu_keys.empty() || any_frames || s->debug) ? 1 : 0;
-
-  phase.mark();   // classify
-  // ---- prepare every launch once; each is then issued per row chunk ----
-  typedef std::function<int(int64_t, int64_t, cudaStream_t)> LaunchFn;
-  std::vector<LaunchFn> gather_launches;
-  LaunchFn fused_launch;
-  bool fused_writes_vecs = false;
-
-  LaunchFn index_launch = [&, p](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
-    p.row_begin = begin;
-    p.row_end = end;
-    const int64_t blocks_needed = (end - begin + kRelabelThreads - 1) / kRelabelThreads;
-    const int flavour = p.kind == OGB_KIND_GC ? FLAVOUR_GC : (p.kind == OGB_KIND_HGC ? FLAVOUR_HGC : FLAVOUR_PLAIN);
-    const bool inject = draws != nullptr;
-    // Big launches over a dataset whose segment table is small: persistent CTAs keep the table in shared memory.
-    const size_t table_bytes = (size_t)p.n_seg_table * 16 + (size_t)p.n_seg_bucket * 4;
-    // Used when the index kernel runs on the auxiliary stream under another call's gather: the persistent form with few
-    // CTAs disturbs the gather less (C3 0.716 vs 0.730 ms); alone on its stream the plain grid is faster (C1 0.047 vs 0.049).
-    const bool smem_tables = st != s->stream && p.valid_mode == 3 && table_bytes > 0 && table_bytes <= 48 * 1024 &&
-                             end - begin >= 65536;
-    const void* fn = nullptr;
-#define OGB_PICK_INDEX_KERNEL(INJ, SM)                                                                                  \
-    fn = flavour == FLAVOUR_GC ? (const void*)relabel_index_kernel<INJ, FLAVOUR_GC, SM>                                   \
-       : flavour == FLAVOUR_HGC ? (const void*)relabel_index_kernel<INJ, FLAVOUR_HGC, SM>                                 \
-                                : (const void*)relabel_index_kernel<INJ, FLAVOUR_PLAIN, SM>
-    if (inject && smem_tables) { OGB_PICK_INDEX_KERNEL(true, true); }
-    else if (inject) { OGB_PICK_INDEX_KERNEL(true, false); }
-    else if (smem_tables) { OGB_PICK_INDEX_KERNEL(false, true); }
-    else { OGB_PICK_INDEX_KERNEL(false, false); }
-#undef OGB_PICK_INDEX_KERNEL
-    if (point_record && !smem_tables)
-      // 48 registers, five CTAs per SM: 0.556 vs 0.541 of peak with four (six spill: 0.541), profiles/r2_ab_shapes.txt
-      fn = inject ? (const void*)relabel_index_kernel<true, FLAVOUR_GC, false, true> : (const void*)relabel_index_kernel<false, FLAVOUR_GC, false, true, 5>;
-    if (point_record && smem_tables && !inject) fn = (const void*)relabel_index_kernel<false, FLAVOUR_GC, true, true, 5>;
-    b->name_index = kernel_name("relabel_index_kernel", {inject ? 1 : 0, flavour, smem_tables ? 1 : 0, point_record && !(smem_tables && inject) ? 1 : 0,
-                                                        point_record && !inject ? 5 : 4});
-    // Grid cap: a whole number of waves of resident CTAs (a 16-per-SM grid of the five-per-SM point-maze kernel is 3.2
-    // waves, and the last, fifth-full wave cost C1 5 %: 0.731 vs 0.771-0.775 of peak for 5, 10 or 32 per SM, batch r2l).
-    static std::mutex occ_mu;
-    static std::map<const void*, int> occ_cache;
-    int resident_index = 0;
-    {
-      std::lock_guard<std::mutex> occ_lock(occ_mu);
-      auto it = occ_cache.find(fn);
-      if (it == occ_cache.end()) {
-        int per_sm = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kRelabelThreads, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
-        it = occ_cache.emplace(fn, per_sm).first;
-      }
-      resident_index = it->second;
-    }
-    int64_t grid_cap = (int64_t)ds->sm_count * 2 * resident_index;
-    size_t smem = 0;
-    if (smem_tables) {
-      smem = table_bytes;
-      int per_sm = 0;
-      if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-          cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kRelabelThreads, smem) != cudaSuccess || per_sm < 1)
-        return fail(OGB_ERR_CUDA, "relabel_index_kernel (shared tables): occupancy query failed");
-      grid_cap = (int64_t)ds->sm_count * per_sm;
-    }
-    const unsigned grid = (unsigned)std::min<int64_t>(blocks_needed, grid_cap);
-    void* args[] = {(void*)&p};
-    if (cudaLaunchKernel(fn, dim3(grid), dim3(kRelabelThreads), args, smem, st) != cudaSuccess)
-      return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed");
-    b->launches++;
-    return 0;
+  p->n_tiny = 0;
+  auto add_tiny = [&](size_t i) -> bool {
+    const Field& f = ds->fields[(size_t)plan[i].field];
+    if (f.row_bytes > 16 || p->n_tiny >= kMaxTinyJobs) return false;
+    TinyJob& t = p->tiny[p->n_tiny++];
+    const int v = largest_vec_log2(f.row_bytes, f.row_bytes);
+    t.src = f.dptr;
+    t.dst = base + offsets[i];
+    t.slot = (uint8_t)plan[i].slot;
+    t.size_log2 = (uint8_t)v;
+    t.n_elem = (uint8_t)(f.row_bytes >> v);
+    t.row_bytes = (uint8_t)f.row_bytes;
+    t.stride = (uint16_t)f.stride;
+    return true;
   };
+  std::map<int, std::vector<size_t>> record_keys;   // slot -> keys whose field lives in the record table
+  for (size_t i = 0; i < plan.size(); ++i) {
+    if (plan[i].route != ROUTE_ROW || plan[i].alias_of >= 0) continue;
+    const Field& f = ds->fields[(size_t)plan[i].field];
+    if (f.in_record && async_reachable(ds, f)) {
+      record_keys[plan[i].slot].push_back(i);
+    } else if (add_tiny(i)) {
+    } else if (f.row_bytes > 16 && async_reachable(ds, f)) {
+      span_jobs.push_back({plan[i].slot, f.dptr, f.stride, round_up(f.row_bytes, 16), {{i, 0}}});
+    } else {
+      lsu_keys->push_back(i);
+    }
+  }
+  for (auto& kv : record_keys) {
+    std::vector<size_t>& keys = kv.second;
+    std::sort(keys.begin(), keys.end(), [&](size_t a, size_t c) {
+      return ds->fields[(size_t)plan[a].field].rec_off < ds->fields[(size_t)plan[c].field].rec_off;
+    });
+    for (size_t k0 = 0; k0 < keys.size();) {
+      // extend the span while the next field starts within 32 bytes of the end of the current one, and while one
+      // gather launch still holds the span's outputs (items x fields, at the span's own stage budget: a launch's
+      // budget is never smaller, so it never has more items per span); an over-full span becomes two at a field boundary
+      const Field& f0 = ds->fields[(size_t)plan[keys[k0]].field];
+      size_t lo = f0.rec_off & ~(size_t)15, hi = f0.rec_off + f0.row_bytes, k1 = k0 + 1;
+      bool has_long = f0.row_bytes > 16;
+      while (k1 < keys.size()) {
+        const Field& fn = ds->fields[(size_t)plan[keys[k1]].field];
+        if (fn.rec_off > hi + 32) break;
+        const size_t pitch = round_up(std::max(hi, fn.rec_off + fn.row_bytes) - lo, 16);
+        if ((32 / rows_per_item(pitch, stage_budget(pitch))) * (k1 - k0 + 1) > (size_t)kMaxItemOuts) break;
+        hi = std::max(hi, fn.rec_off + fn.row_bytes);
+        has_long |= fn.row_bytes > 16;
+        ++k1;
+      }
+      if (has_long) {
+        SpanJob job{kv.first, ds->record_base + lo, ds->record_stride, round_up(hi - lo, 16), {}};
+        for (size_t k = k0; k < k1; ++k) job.outs.push_back({keys[k], ds->fields[(size_t)plan[keys[k]].field].rec_off - lo});
+        span_jobs.push_back(std::move(job));
+      } else {
+        // all tiny.  Fields of whole 4-byte words whose span fits two 16-byte loads become one group of the index
+        // kernel (one record load for all of them); whatever does not fit is copied field by field.
+        size_t k = k0;
+        const bool no_groups = ab().no_tiny_groups;
+        while (!no_groups && k < k1 && p->n_tiny_groups < kMaxTinyGroups) {
+          const Field& fa = ds->fields[(size_t)plan[keys[k]].field];
+          const size_t glo = fa.rec_off & ~(size_t)15;
+          size_t kk = k, n_f = 0;
+          int n_fields_total = 0;
+          for (int gi = 0; gi < p->n_tiny_groups; ++gi) n_fields_total += p->tiny_groups[gi].n_fields;
+          while (kk < k1) {
+            const Field& fk = ds->fields[(size_t)plan[keys[kk]].field];
+            if (fk.row_bytes % 4 != 0 || fk.rec_off % 4 != 0 || fk.rec_off + fk.row_bytes > glo + 32 ||
+                (fk.row_bytes == 16 && (fk.rec_off - glo) % 16 != 0) || n_fields_total + (int)n_f >= kMaxTinyFields) break;
+            ++kk; ++n_f;
+          }
+          if (n_f < 2) break;                    // a single field gains nothing over a plain tiny copy
+          TinyGroup& grp = p->tiny_groups[p->n_tiny_groups++];
+          grp.src = ds->record_base + glo;
+          grp.stride = (uint16_t)ds->record_stride;
+          grp.slot = (uint8_t)kv.first;
+          grp.first_field = (uint8_t)n_fields_total;
+          grp.n_fields = (uint8_t)n_f;
+          size_t ghi = glo;
+          for (size_t t = k; t < kk; ++t) {
+            const Field& fk = ds->fields[(size_t)plan[keys[t]].field];
+            TinyField& tf = p->tiny_fields[n_fields_total++];
+            tf.dst = base + offsets[keys[t]];
+            tf.word = (uint8_t)((fk.rec_off - glo) / 4);
+            tf.n_words = (uint8_t)(fk.row_bytes / 4);
+            tf.group = (uint8_t)(p->n_tiny_groups - 1);
+            ghi = std::max(ghi, fk.rec_off + fk.row_bytes);
+          }
+          grp.n_vec = (uint8_t)(ghi - glo > 16 ? 2 : 1);
+          p->n_tiny_fields = n_fields_total;
+          k = kk;
+        }
+        for (; k < k1; ++k)
+          if (!add_tiny(keys[k])) {   // more tiny rows than the index kernel takes: a span of their own
+            const Field& fk = ds->fields[(size_t)plan[keys[k]].field];
+            const size_t l2 = fk.rec_off & ~(size_t)15;
+            span_jobs.push_back({kv.first, ds->record_base + l2, ds->record_stride, round_up(fk.rec_off + fk.row_bytes - l2, 16),
+                                 {{keys[k], fk.rec_off - l2}}});
+          }
+      }
+      k0 = k1;
+    }
+  }
+  // rows of 4, 8 or 16 bytes first: the index kernel copies those four at a time
+  auto fast = [](const TinyJob& t) { return t.row_bytes == 4 || t.row_bytes == 8 || t.row_bytes == 16; };
+  std::stable_partition(p->tiny, p->tiny + p->n_tiny, fast);
+  p->n_tiny_fast = (int32_t)std::count_if(p->tiny, p->tiny + p->n_tiny, fast);
+  return span_jobs;
+}
 
-  // asynchronous row gather (cp.async ring per warp), all element widths in one launch.  The jobs of a launch are
-  // unrolled into the item list of one 32-row tile (relabel_rows.cuh, ItemDesc / OutDesc); a job list that needs more
-  // items or outputs than a launch holds is split over several launches.
-  for (size_t q = 0; q < span_jobs.size();) {
-    AsyncGatherParams ap;
-    memset(&ap, 0, sizeof(ap));
-    ap.vec_rows = b->vec_rows;
-    ap.total_rows = total;
-    const size_t q0 = q;
-    auto magic = [](uint32_t d) -> uint32_t { return d <= 1 ? 0u : (uint32_t)((((uint64_t)1 << 32) + d - 1) / d); };
+// The point-maze record (relabel_row<..., kPoint>): one group of the transition's own 32-byte record holding
+// observations f32[2] | actions f32[2] | terminals | valids | shadow next observation, and the two 8-byte goal rows;
+// nothing else to gather.  The index kernel then runs with these copies compiled in.
+// (the kernel also compiles out what such a launch cannot need: index vectors in memory -- no later kernel, debug off --,
+// frame-stack rows, the SLOT_NEXT row, the TRL branch, and every valid-row form but the segment table)
+bool is_point_record(const ogb_sampler* s, const RunSpec& spec, const ogb::RelabelParams& p, bool any_gather) {
+  using namespace ogb;
+  if (!(spec.kind == OGB_KIND_GC && !spec.trl && !any_gather &&
+        !s->debug && p.valid_mode == 3 && p.vec_init == nullptr &&
+        p.n_tiny_groups == 1 && p.n_tiny_fields == 5 && p.n_tiny == 2 && p.n_tiny_fast == 2 &&
+        p.tiny_groups[0].slot == SLOT_IDX && p.tiny_groups[0].n_vec == 2 &&
+        p.tiny[0].slot == GC_VALUE_GOAL && p.tiny[0].row_bytes == 8 && p.tiny[1].slot == GC_ACTOR_GOAL && p.tiny[1].row_bytes == 8))
+    return false;
+  static const int kWord[5] = {0, 2, 4, 5, 6}, kCount[5] = {2, 2, 1, 1, 2};
+  for (int f = 0; f < 5; ++f)
+    if (p.tiny_fields[f].word != kWord[f] || p.tiny_fields[f].n_words != kCount[f]) return false;
+  return true;
+}
+
+// One launch of the cp.async row gather: span jobs [first, end), its stage budget and stage bytes, and its shape
+// (100 * stages + warps per CTA).
+struct RowLaunch {
+  size_t first, end, budget;
+  int stage_bytes, shape;
+};
+
+// Splits the span jobs over launches (all element widths in one launch; a job list that needs more items or outputs
+// than a launch holds goes to several).  The first launch is the fused one when `fuse`; `gc_philox`: the call is a
+// GCDataset one with Philox draws.
+int split_span_jobs(const std::vector<SpanJob>& span_jobs, bool fuse, bool gc_philox, std::vector<RowLaunch>* out) {
+  using namespace ogb;
+  for (size_t q0 = 0; q0 < span_jobs.size();) {
     size_t q1 = std::min(span_jobs.size(), q0 + (size_t)kMaxRowJobs), budget = 0;
     for (;; --q1) {   // the largest prefix of the remaining jobs whose items and outputs fit one launch
       size_t max_pitch = 0, n_items = 0, n_outs = 0;
@@ -2330,14 +2075,13 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
       }
       if ((n_items <= (size_t)kMaxItems && n_outs <= (size_t)kMaxItemOuts) || q1 == q0 + 1) {
         if (n_items > (size_t)kMaxItems || n_outs > (size_t)kMaxItemOuts)
-          return bail(fail(OGB_ERR_UNSUPPORTED, "a %zu-byte row span with %zu keys does not fit one gather launch", span_jobs[q0].bytes, span_jobs[q0].outs.size()));
+          return fail(OGB_ERR_UNSUPPORTED, "a %zu-byte row span with %zu keys does not fit one gather launch", span_jobs[q0].bytes, span_jobs[q0].outs.size());
         break;
       }
     }
-    auto rows_for = [&](size_t pitch) { return rows_per_item(pitch, budget); };
     size_t stage = 0;
-    for (size_t t = q0; t < q1; ++t) stage = std::max(stage, rows_for(span_jobs[t].bytes) * span_jobs[t].bytes);
-    ap.stage_bytes = (int)round_up(stage, 128);
+    for (size_t t = q0; t < q1; ++t) stage = std::max(stage, rows_per_item(span_jobs[t].bytes, budget) * span_jobs[t].bytes);
+    const int stage_bytes = (int)round_up(stage, 128);
     // (stages, warps per CTA): 3 x 8 (two CTAs per SM), except for the fused GCDataset launch (2 x 20, or 2 x 16 when
     // 20 warps' rings do not fit) and the un-fused gather with stages over 4 KB (3 x 10).
     // Measured on B200 (profiles/r2_ab_shapes.txt).  Fused GCDataset launch: ONE CTA of 20 warps with two stages per warp
@@ -2348,150 +2092,417 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
     // algebra out of line, to keep the loops under the 80-register cap, lost 25 %).  Un-fused gather: three
     // stages; with 6 KB stages (rows > 256 B: C3) ten warps in one CTA, 0.979 vs 0.964 for eight (twelve: 0.968).
     const bool fused_here = fuse && q0 == 0;
-    const bool fused_gc = fused_here && p.kind == OGB_KIND_GC && draws == nullptr;
     int shape = 308;
-    if (fused_gc) shape = (size_t)20 * 2 * ap.stage_bytes <= (size_t)200 * 1024 ? 220 : 216;
-    else if (!fused_here && ap.stage_bytes > 4096 && (size_t)10 * 3 * ap.stage_bytes <= (size_t)200 * 1024) shape = 310;
-    const int n_stages = shape / 100, n_warps = shape % 100;
-    ap.ring_bytes = n_stages * ap.stage_bytes;
-    for (; q < q1; ++q) {
-      const SpanJob& sj = span_jobs[q];
-      const uint32_t cpr = (uint32_t)(sj.bytes / 16), pitch = cpr * 16u;
-      const uint32_t rpi = (uint32_t)rows_for(pitch);
-      for (uint32_t sub = 0; sub < 32; sub += rpi) {
-        ItemDesc& it = ap.items[ap.n_items++];
-        it.src16 = reinterpret_cast<const uint4*>(sj.src);
-        it.stride16 = (uint32_t)(sj.stride / 16);
-        it.cpr = cpr;
-        it.cpr_magic = magic(cpr);
-        it.dr = 32 / cpr;
-        it.dch = 32 % cpr;
-        it.slot = (uint32_t)sj.slot;
-        it.sub = sub;
-        it.rows = rpi;
-        it.flags = sub == 0 ? 1u : 0u;
-        it.out_begin_n = (uint32_t)ap.n_outs | ((uint32_t)sj.outs.size() << 16);
-        for (const auto& po : sj.outs) {
-          const Field& f = ds->fields[(size_t)plan[po.first].field];
-          OutDesc& out = ap.outs[ap.n_outs++];
-          out.dst = base + b->offsets[po.first] + (size_t)sub * f.row_bytes;
-          out.tile_bytes = (uint32_t)(32 * f.row_bytes);
-          out.soff = (uint32_t)po.second;
-          out.gap = pitch - (uint32_t)f.row_bytes;
-          uint32_t kind, vec_log2 = 0;
-          if (f.row_bytes % 16 == 0 && out.gap == 0) {
-            kind = DRAIN_DENSE16;
-            out.epr = (uint32_t)f.row_bytes;
-          } else if (f.row_bytes % 4 == 0 && po.second % 4 == 0) {
-            // items start on 16-byte boundaries of the dense output unless an item holds fewer than four odd-sized rows
-            kind = ((size_t)sub * f.row_bytes) % 16 == 0 ? DRAIN_WORDS : DRAIN_WORDS_UNALIGNED;
-            out.epr = (uint32_t)(f.row_bytes / 4);
-          } else {
-            kind = DRAIN_ELEMS;
-            vec_log2 = (f.row_bytes % 2 == 0 && po.second % 2 == 0) ? 1 : 0;
-            out.epr = (uint32_t)(f.row_bytes >> vec_log2);
-          }
-          out.epr_magic = magic(out.epr);
-          out.kind = kind | (vec_log2 << 8) | (pitch << 16);
+    if (fused_here && gc_philox) shape = (size_t)20 * 2 * stage_bytes <= (size_t)200 * 1024 ? 220 : 216;
+    else if (!fused_here && stage_bytes > 4096 && (size_t)10 * 3 * stage_bytes <= (size_t)200 * 1024) shape = 310;
+    out->push_back({q0, q1, budget, stage_bytes, shape});
+    q0 = q1;
+  }
+  return 0;
+}
+
+// The item and output tables of one row-gather launch (relabel_rows.cuh, ItemDesc / OutDesc: the jobs unrolled into the
+// items of one 32-row tile), with the drain kind of every output, the index-vector prefetch links and the item at which
+// a warp claims its next tile.  Returns the number of (tile, index vector) pairs.
+size_t fill_row_tables(const ogb_dataset* ds, const std::vector<KeyPlan>& plan, uint8_t* base, const std::vector<size_t>& offsets,
+                       const std::vector<SpanJob>& span_jobs, const RowLaunch& rl, bool fused, ogb::AsyncGatherParams* ap) {
+  using namespace ogb;
+  auto magic = [](uint32_t d) -> uint32_t { return d <= 1 ? 0u : (uint32_t)((((uint64_t)1 << 32) + d - 1) / d); };
+  for (size_t q = rl.first; q < rl.end; ++q) {
+    const SpanJob& sj = span_jobs[q];
+    const uint32_t cpr = (uint32_t)(sj.bytes / 16), pitch = cpr * 16u;
+    const uint32_t rpi = (uint32_t)rows_per_item(pitch, rl.budget);
+    for (uint32_t sub = 0; sub < 32; sub += rpi) {
+      ItemDesc& it = ap->items[ap->n_items++];
+      it.src16 = reinterpret_cast<const uint4*>(sj.src);
+      it.stride16 = (uint32_t)(sj.stride / 16);
+      it.cpr = cpr;
+      it.cpr_magic = magic(cpr);
+      it.dr = 32 / cpr;
+      it.dch = 32 % cpr;
+      it.slot = (uint32_t)sj.slot;
+      it.sub = sub;
+      it.rows = rpi;
+      it.flags = sub == 0 ? 1u : 0u;
+      it.out_begin_n = (uint32_t)ap->n_outs | ((uint32_t)sj.outs.size() << 16);
+      for (const auto& po : sj.outs) {
+        const Field& f = ds->fields[(size_t)plan[po.first].field];
+        OutDesc& out = ap->outs[ap->n_outs++];
+        out.dst = base + offsets[po.first] + (size_t)sub * f.row_bytes;
+        out.tile_bytes = (uint32_t)(32 * f.row_bytes);
+        out.soff = (uint32_t)po.second;
+        out.gap = pitch - (uint32_t)f.row_bytes;
+        uint32_t kind, vec_log2 = 0;
+        if (f.row_bytes % 16 == 0 && out.gap == 0) {
+          kind = DRAIN_DENSE16;
+          out.epr = (uint32_t)f.row_bytes;
+        } else if (f.row_bytes % 4 == 0 && po.second % 4 == 0) {
+          // items start on 16-byte boundaries of the dense output unless an item holds fewer than four odd-sized rows
+          kind = ((size_t)sub * f.row_bytes) % 16 == 0 ? DRAIN_WORDS : DRAIN_WORDS_UNALIGNED;
+          out.epr = (uint32_t)(f.row_bytes / 4);
+        } else {
+          kind = DRAIN_ELEMS;
+          vec_log2 = (f.row_bytes % 2 == 0 && po.second % 2 == 0) ? 1 : 0;
+          out.epr = (uint32_t)(f.row_bytes >> vec_log2);
         }
+        out.epr_magic = magic(out.epr);
+        out.kind = kind | (vec_log2 << 8) | (pitch << 16);
       }
     }
-    // index-vector prefetch of the un-fused kernel: every pair's first item names the slot (and tile) of the pair after it
-    for (int k = 0; k < ap.n_items; ++k) {
-      if (!(ap.items[k].flags & 1u)) continue;
-      int nk = k + 1;
-      while (nk < ap.n_items && !(ap.items[nk].flags & 1u)) ++nk;
-      const bool wraps = nk == ap.n_items;
-      ap.items[k].flags |= (ap.items[wraps ? 0 : nk].slot << 8) | (wraps ? 0x10000u : 0u);
+  }
+  // index-vector prefetch of the un-fused kernel: every pair's first item names the slot (and tile) of the pair after it
+  for (int k = 0; k < ap->n_items; ++k) {
+    if (!(ap->items[k].flags & 1u)) continue;
+    int nk = k + 1;
+    while (nk < ap->n_items && !(ap->items[nk].flags & 1u)) ++nk;
+    const bool wraps = nk == ap->n_items;
+    ap->items[k].flags |= (ap->items[wraps ? 0 : nk].slot << 8) | (wraps ? 0x10000u : 0u);
+  }
+  // Dynamic tile scheduling: the ticket of the next tile is taken ahead of the item where the head needs the tile -- the
+  // fused kernel needs it when it leaves the tile, the un-fused one already at the first item of the last pair, where it
+  // prefetches the next tile's index vector.  How far ahead, measured (profiles/r2_ab_shapes.txt, batch r2k): the fused
+  // launches (16 warps per SM) are best with one pair -- a ticket taken earlier keeps a tile away from a faster warp
+  // (C2 0.890 / 0.888 / 0.876 of peak for 1 / 2 / all pairs ahead); the un-fused gather with 8 warps per SM does not cover
+  // a late ticket's round trip through the busy memory system (C3 0.952 / 0.956 / 0.960 / 0.963 for 1 / 2 / 3 / all),
+  // while C5b's shape prefers <= 3 (1.021 vs 1.011) -> three.
+  std::vector<int> pair_first;
+  for (int k = 0; k < ap->n_items; ++k) if (ap->items[k].flags & 1u) pair_first.push_back(k);
+  // index (into pair_first) of the pair at whose first item the tile is needed; the fused kernel needs it one pair "later"
+  const int need = (int)pair_first.size() - (fused ? 0 : 1);
+  const int ahead = fused ? 1 : 3;
+  ap->claim_item = pair_first[(size_t)std::max(0, need - ahead)];
+  return pair_first.size();
+}
+
+typedef std::function<int(int64_t, int64_t, cudaStream_t)> LaunchFn;
+
+// relabel_index_kernel over rows [begin, end); `dominant`: it is the call's dominant kernel, and names itself as it launches
+LaunchFn index_launch(ogb_sampler* s, ogb_batch* b, const ogb::RelabelParams& params, bool inject, int flavour, bool point_record,
+                      bool dominant) {
+  using namespace ogb;
+  return [=, p = params](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
+    p.row_begin = begin;
+    p.row_end = end;
+    const int64_t blocks_needed = (end - begin + kRelabelThreads - 1) / kRelabelThreads;
+    // Shared memory (0: the plain grid).  Big launches over a dataset whose segment table is small keep the table in shared
+    // memory (persistent CTAs) when they run on the auxiliary stream under another call's gather: the persistent form
+    // with few CTAs disturbs the gather less (C3 0.716 vs 0.730 ms); alone on its stream the plain grid is faster (C1
+    // 0.047 vs 0.049).
+    const size_t table_bytes = (size_t)p.n_seg_table * 16 + (size_t)p.n_seg_bucket * 4;
+    const size_t smem = st != s->stream && p.valid_mode == 3 && table_bytes > 0 && table_bytes <= 48 * 1024 &&
+                        end - begin >= 65536 ? table_bytes : 0;
+    const KernelChoice k = choose_index_kernel(inject, flavour, smem > 0, point_record);
+    // Grid cap: a whole number of waves of resident CTAs (a 16-per-SM grid of the five-per-SM point-maze kernel is 3.2
+    // waves, and the last, fifth-full wave cost C1 5 %: 0.731 vs 0.771-0.775 of peak for 5, 10 or 32 per SM, batch r2l).
+    int64_t grid_cap = (int64_t)s->ds->sm_count * 2 * k.resident;
+    if (smem > 0) {
+      int per_sm = 0;
+      if (cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+          cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k.fn, kRelabelThreads, smem) != cudaSuccess || per_sm < 1)
+        return fail(OGB_ERR_CUDA, "relabel_index_kernel (shared tables): occupancy query failed");
+      grid_cap = (int64_t)s->ds->sm_count * per_sm;
     }
-    // Dynamic tile scheduling: the ticket of the next tile is taken ahead of the item where the head needs the tile -- the
-    // fused kernel needs it when it leaves the tile, the un-fused one already at the first item of the last pair, where it
-    // prefetches the next tile's index vector (a single-pair un-fused launch keeps static tiles).  How far ahead, measured
-    // (profiles/r2_ab_shapes.txt, batch r2k): the fused launches (16 warps per SM) are best with one pair -- a ticket taken
-    // earlier keeps a tile away from a faster warp (C2 0.890 / 0.888 / 0.876 of peak for 1 / 2 / all pairs ahead); the
-    // un-fused gather with 8 warps per SM does not cover a late ticket's round trip through the busy memory system
-    // (C3 0.952 / 0.956 / 0.960 / 0.963 for 1 / 2 / 3 / all), while C5b's shape prefers <= 3 (1.021 vs 1.011) -> three.
-    std::vector<int> pair_first;
-    for (int k = 0; k < ap.n_items; ++k) if (ap.items[k].flags & 1u) pair_first.push_back(k);
-    const bool dyn_tiles = !s->static_tiles && (fused_here || pair_first.size() >= 2);
-    {
-      // index (into pair_first) of the pair at whose first item the tile is needed; the fused kernel needs it one pair "later"
-      const int need = (int)pair_first.size() - (fused_here ? 0 : 1);
-      const int ahead = fused_here ? 1 : 3;
-      ap.claim_item = pair_first[(size_t)std::max(0, need - ahead)];
+    const unsigned grid = (unsigned)std::min<int64_t>(blocks_needed, grid_cap);
+    void* args[] = {(void*)&p};
+    if (cudaLaunchKernel(k.fn, dim3(grid), dim3(kRelabelThreads), args, smem, st) != cudaSuccess)
+      return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed");
+    if (dominant) b->dominant = k.name;
+    b->launches++;
+    return 0;
+  };
+}
+
+// One run_sample call: its arguments, what they imply under the sampler's config, its batch and its launches.  The steps
+// run in this order: check, new_batch, fill_params, the prepare_* steps, issue.
+struct Run {
+  ogb_sampler* s;
+  const ogb_dataset* ds;
+  const ogb_config& cfg;
+  const RunSpec& spec;
+  const std::vector<KeyPlan>& plan;
+  int64_t batch, total;
+  int32_t n_batches;
+  const int64_t* idxs;
+  const ogb_draws* draws;
+  bool stacked_next = false;
+  int64_t idx_last = 0;             // the largest index a given row may have
+  bool defer_check = false;         // given indices are range-checked by the kernel (the flag is read later)
+  int64_t n_choices = 0;
+  bool aug_mode = false;
+  double p_aug = 0.0;
+  int crop_pad = 0;
+  bool goal_used[3] = {false, false, false};   // goal sets drawn: value, low-value, actor
+  ogb_batch* b = nullptr;
+  cudaStream_t first = nullptr;     // stream of the uploads and of the index kernel or fused launch
+  // where the scratch arrays of the batch block start (the keys come first, at ogb_batch::offsets)
+  size_t off_rows = 0, off_init = 0, off_crop = 0, off_idxs = 0, off_idx_error = 0, off_trl_mid = 0;
+  size_t off_draw_i64[1 + 3 * 2 + 1] = {0}, off_draw_f64[3 * 3] = {0};
+  // the launches, prepared once and issued per row chunk: the index kernel -- or the fused launch, which does its work
+  // too -- and the gathers behind it
+  LaunchFn index, fused;
+  std::vector<LaunchFn> gathers;
+  ogb::RelabelParams p;             // of the index algebra (index kernel or fused launch)
+
+  int check(bool evaluation) {
+    if (batch < 0 || n_batches < 1) return fail(OGB_ERR_INVALID, "batch_size must be >= 0 and n_batches >= 1");
+    if (draws && n_batches != 1) return fail(OGB_ERR_INVALID, "validation draws need n_batches == 1");
+    if (total > (int64_t)1 << 31) return fail(OGB_ERR_UNSUPPORTED, "more than 2^31 rows in one launch");
+    stacked_next = (cfg.frame_stack > 0 && spec.kind != OGB_KIND_PLAIN) || spec.kind == OGB_KIND_ATC;
+    idx_last = (stacked_next ? ds->size - spec.next_offset : ds->size) - 1;
+    defer_check = idxs && s->defer_index_check;
+    if (idxs && !defer_check) {  // numpy fancy indexing would raise IndexError (negative wrap-around is not supported here)
+      // branch-free scan (vectorises): idx < 0 or idx > last sets the sign bit of idx | (last - idx)
+      int64_t bad = 0;
+      for (int64_t r = 0; r < total; ++r) bad |= idxs[r] | (idx_last - idxs[r]);
+      if (bad < 0)
+        for (int64_t r = 0; r < total; ++r)
+          if (idxs[r] < 0 || idxs[r] > idx_last)
+            return fail(OGB_ERR_INDEX, "index %lld is out of bounds for axis 0 with size %lld", (long long)idxs[r], (long long)ds->size);
     }
-    // shared memory: item table, output table, one 16-byte tile FIFO per warp, then the rings
-    ap.ring_offset = (int)round_up((size_t)ap.n_items * sizeof(ItemDesc) + (size_t)ap.n_outs * sizeof(OutDesc) + (size_t)n_warps * 16, 128);
-    const size_t smem = (size_t)ap.ring_offset + (size_t)n_warps * ap.ring_bytes;
-    if (smem > (size_t)225 * 1024)
-      return bail(fail(OGB_ERR_UNSUPPORTED, "internal: gather shape %d needs %zu bytes of shared memory", shape, smem));
-    // persistent grid: exactly the CTAs that are resident at once (shared memory bounds them here; the fused kernels are
-    // compiled for gather_min_blocks(warps) CTAs per SM, so registers allow at least that many)
-    const int ctas_per_sm = (int)std::max<size_t>(1, std::min<size_t>(n_warps <= 8 ? 2 : 1, (size_t)(220 * 1024) / smem));
-    if (fused_here) {
+    if (idxs && spec.trl) {
+      // datasets.py:255-256: `assert (idxs != final_state_idxs).all()` -- a given index that is a trajectory's final state
+      // (a terminal row) has no midpoint span, and its idx + 1 belongs to the next trajectory (or lies past the table)
+      for (int64_t r = 0; r < total; ++r)
+        if (idxs[r] >= 0 && idxs[r] < ds->size && !ds->terminals_host.empty() && ds->terminals_host[(size_t)idxs[r]])
+          return fail(OGB_ERR_ASSERT, "assert (idxs != final_state_idxs).all() (datasets.py:256): index %lld is a final state", (long long)idxs[r]);
+    }
+    n_choices = n_choices_for(ds, spec.choice_table, spec.n_choices);
+    if (n_choices < 1) return fail(OGB_ERR_INVALID, "nothing to sample from: the dataset holds no rows yet");
+    const bool forced_crop = spec.crop_padding >= 0;
+    aug_mode = forced_crop || (cfg.has_p_aug && !evaluation && spec.kind != OGB_KIND_PLAIN);
+    p_aug = forced_crop ? 1.0 : cfg.p_aug;
+    crop_pad = forced_crop ? spec.crop_padding : cfg.crop_padding;
+    goal_used[0] = goal_used[2] = spec.kind == OGB_KIND_GC || spec.kind == OGB_KIND_HGC;
+    goal_used[1] = spec.kind == OGB_KIND_HGC && cfg.has_low_discount;
+    if (draws) {
+      const bool geom[3] = {cfg.value_geom_sample != 0, true, cfg.actor_geom_sample != 0};
+      const bool cur_only[3] = {cfg.value_p_curgoal == 1.0, cfg.value_p_curgoal == 1.0, cfg.actor_p_curgoal == 1.0};
+      if (!idxs && !draws->idx_pos) return fail(OGB_ERR_INVALID, "validation mode needs idx_pos or idxs");
+      for (int gs = 0; gs < 3; ++gs) {
+        if (!goal_used[gs]) continue;
+        const ogb_goal_draws& d = draws->goals[gs];
+        if (!d.rand_pos || (geom[gs] ? !d.offset : !d.dist) || (!cur_only[gs] && (!d.u_traj || !d.u_cur)))
+          return fail(OGB_ERR_INVALID, "validation mode: goal set %d is missing draws", gs);
+        for (int64_t r = 0; r < batch; ++r)
+          if (d.rand_pos[r] < 0 || d.rand_pos[r] >= n_choices) return fail(OGB_ERR_INDEX, "rand_pos out of range");
+      }
+      if (draws->idx_pos && !idxs)
+        for (int64_t r = 0; r < batch; ++r)
+          if (draws->idx_pos[r] < 0 || draws->idx_pos[r] >= n_choices) return fail(OGB_ERR_INDEX, "idx_pos out of range");
+      if (aug_mode && !draws->has_aug_coin) return fail(OGB_ERR_INVALID, "validation mode: the augmentation coin is missing");
+      if (aug_mode && draws->aug_coin < p_aug && !draws->crop) return fail(OGB_ERR_INVALID, "validation mode: crop draws are missing");
+    }
+    return 0;
+  }
+  // A batch of the call's keys and the layout of its device block: keys first (so that one D2H copy takes the whole
+  // batch), then the index vectors and the uploaded arguments.
+  void new_batch(bool want_init, bool want_crop) {
+    b = new ogb_batch();
+    b->sampler = s;
+    s->refs.fetch_add(1);
+    b->batch = batch;
+    b->n_batches = n_batches;
+    b->total_rows = total;
+    b->keys = plan;
+    b->offsets.assign(plan.size(), 0);
+    b->n_slots = spec.n_slots;
+    size_t cursor = 0;
+    for (size_t i = 0; i < plan.size(); ++i) {
+      if (plan[i].alias_of >= 0) continue;
+      b->offsets[i] = cursor;
+      cursor = round_up(cursor + (size_t)total * plan[i].row_bytes, 256);
+    }
+    for (size_t i = 0; i < plan.size(); ++i)
+      if (plan[i].alias_of >= 0) b->offsets[i] = b->offsets[(size_t)plan[i].alias_of];
+    b->keys_bytes = cursor;
+    auto carve = [&](size_t bytes) { size_t off = cursor; cursor = round_up(cursor + bytes, 256); return off; };
+    off_rows = carve((size_t)spec.n_slots * total * 4);
+    if (want_init) off_init = carve((size_t)spec.n_slots * total * 4);
+    if (want_crop) off_crop = carve((size_t)total * 2);
+    if (idxs) off_idxs = carve((size_t)total * 8);
+    if (defer_check) off_idx_error = carve(4);
+    if (draws) {
+      off_draw_i64[0] = carve((size_t)batch * 8);
+      for (int gs = 0; gs < 3; ++gs) {
+        off_draw_i64[1 + 2 * gs] = carve((size_t)batch * 8);
+        off_draw_i64[2 + 2 * gs] = carve((size_t)batch * 8);
+        for (int q = 0; q < 3; ++q) off_draw_f64[3 * gs + q] = carve((size_t)batch * 8);
+      }
+      off_draw_i64[7] = carve((size_t)batch * 16);
+      if (spec.trl) off_trl_mid = carve((size_t)batch * 8);
+    }
+    b->block_bytes = std::max<size_t>(cursor, 256);
+  }
+  // The parameters of the index algebra (index kernel or fused launch) except the row keys; uploads the given indices and
+  // validation draws on `first`.
+  int fill_params() {
+    using namespace ogb;
+    uint8_t* base = b->block;
+    memset(&p, 0, sizeof(p));
+    set_row_tables(s, spec.choice_table, n_choices, &p);
+    p.next_offset = (int32_t)spec.next_offset;
+    p.trl = spec.trl ? 1 : 0;
+    // (a ReplayBuffer that is still filling up clamps idx + 1 at its current size, datasets.py:82 with self.size = fill)
+    p.n_rows_ds = (int32_t)(spec.kind == OGB_KIND_PLAIN && ds->active_rows > 0 ? ds->active_rows : ds->size);
+    p.goal[0] = goal_spec(cfg.value_p_curgoal, cfg.value_p_trajgoal, cfg.value_geom_sample != 0, cfg.discount);
+    p.goal[1] = goal_spec(cfg.value_p_curgoal, cfg.value_p_trajgoal, true, cfg.has_low_discount ? cfg.low_discount : cfg.discount);
+    p.goal[2] = goal_spec(cfg.actor_p_curgoal, cfg.actor_p_trajgoal, cfg.actor_geom_sample != 0, cfg.discount);
+    {  // the actor coins are only drawn when they can change the outcome
+      const GoalSpec& a = p.goal[2];
+      const bool cur_fixed = a.cur_only || a.cur_always || a.thr_cur32 == 0;
+      const bool traj_fixed = a.traj_always || a.thr_traj32 == 0;
+      p.actor_mix = (a.cur_only || (cur_fixed && traj_fixed)) ? 0 : 1;
+    }
+    p.neg_lut = s->d_neg_lut;
+    p.pow_lut = s->d_pow_lut;
+    p.kind = spec.kind;
+    p.has_low_goal = goal_used[1];
+    p.k_val = cfg.value_subgoal_steps;
+    p.k_act = cfg.actor_subgoal_steps;
+    p.k_lo = cfg.low_subgoal_steps;
+    p.gc_negative = cfg.gc_negative;
+    p.stacked_next = stacked_next;
+    p.aug_mode = aug_mode;
+    p.crop_pad = crop_pad;
+    p.p_aug = p_aug;
+    p.key = make_rng_key(s->seed, s->stream_id);
+    p.batch0 = s->counter;
+    p.batch = batch;
+    p.batch_magic = batch > 1 && batch < ((int64_t)1 << 32) ? (uint64_t)(~(uint64_t)0 / (uint64_t)batch) + 1 : 0;
+    p.total_rows = total;
+    p.n_slots = spec.n_slots;
+    p.narrow = cfg.jax_compat ? 1 : 0;
+    p.vec_rows = b->vec_rows;
+    p.vec_init = b->vec_init;
+    p.crop_out = b->crop;
+
+    cudaError_t e = cudaSuccess;
+    // copies `src` (when there is one) to the block at `off` unless an earlier copy failed; returns where it went
+    auto up = [&](size_t off, const void* src, size_t bytes) -> uint8_t* {
+      if (!src || e != cudaSuccess) return nullptr;
+      e = cudaMemcpyAsync(base + off, src, bytes, cudaMemcpyHostToDevice, first);
+      return base + off;
+    };
+    if (idxs) {
+      p.given_idxs = (const int64_t*)up(off_idxs, idxs, (size_t)total * 8);
+      if (e != cudaSuccess) return fail(OGB_ERR_CUDA, "H2D of idxs failed");
+      if (defer_check) {
+        b->idx_error = (int32_t*)(base + off_idx_error);
+        if (cudaMemsetAsync(b->idx_error, 0, 4, first) != cudaSuccess) return fail(OGB_ERR_CUDA, "memset of the index flag failed");
+        p.idx_error = b->idx_error;
+        p.idx_last = idx_last;
+      }
+    }
+    if (draws) {
+      const size_t n = (size_t)batch;
+      if (!idxs) p.in_idx_pos = (const int64_t*)up(off_draw_i64[0], draws->idx_pos, n * 8);
+      for (int gs = 0; gs < 3; ++gs) {
+        if (!goal_used[gs]) continue;
+        const ogb_goal_draws& d = draws->goals[gs];
+        GoalInject& g = p.in_goal[gs];
+        g.rand_pos = (const int64_t*)up(off_draw_i64[1 + 2 * gs], d.rand_pos, n * 8);
+        g.offset = (const int64_t*)up(off_draw_i64[2 + 2 * gs], d.offset, n * 8);
+        g.dist = (const double*)up(off_draw_f64[3 * gs], d.dist, n * 8);
+        g.u_traj = (const double*)up(off_draw_f64[3 * gs + 1], d.u_traj, n * 8);
+        g.u_cur = (const double*)up(off_draw_f64[3 * gs + 2], d.u_cur, n * 8);
+      }
+      p.in_crop = (const int64_t*)up(off_draw_i64[7], draws->crop, n * 16);
+      if (spec.trl && e == cudaSuccess && !draws->trl_midpoints)
+        return fail(OGB_ERR_INVALID, "validation mode: TRL midpoint draws are missing");
+      if (spec.trl) p.in_trl_mid = (const int64_t*)up(off_trl_mid, draws->trl_midpoints, n * 8);
+      p.in_coin = draws->has_aug_coin ? draws->aug_coin : 2.0;
+      if (p.aug_mode && !(p.in_coin < p.p_aug)) p.in_crop = nullptr;
+      if (e != cudaSuccess) return fail(OGB_ERR_CUDA, "H2D of validation draws failed: %s", cudaGetErrorString(e));
+    }
+    for (size_t i = 0; i < plan.size(); ++i) {
+      if (plan[i].route != ROUTE_SCALAR) continue;
+      void* ptr = base + b->offsets[i];
+      switch (plan[i].scalar) {
+        case SC_MASKS: p.masks = (double*)ptr; break;
+        case SC_REWARDS: p.rewards = (double*)ptr; break;
+        case SC_HV_OFFSETS: p.hv_offsets = (int64_t*)ptr; break;
+        case SC_HV_STEPS: p.hv_steps = (int64_t*)ptr; break;
+        case SC_HV_MASKS: p.hv_masks = (double*)ptr; break;
+        case SC_HV_REWARDS: p.hv_rewards = (double*)ptr; break;
+        case SC_LV_STEPS: p.lv_steps = (int64_t*)ptr; break;
+        case SC_LV_MASKS: p.lv_masks = (double*)ptr; break;
+        case SC_LV_REWARDS: p.lv_rewards = (double*)ptr; break;
+        case SC_TRL_OFFSETS: p.trl_offsets = (int64_t*)ptr; break;
+        case SC_TRL_MID_OFFSETS: p.trl_mid_offsets = (int64_t*)ptr; break;
+        default: break;
+      }
+    }
+    return 0;
+  }
+  // The cp.async row gathers of the span jobs; with `fuse`, the first launch is the fused one, which also does the index
+  // algebra of `p` (and stores the index vectors when later launches read them).
+  int prepare_row_gathers(const std::vector<SpanJob>& span_jobs, bool fuse, bool inject, int flavour) {
+    using namespace ogb;
+    std::vector<RowLaunch> split;
+    OGB_TRY(split_span_jobs(span_jobs, fuse, p.kind == OGB_KIND_GC && !inject, &split));
+    for (const RowLaunch& rl : split) {
+      const bool fused_here = fuse && rl.first == 0;
+      const int n_stages = rl.shape / 100, n_warps = rl.shape % 100;
+      AsyncGatherParams ap;
+      memset(&ap, 0, sizeof(ap));
+      ap.vec_rows = b->vec_rows;
+      ap.total_rows = total;
+      ap.stage_bytes = rl.stage_bytes;
+      ap.ring_bytes = n_stages * ap.stage_bytes;
+      const size_t n_pairs = fill_row_tables(ds, plan, b->block, b->offsets, span_jobs, rl, fused_here, &ap);
+      // (a single-pair un-fused launch keeps static tiles)
+      const bool dyn_tiles = !s->static_tiles && (fused_here || n_pairs >= 2);
+      // shared memory: item table, output table, one 16-byte tile FIFO per warp, then the rings
+      ap.ring_offset = (int)round_up((size_t)ap.n_items * sizeof(ItemDesc) + (size_t)ap.n_outs * sizeof(OutDesc) + (size_t)n_warps * 16, 128);
+      const size_t smem = (size_t)ap.ring_offset + (size_t)n_warps * ap.ring_bytes;
+      if (smem > (size_t)225 * 1024)
+        return fail(OGB_ERR_UNSUPPORTED, "internal: gather shape %d needs %zu bytes of shared memory", rl.shape, smem);
+      // persistent grid: exactly the CTAs that are resident at once.  Fused: shared memory bounds them (the fused kernels
+      // are compiled for gather_min_blocks(warps) CTAs per SM, so registers allow at least that many); un-fused: what the
+      // occupancy query finds for registers and shared memory together.
+      const KernelChoice k = fused_here ? choose_fused_kernel(inject, flavour, rl.shape)
+                           : rl.shape == 310 ? async_instance<3, 10>() : async_instance<kAsyncStages, kAsyncWarps>();
+      int per_sm = (int)std::max<size_t>(1, std::min<size_t>(n_warps <= 8 ? 2 : 1, (size_t)(220 * 1024) / smem));
+      if (!fused_here) {
+        OGB_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k.fn, n_warps * 32, smem) != cudaSuccess || per_sm < 1)
+          return fail(OGB_ERR_CUDA, "gather_rows_async_kernel: occupancy query failed (%zu bytes of shared memory)", smem);
+      }
+      if (rl.first == 0) b->dominant = k.name;
       // index algebra + the first (normally the only) group of row jobs in ONE launch; the launches that take the
       // remaining jobs read the index vectors this one computes
-      if (q1 < span_jobs.size()) p.write_vecs = 1;
-      fused_writes_vecs = p.write_vecs != 0;
-      FusedParams* fp = new FusedParams();
-      fp->relabel = p;
-      fp->gather = ap;
-      std::shared_ptr<FusedParams> keep(fp);
-      const int flavour = p.kind == OGB_KIND_GC ? FLAVOUR_GC : (p.kind == OGB_KIND_HGC ? FLAVOUR_HGC : FLAVOUR_PLAIN);
-      const bool inject = draws != nullptr;
-      b->name_fused = kernel_name("relabel_gather_kernel", {inject ? 1 : 0, flavour, n_stages, n_warps});
-      fused_launch = [=](int64_t begin, int64_t end, cudaStream_t st) -> int {
+      if (fused_here && rl.end < span_jobs.size()) p.write_vecs = 1;
+      std::shared_ptr<FusedParams> keep(new FusedParams);   // (the un-fused kernel takes .gather alone)
+      if (fused_here) keep->relabel = p;
+      keep->gather = ap;
+      const char* what = fused_here ? "relabel_gather_kernel" : "gather_rows_async_kernel";
+      LaunchFn launch = [=](int64_t begin, int64_t end, cudaStream_t st) -> int {
         FusedParams& f = *keep;
         f.relabel.row_begin = f.gather.row_begin = begin;
         f.relabel.row_end = f.gather.row_end = end;
         const int64_t n_warp_tiles = (end - begin + 31) / 32;
-        const unsigned grid = (unsigned)std::min<int64_t>((n_warp_tiles + n_warps - 1) / n_warps, (int64_t)ds->sm_count * ctas_per_sm);
+        const unsigned grid = (unsigned)std::min<int64_t>((n_warp_tiles + n_warps - 1) / n_warps, (int64_t)ds->sm_count * per_sm);
         // (tickets only when there are more tiles than warps: a small launch gives every warp at most its first tile)
         f.gather.sched = dyn_tiles && n_warp_tiles > (int64_t)grid * n_warps ? s->next_sched() : nullptr;
-        // (2 x 20 and 2 x 16 are compiled for the fused GCDataset launch with Philox draws only: fused_gc)
-        const void* fn = shape == 220 ? (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 20>
-                       : shape == 216 ? (const void*)relabel_gather_kernel<false, FLAVOUR_GC, 2, 16>
-                       : flavour == FLAVOUR_GC ? (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_GC>
-                                                         : (const void*)relabel_gather_kernel<false, FLAVOUR_GC>)
-                       : flavour == FLAVOUR_HGC ? (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_HGC>
-                                                          : (const void*)relabel_gather_kernel<false, FLAVOUR_HGC>)
-                                                : (inject ? (const void*)relabel_gather_kernel<true, FLAVOUR_PLAIN>
-                                                          : (const void*)relabel_gather_kernel<false, FLAVOUR_PLAIN>);
-        if (cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (fused_here && cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
           return fail(OGB_ERR_CUDA, "cudaFuncSetAttribute(relabel_gather_kernel) failed");
-        void* args[] = {(void*)&f};
-        if (cudaLaunchKernel(fn, dim3(grid), dim3((unsigned)n_warps * 32), args, smem, st) != cudaSuccess)
-          return fail(OGB_ERR_CUDA, "relabel_gather_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        void* args[] = {fused_here ? (void*)&f : (void*)&f.gather};
+        if (cudaLaunchKernel(k.fn, dim3(grid), dim3((unsigned)n_warps * 32), args, smem, st) != cudaSuccess)
+          return fail(OGB_ERR_CUDA, "%s launch failed: %s", what, cudaGetErrorString(cudaGetLastError()));
+        if (!fused_here && cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "%s launch failed", what);
         b->launches++;
         return 0;
       };
-      continue;
+      if (fused_here) fused = launch;
+      else gathers.push_back(launch);
     }
-    const void* gather_fn = shape == 310 ? (const void*)gather_rows_async_kernel<3, 10>
-                                         : (const void*)gather_rows_async_kernel<kAsyncStages, kAsyncWarps>;
-    OGB_CUDA(cudaFuncSetAttribute(gather_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (b->name_async.empty()) b->name_async = kernel_name("gather_rows_async_kernel", {n_stages, n_warps});
-    int resident = 0;   // CTAs of this kernel that fit one SM (registers and shared memory): the persistent grid is exactly that
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, gather_fn, n_warps * 32, smem) != cudaSuccess || resident < 1)
-      return bail(fail(OGB_ERR_CUDA, "gather_rows_async_kernel: occupancy query failed (%zu bytes of shared memory)", smem));
-    gather_launches.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
-      ap.row_begin = begin;
-      ap.row_end = end;
-      const int64_t n_warp_tiles = (end - begin + 31) / 32;
-      const unsigned grid = (unsigned)std::min<int64_t>((n_warp_tiles + n_warps - 1) / n_warps, (int64_t)ds->sm_count * resident);
-      ap.sched = dyn_tiles && n_warp_tiles > (int64_t)grid * n_warps ? s->next_sched() : nullptr;
-      void* args[] = {(void*)&ap};
-      if (cudaLaunchKernel(gather_fn, dim3(grid), dim3((unsigned)n_warps * 32), args, smem, st) != cudaSuccess)
-        return fail(OGB_ERR_CUDA, "gather_rows_async_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-      if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "gather_rows_async_kernel launch failed");
-      b->launches++;
-      return 0;
-    });
+    return 0;
   }
-
-  // register-staged gather for what the asynchronous kernel does not take (very long rows)
-  if (!lsu_keys.empty()) {
-    const std::vector<size_t>& row_keys = lsu_keys;
+  // register-staged gather for what the asynchronous kernel does not take (very long rows): one launch per element width
+  // and kMaxRowJobs keys
+  int prepare_lsu_gathers(const std::vector<size_t>& row_keys) {
+    using namespace ogb;
     std::vector<int> vec_of(row_keys.size());
     for (size_t q = 0; q < row_keys.size(); ++q) {
       const Field& f = ds->fields[(size_t)plan[row_keys[q]].field];
@@ -2508,10 +2519,10 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
           if (vec_of[q] != v) continue;
           const KeyPlan& k = plan[row_keys[q]];
           const Field& f = ds->fields[(size_t)k.field];
-          if ((f.row_bytes >> v) > 65535) return bail(fail(OGB_ERR_UNSUPPORTED, "row of field '%s' too long for the row path", f.name.c_str()));
+          if ((f.row_bytes >> v) > 65535) return fail(OGB_ERR_UNSUPPORTED, "row of field '%s' too long for the row path", f.name.c_str());
           RowJob& job = gp.jobs[gp.n_jobs++];
           job.src = f.dptr;
-          job.dst = base + b->offsets[row_keys[q]];
+          job.dst = b->block + b->offsets[row_keys[q]];
           job.src_stride = (uint32_t)f.stride;
           job.row_bytes = (uint32_t)f.row_bytes;
           job.vec_log2 = (uint8_t)v;
@@ -2523,33 +2534,32 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
           job.slot = (uint8_t)k.slot;
         }
         if (gp.n_jobs == 0) break;
-        gather_launches.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
+        gathers.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
           gp.row_begin = begin;
           gp.row_end = end;
           const int64_t n_warp_tiles = (end - begin + 31) / 32;
           const unsigned grid = (unsigned)std::min<int64_t>((n_warp_tiles + 7) / 8, (int64_t)ds->sm_count * 32);
-          switch (v) {
-            case 4: gather_rows_kernel<uint4><<<grid, kRelabelThreads, 0, st>>>(gp); break;
-            case 3: gather_rows_kernel<uint2><<<grid, kRelabelThreads, 0, st>>>(gp); break;
-            case 2: gather_rows_kernel<uint32_t><<<grid, kRelabelThreads, 0, st>>>(gp); break;
-            case 1: gather_rows_kernel<uint16_t><<<grid, kRelabelThreads, 0, st>>>(gp); break;
-            default: gather_rows_kernel<uint8_t><<<grid, kRelabelThreads, 0, st>>>(gp); break;
-          }
+          static const void* const kWidth[5] = {(const void*)gather_rows_kernel<uint8_t>, (const void*)gather_rows_kernel<uint16_t>,
+              (const void*)gather_rows_kernel<uint32_t>, (const void*)gather_rows_kernel<uint2>, (const void*)gather_rows_kernel<uint4>};
+          void* args[] = {(void*)&gp};
+          (void)cudaLaunchKernel(kWidth[v], dim3(grid), dim3(kRelabelThreads), args, 0, st);   // reported below
           if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "gather_rows_kernel launch failed");
           b->launches++;
           return 0;
         });
       }
     }
+    if (!*b->dominant) b->dominant = "gather_rows_kernel";   // no row gather outranks it
+    return 0;
   }
-
-  // image keys: frame stacking + crop fused into the gather
-  bool any_frames_tma = false;
-  if (any_frames) {
+  // image keys: frame stacking + crop fused into the gather; one launch per field and stack depth
+  int prepare_frame_gathers() {
+    using namespace ogb;
     std::vector<size_t> frame_keys;
     for (size_t i = 0; i < plan.size(); ++i)
       if (plan[i].route == ROUTE_FRAMES && plan[i].alias_of < 0) frame_keys.push_back(i);
     std::vector<bool> taken(frame_keys.size(), false);
+    const char* tma_name = nullptr;   // the first TMA launch's kernel
     for (size_t a = 0; a < frame_keys.size(); ++a) {
       if (taken[a]) continue;
       const KeyPlan& ka = plan[frame_keys[a]];
@@ -2567,14 +2577,14 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         fp.H = 1; fp.W = (int)outer; fp.inner_bytes = (int)((f.ndim > 1 ? f.shape[f.ndim - 1] : 1) * f.itemsize);
       }
       // rb == 0: not a TMA shape, or no band height in (padding, 32] divides H; the generic kernel serves those
-      const int rb = tma_eligible(f, cfg, ka.fs) && crop_pad_eff <= 4 ? band_rows_for(fp.H, crop_pad_eff) : 0;
+      const int rb = tma_eligible(f, cfg, ka.fs) && crop_pad <= 4 ? band_rows_for(fp.H, crop_pad) : 0;
       for (size_t c = a; c < frame_keys.size() && fp.n_jobs < kMaxFrameJobs; ++c) {
         const KeyPlan& kc = plan[frame_keys[c]];
         if (taken[c] || kc.field != ka.field || kc.fs != ka.fs) continue;
         taken[c] = true;
         FrameJob& job = fp.jobs[fp.n_jobs++];
         job.src = f.dptr;
-        job.dst = base + b->offsets[frame_keys[c]];
+        job.dst = b->block + b->offsets[frame_keys[c]];
         job.src_row_stride = (int64_t)f.stride;
         job.slot = kc.slot;
         job.crop = kc.crop;
@@ -2584,32 +2594,27 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         fp.band_rows = rb;
         fp.n_bands = fp.H / rb;
         CUtensorMap tm;
-        int rc = get_tmap(s, ka.field, rb, &tm);
-        if (rc) return bail(rc);
+        OGB_TRY(get_tmap(s, ka.field, rb, &tm));
         const int band_bytes = rb * fp.W * 3;
         const size_t smem = (size_t)ka.fs * (ogb::frame_stride_bytes(band_bytes) + band_bytes);
-        const int fs = ka.fs;
-        any_frames_tma = true;
-        if (b->name_frames.empty()) b->name_frames = kernel_name("gather_frames_tma_kernel", {fs >= 1 && fs <= 3 ? fs : 4});
-        gather_launches.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
+        // (the last instance serves every stack deeper than three)
+        const KernelChoice k = ka.fs == 1 ? frames_instance<1>() : ka.fs == 2 ? frames_instance<2>() : ka.fs == 3 ? frames_instance<3>() : frames_instance<4>();
+        if (!tma_name) tma_name = k.name;
+        gathers.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
           fp.row_begin = begin;
           fp.row_end = end;
           const int64_t n_items = (end - begin) * fp.n_jobs * fp.n_bands;
           if (n_items > 0x7fffffff) return fail(OGB_ERR_UNSUPPORTED, "too many frame tiles in one launch");
-          int rc2;
-          switch (fs) {
-            case 1: rc2 = launch_frames_tma<1>(tm, fp, n_items, smem, st); break;
-            case 2: rc2 = launch_frames_tma<2>(tm, fp, n_items, smem, st); break;
-            case 3: rc2 = launch_frames_tma<3>(tm, fp, n_items, smem, st); break;
-            default: rc2 = launch_frames_tma<4>(tm, fp, n_items, smem, st); break;
-          }
-          if (rc2) return rc2;
+          OGB_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+          void* args[] = {(void*)&tm, (void*)&fp};
+          (void)cudaLaunchKernel(k.fn, dim3((unsigned)n_items), dim3(kFramesThreads), args, smem, st);   // reported below
+          OGB_CUDA(cudaGetLastError());
           b->launches++;
           return 0;
         });
       } else {
         const int v = largest_vec_log2((size_t)fp.inner_bytes, f.stride);
-        gather_launches.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
+        gathers.push_back([=](int64_t begin, int64_t end, cudaStream_t st) mutable -> int {
           fp.row_begin = begin;
           fp.row_end = end;
           for (int jj = 0; jj < fp.n_jobs; ++jj) {
@@ -2621,15 +2626,12 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
         });
       }
     }
+    b->dominant = tma_name ? tma_name : "gather_frames_generic_kernel";
+    return 0;
   }
-
-  // every launch after a fused one reads the index vectors from memory: the fused launch must have stored them
-  if (fused_launch && !gather_launches.empty() && !fused_writes_vecs)
-    return bail(fail(OGB_ERR_UNSUPPORTED, "internal: a fused launch followed by %zu gather launches does not store the index vectors",
-                     gather_launches.size()));
-
-  // ---- issue: index kernel on `first`, gathers on the main stream behind it ----
-  {
+  // Issues the launches row chunk by row chunk: the index kernel (or the fused launch) on `first`, the gathers on the
+  // sampler's stream behind it.
+  int issue() {
     const bool timeline = ab().timeline;   // debug: when did each phase run on the device
     auto stamp = [&](cudaStream_t st) {
       if (!timeline) return;
@@ -2638,63 +2640,175 @@ int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t 
       cudaEventRecord(ev, st);
       g_timeline.push_back(ev);
     };
-    phase.mark();   // prepare
-    // dominant kernel = the one that moves the batch's bytes: the frame gather, else the row gather (fused or not),
-    // else the index kernel itself (datasets whose rows are all <= 16 bytes)
-    b->dominant = any_frames ? (any_frames_tma ? "gather_frames_tma_kernel" : "gather_frames_generic_kernel") : fused_launch ? "relabel_gather_kernel"
-                : any_async ? "gather_rows_async_kernel" : !lsu_keys.empty() ? "gather_rows_kernel" : "relabel_index_kernel";
+    // profile mode: events around the launches `launch` makes on `st` (those of the dominant kernel)
+    auto profiled = [&](bool on, cudaStream_t st, auto&& launch) -> int {
+      if (on) {
+        cudaEventCreate(&b->prof_begin);
+        cudaEventCreate(&b->prof_end);
+        cudaEventRecord(b->prof_begin, st);
+      }
+      const int rc = launch();
+      if (!rc && on) cudaEventRecord(b->prof_end, st);
+      return rc;
+    };
     // row chunks (multiples of 32 rows, each at least kChunkMinRows): one unless the batch is headed for host memory
     constexpr int64_t kChunkMinRows = 16384;
     int n_chunks = 1;
     if (s->host_chunks > 1 && !draws && total >= 2 * kChunkMinRows) n_chunks = (int)std::min<int64_t>(std::min(s->host_chunks, kMaxChunks), total / kChunkMinRows);
     const int64_t chunk_rows = ((total + n_chunks - 1) / n_chunks + 31) / 32 * 32;
+    const bool gathers_dominate = !gathers.empty() && !fused;
     for (int c = 0; c < n_chunks; ++c) {
       const int64_t begin = (int64_t)c * chunk_rows, end = std::min<int64_t>(total, begin + chunk_rows);
       if (begin >= end) break;
+      const bool prof = s->profile && c == 0 && n_chunks == 1;
       stamp(first);
-      const bool prof_first = s->profile && c == 0 && n_chunks == 1 && (fused_launch || gather_launches.empty());
-      if (prof_first) {
-        cudaEventCreate(&b->prof_begin);
-        cudaEventCreate(&b->prof_end);
-        cudaEventRecord(b->prof_begin, first);
-      }
-      int rc = fused_launch ? fused_launch(begin, end, first) : index_launch(begin, end, first);
-      if (rc) return bail(rc);
-      if (prof_first) cudaEventRecord(b->prof_end, first);
+      int rc = profiled(prof && !gathers_dominate, first, [&] { return fused ? fused(begin, end, first) : index(begin, end, first); });
+      if (rc) return rc;
       stamp(first);
-      if (first != s->stream) {
-        cudaEvent_t ev = s->chunk_events[s->next_event];
-        s->next_event = (s->next_event + 1) % (int)s->chunk_events.size();
-        if (cudaEventRecord(ev, first) != cudaSuccess || cudaStreamWaitEvent(s->stream, ev, 0) != cudaSuccess)
-          return bail(fail(OGB_ERR_CUDA, "stream join failed"));
-      }
+      if (first != s->stream && join_streams(s, first, s->stream)) return fail(OGB_ERR_CUDA, "stream join failed");
       stamp(s->stream);
-      const bool prof_gathers = s->profile && c == 0 && n_chunks == 1 && !gather_launches.empty() && !fused_launch;
-      if (prof_gathers) {
-        cudaEventCreate(&b->prof_begin);
-        cudaEventCreate(&b->prof_end);
-        cudaEventRecord(b->prof_begin, s->stream);
-      }
-      for (size_t q = 0; q < gather_launches.size() && !rc; ++q) rc = gather_launches[q](begin, end, s->stream);
-      if (rc) return bail(rc);
-      if (prof_gathers) cudaEventRecord(b->prof_end, s->stream);
+      rc = profiled(prof && gathers_dominate, s->stream, [&] {
+        int r = 0;
+        for (size_t q = 0; q < gathers.size() && !r; ++q) r = gathers[q](begin, end, s->stream);
+        return r;
+      });
+      if (rc) return rc;
       stamp(s->stream);
       if (n_chunks > 1) {
         cudaEvent_t done;
         if (cudaEventCreateWithFlags(&done, cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(done, s->stream) != cudaSuccess)
-          return bail(fail(OGB_ERR_CUDA, "chunk event failed"));
+          return fail(OGB_ERR_CUDA, "chunk event failed");
         b->chunk_done.push_back(done);
         b->chunk_end.push_back(end);
       }
     }
+    return 0;
+  }
+};
+
+int run_sample(ogb_sampler* s, const RunSpec& spec, int64_t batch_size, int32_t n_batches, const int64_t* idxs, int32_t evaluation,
+               const ogb_draws* draws, ogb_batch** out) {
+  PhaseClock phase;
+  if (!s || !out) return fail(OGB_ERR_INVALID, "ogb_sampler_sample: null argument");
+  const ogb_dataset* ds = s->ds;
+  Run r{s, ds, s->cfg, spec, *spec.plan, batch_size, batch_size * (int64_t)n_batches, n_batches, idxs, draws};
+  OGB_TRY(r.check(evaluation != 0));
+  DeviceGuard device_guard(ds->device);
+  OGB_CUDA(device_guard.status);
+  std::lock_guard<std::mutex> lock(s->mu);
+  phase.mark();   // checks
+
+  bool any_frames = false, any_long = false, any_async = false;   // image keys; row keys over 16 bytes, and on the cp.async path
+  for (const KeyPlan& k : r.plan) {
+    if (k.alias_of >= 0) continue;
+    any_frames |= k.route == ROUTE_FRAMES;
+    if (k.route != ROUTE_ROW || ds->fields[(size_t)k.field].row_bytes <= 16) continue;
+    any_long = true;
+    any_async |= async_reachable(ds, ds->fields[(size_t)k.field]);
+  }
+  const bool want_init = any_frames && s->cfg.frame_stack > 1;
+  r.new_batch(want_init, any_frames);
+  ogb_batch* b = r.b;
+  auto bail = [&](int code) { batch_unref(b); return code; };
+  // When some key goes through the cp.async row gather, the index algebra is fused into that launch (one kernel per
+  // sample() for vector observations); otherwise the index kernel runs on its own.
+  // Measured on B200 with ~1M-row launches: fused wins for GCDataset shapes (C2 0.201 vs 0.216 ms, C5 0.356 vs 0.372)
+  // and loses for the heavier HGC algebra with its 16-row items (C3 0.757 vs 0.730 ms), so big HGC launches stay split;
+  // small launches always fuse (one kernel launch less).  Image batches keep the index kernel apart (it overlaps the
+  // previous call's frame gathers).  OGB_FUSE=0/1 forces either.
+  const int fuse_env = ab().fuse;
+  bool fuse = any_async && (fuse_env >= 0 ? fuse_env != 0 : (!any_frames && (r.total < kOverlapMinRows || spec.kind != OGB_KIND_HGC)));
+  // Phase-one work (uploads of validation draws, the index kernel) goes to `first`: for big launches that is the
+  // auxiliary stream, so that the index kernel of this call overlaps the gathers of the previous call, which are
+  // still running on the main stream.  The recycled block only has to wait for its own previous owner.
+  // Image batches are few rows with long gathers: their (latency-bound) index kernel always goes to the auxiliary
+  // stream, where it runs under the frame gathers of the previous call.
+  // (any_frames || any_long: is there a gather launch for the index kernel to hide under?)
+  const bool use_aux = !fuse && (any_frames || any_long) && (r.total >= kOverlapMinRows || any_frames);
+  if (use_aux) {
+    int rc = ensure_aux(s);
+    if (rc) return bail(rc);
+  }
+  cudaStream_t first = r.first = use_aux ? s->aux_stream : s->stream;
+  phase.mark();   // batch + layout
+  {
+    std::vector<cudaEvent_t> free_after;
+    int rc = block_take(s, b->block_bytes, &b->block, &b->block_bytes, &free_after);
+    for (cudaEvent_t ev : free_after) {
+      cudaStreamWaitEvent(first, ev, 0);
+      if (first != s->stream) cudaStreamWaitEvent(s->stream, ev, 0);
+      cudaEventDestroy(ev);
+    }
+    if (rc) return bail(rc);
+  }
+  uint8_t* base = b->block;
+  phase.mark();   // block
+  if (s->canary) {
+    cudaMemsetAsync(base, 0xA5, b->block_bytes, first);
+    // the gathers on the main stream must not start before the fill has finished
+    if (first != s->stream) join_streams(s, first, s->stream);
+  }
+  b->vec_rows = (int32_t*)(base + r.off_rows);
+  if (any_frames) b->crop = (int8_t*)(base + r.off_crop);
+  if (want_init) b->vec_init = (int32_t*)(base + r.off_init);
+  if (r.total > 0) {   // an empty batch is legal (np.random.randint(n, size=0) in the reference): every key with zero rows, no launch
+    ogb::RelabelParams& p = r.p;
+    int rc = r.fill_params();
+    if (rc) return bail(rc);
+    phase.mark();   // params
+    std::vector<size_t> lsu_keys;
+    const std::vector<SpanJob> spans = classify_rows(ds, r.plan, base, b->offsets, &p, &lsu_keys);
+    fuse = fuse && !spans.empty();
+    const bool any_gather = !spans.empty() || !lsu_keys.empty() || any_frames;   // a launch after the index kernel
+    const bool point_record = is_point_record(s, spec, p, any_gather);
+    // the index vectors only go to memory when a later launch (or the debug interface) reads them; a fused launch that
+    // leaves span jobs to a second row-gather launch sets it in prepare_row_gathers, where the launch split is known
+    p.write_vecs = ((!fuse && !spans.empty()) || !lsu_keys.empty() || any_frames || s->debug) ? 1 : 0;
+    phase.mark();   // classify
+    // Every launch.  Each family names the dominant kernel -- the one that moves the batch's bytes -- as it is prepared, in
+    // rising precedence: the row gather (fused or not), the register-staged one, the frame gather; when there is none of
+    // them, the index kernel names itself as it launches (datasets whose rows are all <= 16 bytes).  (The index launch
+    // takes the parameters as they are: they change only for a fused launch, which replaces it.)
+    const int flavour = spec.kind == OGB_KIND_GC ? ogb::FLAVOUR_GC : (spec.kind == OGB_KIND_HGC ? ogb::FLAVOUR_HGC : ogb::FLAVOUR_PLAIN);
+    r.index = index_launch(s, b, p, draws != nullptr, flavour, point_record, !any_gather);
+    rc = r.prepare_row_gathers(spans, fuse, draws != nullptr, flavour);
+    if (!rc && !lsu_keys.empty()) rc = r.prepare_lsu_gathers(lsu_keys);
+    if (!rc && any_frames) rc = r.prepare_frame_gathers();
+    // every launch after a fused one reads the index vectors from memory: the fused launch must have stored them
+    if (!rc && r.fused && !r.gathers.empty() && !p.write_vecs)
+      rc = fail(OGB_ERR_UNSUPPORTED, "internal: a fused launch followed by %zu gather launches does not store the index vectors",
+                r.gathers.size());
+    if (rc) return bail(rc);
+    phase.mark();   // prepare
+    rc = r.issue();
+    if (rc) return bail(rc);
   }
   if (cudaEventCreateWithFlags(&b->ready, cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(b->ready, s->stream) != cudaSuccess)
     return bail(fail(OGB_ERR_CUDA, "ready event failed"));
   if (!draws) s->counter += (uint64_t)n_batches;
   *out = b;
+  if (r.total == 0) return 0;
   phase.mark();   // launch + event
   if (g_phases.on) ++g_phases.calls;
   return 0;
+}
+
+// One key of rows `idxs`: the observations -- cropped with the injected shifts and `crop_padding` when that is >= 0 -- or
+// the goal observations (get_observations, get_goal_observations, augment).
+int run_rows(ogb_sampler* s, bool goal, int crop_padding, const int64_t* idxs, int64_t n, const ogb_draws* draws, ogb_batch** out) {
+  PlanBuilder pb;
+  pb.ds = s->ds;
+  pb.cfg = &s->cfg;
+  pb.crop_possible = crop_padding >= 0;
+  for (int v = 0; v < ogb::kMaxSlots; ++v) pb.slot_canon[v] = v;
+  if (goal) pb.goal_key("goal_observations", ogb::SLOT_IDX, false);
+  else pb.obs_key("observations", ogb::SLOT_IDX, crop_padding >= 0);
+  RunSpec spec;
+  spec.kind = OGB_KIND_PLAIN;
+  spec.plan = &pb.keys;
+  spec.n_slots = 2;
+  spec.crop_padding = crop_padding;
+  return run_sample(s, spec, n, 1, idxs, draws ? 0 : 1, draws, out);
 }
 
 }  // namespace
@@ -2724,20 +2838,8 @@ int ogb_sampler_gather(ogb_sampler* s, int32_t which, const int64_t* idxs, int64
   static const int64_t no_rows = 0;
   if (n == 0) idxs = &no_rows;   // an empty gather is legal (observations[np.zeros(0, int)]); run_sample wants a non-null pointer
   if (which < 0 || which > 1) return fail(OGB_ERR_INVALID, "which must be 0 (observations) or 1 (goal observations)");
-  PlanBuilder pb;
-  pb.ds = s->ds;
-  pb.cfg = &s->cfg;
-  pb.crop_possible = false;
-  for (int v = 0; v < ogb::kMaxSlots; ++v) pb.slot_canon[v] = v;
-  if (which == 0) pb.obs_key("observations", ogb::SLOT_IDX, false);
-  else pb.goal_key("goal_observations", ogb::SLOT_IDX, false);
-  RunSpec spec;
-  spec.kind = OGB_KIND_PLAIN;
-  spec.plan = &pb.keys;
-  spec.n_slots = 2;
-  const int fs = s->cfg.frame_stack;
-  if (fs > 0 && s->term_host.empty()) return fail(OGB_ERR_INVALID, "frame stacking needs trajectory boundaries");
-  return run_sample(s, spec, n, 1, idxs, 1, nullptr, out);
+  if (s->cfg.frame_stack > 0 && s->term_host.empty()) return fail(OGB_ERR_INVALID, "frame stacking needs trajectory boundaries");
+  return run_rows(s, which == 1, -1, idxs, n, nullptr, out);
 } OGB_CATCH_ALL
 
 // GCDataset.augment (datasets.py:329-339) for one image array: rows `idxs` of the observations, each cropped with its
@@ -2748,23 +2850,12 @@ int ogb_sampler_gather_cropped(ogb_sampler* s, const int64_t* idxs, int64_t n, c
   if (padding > 127) return fail(OGB_ERR_INVALID, "crop padding %d out of [0, 127]", padding);   // int8 shifts, as in ogb_sampler_create
   for (int64_t r = 0; r < 2 * n; ++r)
     if (crop[r] < 0 || crop[r] > 2 * (int64_t)padding) return fail(OGB_ERR_INVALID, "crop shift out of [0, 2 * padding]");
-  PlanBuilder pb;
-  pb.ds = s->ds;
-  pb.cfg = &s->cfg;
-  pb.crop_possible = true;
-  for (int v = 0; v < ogb::kMaxSlots; ++v) pb.slot_canon[v] = v;
-  pb.obs_key("observations", ogb::SLOT_IDX, true);
-  RunSpec spec;
-  spec.kind = OGB_KIND_PLAIN;
-  spec.plan = &pb.keys;
-  spec.n_slots = 2;
-  spec.crop_padding = padding;
   ogb_draws d;
   memset(&d, 0, sizeof(d));
   d.has_aug_coin = 1;
   d.aug_coin = 0.0;
   d.crop = crop;
-  return run_sample(s, spec, n, 1, idxs, 0, &d, out);
+  return run_rows(s, false, padding, idxs, n, &d, out);
 } OGB_CATCH_ALL
 
 }  // extern "C"
@@ -2836,7 +2927,7 @@ int ogb_sampler_sample_goals(ogb_sampler* s, const int64_t* idxs, int64_t n, dou
   for (int64_t r = 0; r < n; ++r)
     if (idxs[r] < 0 || idxs[r] >= ds->size) return fail(OGB_ERR_INDEX, "index %lld is out of bounds for axis 0 with size %lld", (long long)idxs[r], (long long)ds->size);
   const bool cur_only = p_curgoal == 1.0;
-  const int64_t n_choices = s->trl_rows.dev ? (int64_t)s->trl_rows.host.size() : (ds->valid_mode == 0 ? ds->active_rows : ds->n_valid);
+  const int64_t n_choices = n_choices_for(ds, s->trl_rows.dev, (int64_t)s->trl_rows.host.size());
   if (draws) {
     if (!draws->rand_pos || (geom_sample ? !draws->offset : !draws->dist) || (!cur_only && (!draws->u_traj || !draws->u_cur)))
       return fail(OGB_ERR_INVALID, "sample_goals: missing draws");
@@ -2849,36 +2940,9 @@ int ogb_sampler_sample_goals(ogb_sampler* s, const int64_t* idxs, int64_t n, dou
   GoalsParams q;
   memset(&q, 0, sizeof(q));
   RelabelParams& p = q.r;
-  p.term = s->d_term;
-  p.term_bucket = s->d_term_bucket;
-  p.term_shift = s->term_shift;
-  p.valid_table = s->trl_rows.dev ? s->trl_rows.dev : ds->d_valid_table;
-  p.gap_c = ds->d_gap_c;
-  p.gap_bucket = ds->d_gap_bucket;
-  p.gap_shift = ds->gap_shift;
-  p.valid_mode = s->trl_rows.dev ? 1 : ds->valid_mode;
-  if (!s->trl_rows.dev && s->seg_shift >= 0) {
-    p.valid_mode = 3;
-    p.seg_table = s->d_seg_table;
-    p.seg_bucket = s->d_seg_bucket;
-    p.seg_shift = s->seg_shift;
-  }
-  p.n_choices = n_choices;
+  set_row_tables(s, s->trl_rows.dev, n_choices, &p);
   p.n_rows_ds = (int32_t)ds->size;
-  GoalSpec& spec = p.goal[0];
-  spec.geom = geom_sample != 0;
-  spec.cur_only = cur_only;
-  spec.p_cur = p_curgoal;
-  spec.thr_traj = cur_only ? 0.0 : p_trajgoal / (1.0 - p_curgoal);
-  spec.log_1mp = std::log(1.0 - (1.0 - discount));
-  spec.geo_abs_margin = (float)(1.5e-8 / std::fabs(spec.log_1mp));
-  auto word_threshold = [](double prob, uint32_t* thr, uint8_t* always) {
-    const double t = std::ceil(prob * 4294967296.0);
-    *always = t >= 4294967296.0 ? 1 : 0;
-    *thr = t <= 0.0 ? 0u : (t >= 4294967296.0 ? 0xFFFFFFFFu : (uint32_t)t);
-  };
-  word_threshold(spec.thr_traj, &spec.thr_traj32, &spec.traj_always);
-  word_threshold(spec.p_cur, &spec.thr_cur32, &spec.cur_always);
+  p.goal[0] = goal_spec(p_curgoal, p_trajgoal, geom_sample != 0, discount);
   p.key = make_rng_key(s->seed, s->stream_id);
   p.batch0 = s->counter;
   DeviceScratch tmp;
@@ -3047,14 +3111,7 @@ int ogb_batch_launches(const ogb_batch* b, int32_t* out) try {
 } OGB_CATCH_ALL
 int ogb_batch_dominant_kernel(ogb_batch* b, const char** name, float* ms) try {
   if (!b || !name || !ms) return fail(OGB_ERR_INVALID, "null argument");
-  {
-    const std::string d = b->dominant;
-    const std::string& full = d == "gather_frames_tma_kernel" ? b->name_frames
-                            : d == "relabel_gather_kernel" ? b->name_fused
-                            : d == "gather_rows_async_kernel" ? b->name_async : d == "relabel_index_kernel" ? b->name_index : d;
-    b->dominant_full = full.empty() ? d : full;
-  }
-  *name = b->dominant_full.c_str();
+  *name = b->dominant;
   *ms = -1.0f;
   if (b->prof_begin && b->prof_end) {
     OGB_CUDA(cudaEventSynchronize(b->prof_end));

@@ -1,5 +1,6 @@
 """Row gathers (every vector key of GCDataset, HGCDataset, TRL and Dataset.sample) against plain references, at every row
-size class, drain kind, rows-per-item value and launch split of the host planner (`run_sample`, ogb_sampler.cu).
+size class, drain kind, rows-per-item value and launch split of the host planner (`classify_rows`, `split_span_jobs` and
+`fill_row_tables`, ogb_sampler.cu).
 
 `RowPlan` below restates the planner in Python: the record layout of `ogb_dataset_create`, the key plan, tiny versus span
 fields and span merging, stage budget and rows per item, the launch split, the drain kind of every output, fused versus
@@ -209,7 +210,7 @@ class Span:
 
 
 class RowPlan:
-    """run_sample's classification and launch plan for one sample() call of `total` rows (no image keys)."""
+    """classify_rows and split_span_jobs for one sample() call of `total` rows (no image keys)."""
 
     def __init__(self, fields, kind, config=None, total=1, dedup=True, env=None, philox=True, host_chunks=1):
         env = env or {}
