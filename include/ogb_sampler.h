@@ -181,6 +181,17 @@ int ogb_sampler_write_ring(ogb_sampler* s, int64_t row0, int64_t n, int64_t skip
 /* The CUDA stream the sampler launches on (a DLPack producer orders its writes before it: __dlpack__(stream=...)). */
 int ogb_sampler_get_stream(const ogb_sampler* s, void** out);
 int ogb_sampler_copy_bounds(const ogb_sampler* s, int64_t* terminal_locs, int64_t* initial_locs); /* host out */
+/* Debug: the start-row and trajectory tables sample() reads (read-only; changes nothing). */
+typedef struct {
+  int32_t valid_mode;        /* 0 no 'valids', 1 explicit row table (also TRL rows), 2 gap ranks, 3 one-probe segment table */
+  int32_t seg_shift;         /* bucket width log2 of the segment table, -1 when it was refused */
+  int32_t n_seg_table;       /* its entries (16 bytes each) */
+  int32_t gap_shift;         /* bucket width log2 of the gap-rank search */
+  int32_t term_shift;        /* bucket width log2 of the terminal search */
+  int32_t pad_;
+  int64_t n_choices;         /* len(valid_idxs) as this sampler sees it */
+} ogb_table_info;
+int ogb_sampler_table_info(const ogb_sampler* s, ogb_table_info* info);
 int ogb_sampler_get_counter(const ogb_sampler* s, uint64_t* out); /* checkpointable RNG position */
 int ogb_sampler_set_counter(ogb_sampler* s, uint64_t counter);
 int ogb_sampler_destroy(ogb_sampler* s);
@@ -223,6 +234,10 @@ int ogb_batch_keep_leading_axis(ogb_batch* b, int32_t on);        /* shapes keep
 int ogb_batch_nbytes(const ogb_batch* b, size_t* out);            /* size of the single device block */
 int ogb_batch_device_block(const ogb_batch* b, void** out);       /* its base: key i lives at base + ogb_key_info.offset */
 int ogb_batch_launches(const ogb_batch* b, int32_t* out);         /* kernels launched to produce it */
+int ogb_batch_kernel_names(const ogb_batch* b, const char** buf, int32_t cap, int32_t* n_out);
+                                                                  /* debug: the kernel of every launch, in issue order, named as
+                                                                     ogb_batch_dominant_kernel names them (static strings); the
+                                                                     first min(cap, n) go to buf, *n_out = n */
 int ogb_batch_dominant_kernel(ogb_batch* b, const char** name, float* ms); /* the kernel that moved the batch's bytes, named with its
                                                                      template arguments as ncu prints them (the string lives
                                                                      as long as the batch), and, in profile mode, its device

@@ -63,6 +63,11 @@ class KeyInfo(C.Structure):
                 ('device_ptr', C.c_void_p), ('nbytes', C.c_size_t), ('offset', C.c_size_t), ('alias_of', C.c_int32)]
 
 
+class TableInfo(C.Structure):
+    _fields_ = [('valid_mode', C.c_int32), ('seg_shift', C.c_int32), ('n_seg_table', C.c_int32), ('gap_shift', C.c_int32),
+                ('term_shift', C.c_int32), ('pad_', C.c_int32), ('n_choices', C.c_int64)]
+
+
 class NativeError(RuntimeError):
     pass
 
@@ -98,6 +103,7 @@ SIGNATURES = [
                                          C.POINTER(C.c_int32), _P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     ('ogb_sampler_get_stream', C.c_int, [_P, C.POINTER(_P)]),
     ('ogb_sampler_copy_bounds', C.c_int, [_P, _P, _P]),
+    ('ogb_sampler_table_info', C.c_int, [_P, C.POINTER(TableInfo)]),
     ('ogb_sampler_get_counter', C.c_int, [_P, C.POINTER(C.c_uint64)]),
     ('ogb_sampler_set_counter', C.c_int, [_P, C.c_uint64]),
     ('ogb_sampler_destroy', C.c_int, [_P]),
@@ -114,6 +120,7 @@ SIGNATURES = [
     ('ogb_batch_nbytes', C.c_int, [_P, C.POINTER(C.c_size_t)]),
     ('ogb_batch_device_block', C.c_int, [_P, C.POINTER(_P)]),
     ('ogb_batch_launches', C.c_int, [_P, C.POINTER(C.c_int32)]),
+    ('ogb_batch_kernel_names', C.c_int, [_P, C.POINTER(C.c_char_p), C.c_int32, C.POINTER(C.c_int32)]),
     ('ogb_batch_dominant_kernel', C.c_int, [_P, _P, _P]),
     ('ogb_batch_keep_leading_axis', C.c_int, [_P, C.c_int32]),
     ('ogb_batch_sync', C.c_int, [_P]),

@@ -547,6 +547,7 @@ struct ogb_batch {
   cudaEvent_t prof_begin = nullptr, prof_end = nullptr;   // profile mode: brackets of the dominant kernel
   const char* dominant = "";                               // its name, with the template arguments ncu prints, e.g.
                                                            // "relabel_gather_kernel<0, 0, 2, 20>" (static storage)
+  std::vector<const char*> kernel_names;                   // every launch's kernel, in issue order (static storage)
   cudaEvent_t ready = nullptr;
   cudaEvent_t copied = nullptr;                            // ogb_batch_copy_to_host_begin: the D2H copy of the block has finished
   volatile int32_t* h_idx_flag = nullptr;                  // ... and where the deferred index flag lands (pinned, sampler-owned)
@@ -2208,6 +2209,7 @@ LaunchFn index_launch(ogb_sampler* s, ogb_batch* b, const ogb::RelabelParams& pa
       return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "relabel_index_kernel launch failed");
     if (dominant) b->dominant = k.name;
+    b->kernel_names.push_back(k.name);
     b->launches++;
     return 0;
   };
@@ -2491,6 +2493,7 @@ struct Run {
         if (cudaLaunchKernel(k.fn, dim3(grid), dim3((unsigned)n_warps * 32), args, smem, st) != cudaSuccess)
           return fail(OGB_ERR_CUDA, "%s launch failed: %s", what, cudaGetErrorString(cudaGetLastError()));
         if (!fused_here && cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "%s launch failed", what);
+        b->kernel_names.push_back(k.name);
         b->launches++;
         return 0;
       };
@@ -2544,6 +2547,7 @@ struct Run {
           void* args[] = {(void*)&gp};
           (void)cudaLaunchKernel(kWidth[v], dim3(grid), dim3(kRelabelThreads), args, 0, st);   // reported below
           if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "gather_rows_kernel launch failed");
+          b->kernel_names.push_back("gather_rows_kernel");
           b->launches++;
           return 0;
         });
@@ -2609,6 +2613,7 @@ struct Run {
           void* args[] = {(void*)&tm, (void*)&fp};
           (void)cudaLaunchKernel(k.fn, dim3((unsigned)n_items), dim3(kFramesThreads), args, smem, st);   // reported below
           OGB_CUDA(cudaGetLastError());
+          b->kernel_names.push_back(k.name);
           b->launches++;
           return 0;
         });
@@ -2620,6 +2625,7 @@ struct Run {
           for (int jj = 0; jj < fp.n_jobs; ++jj) {
             gather_frames_generic_kernel<<<ds->sm_count * 8, 256, 0, st>>>(fp, jj, v);
             if (cudaGetLastError() != cudaSuccess) return fail(OGB_ERR_CUDA, "gather_frames_generic_kernel launch failed");
+            b->kernel_names.push_back("gather_frames_generic_kernel");
             b->launches++;
           }
           return 0;
@@ -2917,6 +2923,22 @@ struct DeviceScratch {   // a few temporary device arrays of a helper call
 
 extern "C" {
 
+int ogb_sampler_table_info(const ogb_sampler* s, ogb_table_info* info) try {
+  if (!s || !info) return fail(OGB_ERR_INVALID, "ogb_sampler_table_info: null argument");
+  const int64_t n_choices = n_choices_for(s->ds, s->trl_rows.dev, (int64_t)s->trl_rows.host.size());
+  ogb::RelabelParams p;
+  memset(&p, 0, sizeof(p));
+  set_row_tables(s, s->trl_rows.dev, n_choices, &p);
+  memset(info, 0, sizeof(*info));
+  info->valid_mode = p.valid_mode;
+  info->seg_shift = s->seg_shift;
+  info->n_seg_table = s->n_seg_table;
+  info->gap_shift = s->ds->gap_shift;
+  info->term_shift = s->term_shift;
+  info->n_choices = n_choices;
+  return 0;
+} OGB_CATCH_ALL
+
 int ogb_sampler_sample_goals(ogb_sampler* s, const int64_t* idxs, int64_t n, double p_curgoal, double p_trajgoal, int32_t geom_sample,
                              double discount, const ogb_goal_draws* draws, int64_t* out_goal_idxs) try {
   using namespace ogb;
@@ -3107,6 +3129,12 @@ int ogb_batch_device_block(const ogb_batch* b, void** out) try {
 int ogb_batch_launches(const ogb_batch* b, int32_t* out) try {
   if (!b || !out) return fail(OGB_ERR_INVALID, "null argument");
   *out = b->launches;
+  return 0;
+} OGB_CATCH_ALL
+int ogb_batch_kernel_names(const ogb_batch* b, const char** buf, int32_t cap, int32_t* n_out) try {
+  if (!b || !n_out || cap < 0 || (!buf && cap > 0)) return fail(OGB_ERR_INVALID, "ogb_batch_kernel_names: bad argument");
+  *n_out = (int32_t)b->kernel_names.size();
+  for (int32_t i = 0; i < cap && i < *n_out; ++i) buf[i] = b->kernel_names[(size_t)i];
   return 0;
 } OGB_CATCH_ALL
 int ogb_batch_dominant_kernel(ogb_batch* b, const char** name, float* ms) try {

@@ -39,15 +39,15 @@ def test_struct_layouts_match_header():
     import subprocess
     import tempfile
 
-    src = '#include <stdio.h>\n#include "ogb_sampler.h"\nint main(){printf("%zu %zu %zu %zu %zu\\n", sizeof(ogb_field), ' \
-          'sizeof(ogb_config), sizeof(ogb_goal_draws), sizeof(ogb_draws), sizeof(ogb_key_info));return 0;}\n'
+    src = '#include <stdio.h>\n#include "ogb_sampler.h"\nint main(){printf("%zu %zu %zu %zu %zu %zu\\n", sizeof(ogb_field), ' \
+          'sizeof(ogb_config), sizeof(ogb_goal_draws), sizeof(ogb_draws), sizeof(ogb_key_info), sizeof(ogb_table_info));return 0;}\n'
     with tempfile.TemporaryDirectory() as tmp:
         c = os.path.join(tmp, 'sz.c')
         open(c, 'w').write(src)
         exe = os.path.join(tmp, 'sz')
         subprocess.check_call(['gcc', '-I', os.path.join(ROOT, 'include'), c, '-o', exe])
         sizes = list(map(int, subprocess.check_output([exe]).split()))
-    mirrors = [_native.Field, _native.Config, _native.GoalDraws, _native.Draws, _native.KeyInfo]
+    mirrors = [_native.Field, _native.Config, _native.GoalDraws, _native.Draws, _native.KeyInfo, _native.TableInfo]
     assert sizes == [ctypes.sizeof(m) for m in mirrors]
 
 
