@@ -10,6 +10,8 @@ thread while the current one is being sampled, so the swap every `dataset_replac
 shard is a view of it (the dataset the shard's file would give) and the whole table is the concatenated dataset.
 `upload_dataset` gives load_dataset's result in HBM without the host copy: the file is inflated, cast, laid out and
 written a block at a time, which is also how ResidentShards reads its files with the default loader.
+`upload_datasets` does the same for `make_datasets`, whose '-oraclerep-' and 'singletask' relabellings are row-local
+and run per block.
 """
 
 from __future__ import annotations
@@ -18,13 +20,14 @@ import ast
 import atexit
 import contextlib
 import ctypes as C
+import functools
 import glob
 import queue
 import threading
 import weakref
 import zipfile
 from collections.abc import Mapping
-from typing import Any, Callable, List, Optional
+from typing import Any, Callable, List, NamedTuple, Optional, Tuple
 
 import numpy as np
 
@@ -70,6 +73,109 @@ def load_dataset(dataset_path, ob_dtype=np.float32, action_dtype=np.float32, com
     return dataset
 
 
+class _Relabelling(NamedTuple):
+    """A relabelling with its constants resolved: `rows(info)` maps rows of the info members `members` ({'qpos': rows,
+    'button_states': rows}) to the same rows of the derived fields.  Every expression is row-local, so the whole arrays
+    and any block of their rows give the same elements."""
+    members: Tuple[str, ...]
+    rows: Callable[[Mapping], dict]
+
+
+def _oracle_relabelling(env_name, env, num_cubes=None, num_buttons=None) -> _Relabelling:
+    """add_oracle_reps' constants for `env_name`, read once, and its per-row arithmetic (ogbench/relabel_utils.py:93-155)."""
+    def count(attr, given):
+        return given if given is not None else getattr(env.unwrapped, attr)
+
+    obj0, cube_len = 14, 7
+    xyz_center = np.array([0.425, 0.0, 0.0])
+    if 'maze' in env_name or 'soccer' in env_name:
+        start = 0 if 'maze' in env_name else 15            # agent xy, or the ball's xy for antsoccer
+        members = ('qpos',)
+    elif 'cube' in env_name or 'scene' in env_name or 'puzzle' in env_name:
+        if 'puzzle' in env_name:
+            members = ('button_states',)
+        else:
+            n_cubes = count('_num_cubes', num_cubes)
+            if 'cube' in env_name:
+                members = ('qpos',)
+            else:
+                drawer = obj0 + n_cubes * cube_len + count('_num_buttons', num_buttons)
+                members = ('qpos', 'button_states')
+    else:
+        raise ValueError(f'Unsupported environment: {env_name}')
+
+    def rows(info):
+        if 'maze' in env_name or 'soccer' in env_name:
+            oracle_reps = info['qpos'][:, start:start + 2]
+        elif 'puzzle' in env_name:
+            oracle_reps = info['button_states'].copy()
+        else:
+            qpos = info['qpos']
+            cube_xyzs = np.stack([qpos[:, obj0 + i * cube_len:obj0 + i * cube_len + 3] for i in range(n_cubes)], axis=1)
+            cube_reps = ((cube_xyzs - xyz_center) * 10.0).reshape(-1, n_cubes * 3)
+            if 'cube' in env_name:
+                oracle_reps = cube_reps
+            else:
+                oracle_reps = np.concatenate(
+                    [cube_reps, info['button_states'].copy(), qpos[:, [drawer]] * 18.0, qpos[:, [drawer + 1]] * 15.0], axis=-1)
+        return {'oracle_reps': oracle_reps.astype(np.float32)}
+
+    return _Relabelling(members, rows)
+
+
+def _task_relabelling(env_name, env) -> _Relabelling:
+    """relabel_dataset's constants for `env_name`, read from the single-task `env` after its reset, and its per-row
+    arithmetic (ogbench/relabel_utils.py:4-90)."""
+    task = env.unwrapped
+    assert task._reward_task_id is not None, 'The environment is not in the single-task mode.'
+    env.reset()
+    tol = 0.04                                              # object / drawer / window tolerance of the manipulation tasks
+    obj0, cube_len = 14, 7
+    maze = 'maze' in env_name or 'soccer' in env_name
+    cubes = 'cube' in env_name or 'scene' in env_name
+    scene = 'scene' in env_name and 'cube' not in env_name
+    puzzle = 'puzzle' in env_name and 'cube' not in env_name and 'scene' not in env_name
+    if maze:
+        first = 0 if 'maze' in env_name else 15             # the agent's xy, or the ball's for antsoccer
+        goal_xy, goal_tol = task.cur_goal_xy, task._goal_tol
+        members = ('qpos',)
+    elif cubes or 'puzzle' in env_name:
+        if cubes:
+            n_cubes, mocap_pos = task._num_cubes, task._data.mocap_pos.copy()
+        if scene:
+            drawer = obj0 + task._num_cubes * cube_len + task._num_buttons
+        if scene or puzzle:
+            target_buttons = task._target_button_states.copy()
+        if scene:
+            target_drawer, target_window = task._target_drawer_pos, task._target_window_pos
+        members = ('qpos',) * cubes + ('button_states',) * (scene or puzzle)
+    else:
+        raise ValueError(f'Unsupported environment: {env_name}')
+
+    def rows(info):
+        if maze:
+            gap = np.linalg.norm(info['qpos'][:, first:first + 2] - goal_xy, axis=-1)
+            reached = (gap <= goal_tol).astype(np.float32)
+            rewards, masks = reached - 1.0, 1.0 - reached   # -1 until the goal is reached; the episode stops mattering there
+        else:
+            done = []                                       # one boolean column per sub-goal of the task
+            if cubes:
+                xyz = np.stack([info['qpos'][:, obj0 + c * cube_len:obj0 + c * cube_len + 3] for c in range(n_cubes)], axis=1)
+                done.append(np.linalg.norm(mocap_pos - xyz, axis=-1) <= tol)
+            if scene:
+                done.append(info['button_states'] == target_buttons)
+                done.append((np.abs(info['qpos'][:, drawer] - target_drawer) <= tol)[:, None])
+                done.append((np.abs(info['qpos'][:, drawer + 1] - target_window) <= tol)[:, None])
+            if puzzle:
+                done.append(info['button_states'] == target_buttons)
+            done = np.concatenate(done, axis=-1)
+            rewards = done.sum(axis=-1) - done.shape[-1]    # minus the number of unfinished sub-goals
+            masks = 1.0 - np.all(done, axis=-1)
+        return {'rewards': rewards.astype(np.float32), 'masks': masks.astype(np.float32)}
+
+    return _Relabelling(members, rows)
+
+
 def add_oracle_reps(env_name, env, dataset, num_cubes=None, num_buttons=None):
     """Add oracle goal representations to the dataset (same contract as ogbench/relabel_utils.py:93-155).
 
@@ -77,31 +183,7 @@ def add_oracle_reps(env_name, env, dataset, num_cubes=None, num_buttons=None):
     `env.unwrapped._num_cubes` / `_num_buttons`); the dataset must have been loaded with add_info=True ('qpos',
     'button_states').  The sampler then serves goals from `oracle_reps` (datasets.py:348-357).
     """
-    def count(attr, given):
-        return given if given is not None else getattr(env.unwrapped, attr)
-
-    qpos = dataset['qpos'] if ('maze' in env_name or 'soccer' in env_name or 'cube' in env_name or 'scene' in env_name) else None
-    if 'maze' in env_name or 'soccer' in env_name:
-        start = 0 if 'maze' in env_name else 15            # agent xy, or the ball's xy for antsoccer
-        oracle_reps = qpos[:, start:start + 2]
-    elif 'cube' in env_name or 'scene' in env_name or 'puzzle' in env_name:
-        obj0, cube_len = 14, 7
-        xyz_center = np.array([0.425, 0.0, 0.0])
-        if 'puzzle' in env_name:
-            oracle_reps = dataset['button_states'].copy()
-        else:
-            n_cubes = count('_num_cubes', num_cubes)
-            cube_xyzs = np.stack([qpos[:, obj0 + i * cube_len:obj0 + i * cube_len + 3] for i in range(n_cubes)], axis=1)
-            cube_reps = ((cube_xyzs - xyz_center) * 10.0).reshape(-1, n_cubes * 3)
-            if 'cube' in env_name:
-                oracle_reps = cube_reps
-            else:
-                drawer = obj0 + n_cubes * cube_len + count('_num_buttons', num_buttons)
-                oracle_reps = np.concatenate(
-                    [cube_reps, dataset['button_states'].copy(), qpos[:, [drawer]] * 18.0, qpos[:, [drawer + 1]] * 15.0], axis=-1)
-    else:
-        raise ValueError(f'Unsupported environment: {env_name}')
-    dataset['oracle_reps'] = oracle_reps.astype(np.float32)
+    dataset.update(_oracle_relabelling(env_name, env, num_cubes, num_buttons).rows(dataset))
 
 
 def relabel_dataset(env_name, env, dataset):
@@ -112,36 +194,64 @@ def relabel_dataset(env_name, env, dataset):
     manipulation); `env.reset()` is called first, as in the reference, so that the task is set.  The dataset must carry
     'qpos' (and 'button_states' for scene / puzzle), i.e. be loaded with add_info=True.
     """
-    task = env.unwrapped
-    assert task._reward_task_id is not None, 'The environment is not in the single-task mode.'
-    env.reset()
-    tol = 0.04                                              # object / drawer / window tolerance of the manipulation tasks
-    if 'maze' in env_name or 'soccer' in env_name:
-        first = 0 if 'maze' in env_name else 15             # the agent's xy, or the ball's for antsoccer
-        gap = np.linalg.norm(dataset['qpos'][:, first:first + 2] - task.cur_goal_xy, axis=-1)
-        reached = (gap <= task._goal_tol).astype(np.float32)
-        rewards, masks = reached - 1.0, 1.0 - reached       # -1 until the goal is reached; the episode stops mattering there
-    elif 'cube' in env_name or 'scene' in env_name or 'puzzle' in env_name:
-        obj0, cube_len = 14, 7
-        done = []                                           # one boolean column per sub-goal of the task
-        if 'cube' in env_name or 'scene' in env_name:
-            n_cubes = task._num_cubes
-            xyz = np.stack([dataset['qpos'][:, obj0 + c * cube_len:obj0 + c * cube_len + 3] for c in range(n_cubes)], axis=1)
-            done.append(np.linalg.norm(task._data.mocap_pos.copy() - xyz, axis=-1) <= tol)
-        if 'scene' in env_name and 'cube' not in env_name:
-            drawer = obj0 + task._num_cubes * cube_len + task._num_buttons
-            done.append(dataset['button_states'] == task._target_button_states.copy())
-            done.append((np.abs(dataset['qpos'][:, drawer] - task._target_drawer_pos) <= tol)[:, None])
-            done.append((np.abs(dataset['qpos'][:, drawer + 1] - task._target_window_pos) <= tol)[:, None])
-        if 'puzzle' in env_name and 'cube' not in env_name and 'scene' not in env_name:
-            done.append(dataset['button_states'] == task._target_button_states.copy())
-        done = np.concatenate(done, axis=-1)
-        rewards = done.sum(axis=-1) - done.shape[-1]        # minus the number of unfinished sub-goals
-        masks = 1.0 - np.all(done, axis=-1)
+    dataset.update(_task_relabelling(env_name, env).rows(dataset))
+
+
+class _DatasetName(NamedTuple):
+    """What a dataset name of make_datasets says: the environment, the files' stem, the dtypes of the family, whether the
+    info members are read (the relabelled names need them) and which relabellings apply."""
+    env_name: str
+    file_stem: str
+    ob_dtype: type
+    action_dtype: type
+    load_info: bool
+    singletask: bool
+    oraclerep: bool
+
+    def paths(self, dataset_dir='~/.ogbench/data', dataset_path=None):
+        """(train, validation) files; FileNotFoundError when either is missing."""
+        import os
+
+        if dataset_path is None:
+            dataset_dir = os.path.expanduser(dataset_dir)
+            out = os.path.join(dataset_dir, f'{self.file_stem}.npz'), os.path.join(dataset_dir, f'{self.file_stem}-val.npz')
+        else:
+            out = dataset_path, dataset_path.replace('.npz', '-val.npz')
+        for path in out:
+            if not os.path.exists(path):
+                raise FileNotFoundError(f'{path} (datasets are not downloaded by this loader)')
+        return out
+
+    def stream(self, path, compact_dataset, add_info, env, num_cubes=None, num_buttons=None) -> '_FileStream':
+        """make_datasets' result for the split `path` as a _FileStream; a single-task `env` is reset here, once."""
+        relabellings = [_task_relabelling(self.env_name, env)] if self.singletask else []
+        if self.oraclerep:
+            relabellings.append(_oracle_relabelling(self.env_name, env, num_cubes, num_buttons))
+        return _FileStream(path, self.ob_dtype, self.action_dtype, compact_dataset, add_info, relabellings)
+
+
+def _parse_dataset_name(dataset_name, add_info=False, env=None) -> _DatasetName:
+    """make_datasets' reading of `dataset_name` (ogbench/utils.py:164-203); a 'singletask' name without `env` is a
+    ValueError."""
+    splits = dataset_name.split('-')
+    load_info = add_info
+    if 'singletask' in splits:
+        if env is None:
+            raise ValueError("'singletask' datasets are relabelled with the task of the single-task environment: pass env= "
+                             '(ogbench/utils.py:164-171, relabel_utils.py:4-90)')
+        pos = splits.index('singletask')
+        env_name = '-'.join(splits[:pos - 1] + splits[pos:])      # remove the dataset type
+        dataset_name = '-'.join(splits[:pos] + splits[-1:])        # the files carry neither 'singletask' nor 'task<n>'
+        load_info = True
+    elif 'oraclerep' in splits:
+        env_name = '-'.join(splits[:-3] + splits[-1:])         # remove the dataset type and the word 'oraclerep'
+        dataset_name = '-'.join(splits[:-2] + splits[-1:])     # the files carry no 'oraclerep'
+        load_info = True
     else:
-        raise ValueError(f'Unsupported environment: {env_name}')
-    dataset['rewards'] = rewards.astype(np.float32)
-    dataset['masks'] = masks.astype(np.float32)
+        env_name = '-'.join(splits[:-2] + splits[-1:])         # remove the dataset type
+    ob_dtype = np.uint8 if ('visual' in env_name or 'powderworld' in env_name) else np.float32
+    action_dtype = np.int32 if 'powderworld' in env_name else np.float32
+    return _DatasetName(env_name, dataset_name, ob_dtype, action_dtype, load_info, 'singletask' in splits, 'oraclerep' in splits)
 
 
 def make_datasets(dataset_name, dataset_dir='~/.ogbench/data', dataset_path=None, compact_dataset=False, add_info=False,
@@ -150,44 +260,17 @@ def make_datasets(dataset_name, dataset_dir='~/.ogbench/data', dataset_path=None
     train / validation files of `dataset_name`, picks the dtypes by environment family, loads both splits and, for
     '-oraclerep-' names, adds the oracle goal representations.  Returns (train_dataset, val_dataset) as dicts of host
     arrays; 'singletask' names are relabelled with the rewards / masks of `env`'s fixed task (relabel_dataset).  Nothing is
-    downloaded (the files must exist).
+    downloaded (the files must exist).  upload_datasets gives the same datasets in HBM without the host copy.
     """
-    import os
-
-    splits = dataset_name.split('-')
-    dataset_add_info = add_info
-    if 'singletask' in splits:
-        if env is None:
-            raise ValueError("'singletask' datasets are relabelled with the task of the single-task environment: pass env= "
-                             '(ogbench/utils.py:164-171, relabel_utils.py:4-90)')
-        pos = splits.index('singletask')
-        env_name = '-'.join(splits[:pos - 1] + splits[pos:])      # remove the dataset type
-        dataset_name = '-'.join(splits[:pos] + splits[-1:])        # the files carry neither 'singletask' nor 'task<n>'
-        dataset_add_info = True
-    elif 'oraclerep' in splits:
-        env_name = '-'.join(splits[:-3] + splits[-1:])         # remove the dataset type and the word 'oraclerep'
-        dataset_name = '-'.join(splits[:-2] + splits[-1:])     # the files carry no 'oraclerep'
-        dataset_add_info = True
-    else:
-        env_name = '-'.join(splits[:-2] + splits[-1:])         # remove the dataset type
-    if dataset_path is None:
-        dataset_dir = os.path.expanduser(dataset_dir)
-        train_path = os.path.join(dataset_dir, f'{dataset_name}.npz')
-        val_path = os.path.join(dataset_dir, f'{dataset_name}-val.npz')
-    else:
-        train_path, val_path = dataset_path, dataset_path.replace('.npz', '-val.npz')
-    for path in (train_path, val_path):
-        if not os.path.exists(path):
-            raise FileNotFoundError(f'{path} (datasets are not downloaded by this loader)')
-    ob_dtype = np.uint8 if ('visual' in env_name or 'powderworld' in env_name) else np.float32
-    action_dtype = np.int32 if 'powderworld' in env_name else np.float32
+    name = _parse_dataset_name(dataset_name, add_info, env)
     out = []
-    for path in (train_path, val_path):
-        ds = load_dataset(path, ob_dtype=ob_dtype, action_dtype=action_dtype, compact_dataset=compact_dataset, add_info=dataset_add_info)
-        if 'singletask' in splits:
-            relabel_dataset(env_name, env, ds)
-        if 'oraclerep' in splits:
-            add_oracle_reps(env_name, env, ds, num_cubes=num_cubes, num_buttons=num_buttons)
+    for path in name.paths(dataset_dir, dataset_path):
+        ds = load_dataset(path, ob_dtype=name.ob_dtype, action_dtype=name.action_dtype, compact_dataset=compact_dataset,
+                          add_info=name.load_info)
+        if name.singletask:
+            relabel_dataset(name.env_name, env, ds)
+        if name.oraclerep:
+            add_oracle_reps(name.env_name, env, ds, num_cubes=num_cubes, num_buttons=num_buttons)
         if not add_info:
             for k in ('qpos', 'qvel', 'button_states'):
                 ds.pop(k, None)
@@ -376,6 +459,19 @@ def _terminal_rows(terminals, r0, r1):
     return t, follows
 
 
+def _lockstep(readers):
+    """Lists of same-row blocks, one per reader, from readers that yield the consecutive rows of members of equal length
+    (a block is cut where another reader's block ends first: a member read whole yields one block)."""
+    pending = [None] * len(readers)
+    while True:
+        pending = [p if p is not None and len(p) else next(r, None) for p, r in zip(pending, readers)]
+        if any(p is None for p in pending):
+            return
+        m = min(len(p) for p in pending)
+        yield [p[:m] for p in pending]
+        pending = [p[m:] for p in pending]
+
+
 class _FileStream:
     """`load_dataset(path, ...)` of one `.npz` file as row writes computed a block at a time.
 
@@ -386,15 +482,23 @@ class _FileStream:
     block go to `i - (terminals before i)`, and the same cast observation block, shifted by one row, gives the block's
     `next_observations`.  With the compact layout `flags` holds one byte of `valids > 0` per row once the terminal
     producer has run.
+
+    `relabellings` (make_datasets' for a relabelled name) add their derived fields after load_dataset's, as make_datasets
+    does.  One producer reads the info members they need in blocks of the same rows, lays them out like any member and
+    yields the derived rows of each block, and the info rows too when `add_info` keeps them; without `add_info` no info
+    field is kept and an info member nothing is derived from is not read.
     """
 
-    def __init__(self, path, ob_dtype=np.float32, action_dtype=np.float32, compact_dataset=False, add_info=False):
+    def __init__(self, path, ob_dtype=np.float32, action_dtype=np.float32, compact_dataset=False, add_info=False,
+                 relabellings=()):
         self.path, self.compact = str(path), compact_dataset
+        self.relabellings = list(relabellings)
+        self.sources = [k for k in _INFO_KEYS if any(k in r.members for r in self.relabellings)]
         with zipfile.ZipFile(self.path) as zf:
             present = set(zf.namelist())
             keys = ['observations', 'actions', 'terminals'] + [k for k in _INFO_KEYS if add_info and f'{k}.npy' in present]
             heads = {}
-            for k in keys:
+            for k in keys + [k for k in self.sources if k not in keys]:
                 with _open_member(zf, self.path, k) as f:
                     heads[k] = _read_npy_header(f, self.path, k)
         self.terminals = _read_member(self.path, 'terminals')
@@ -403,7 +507,8 @@ class _FileStream:
             if len(shape) < 1 or shape[0] != n:
                 raise ValueError(f'{self.path}: member {k!r} of shape {shape} does not have the {n} rows of terminals')
         self.casts = {'observations': np.dtype(ob_dtype), 'actions': np.dtype(action_dtype)}
-        self.members = [k for k in keys if k != 'terminals']
+        self.members = [k for k in keys if k != 'terminals' and k not in self.sources]
+        self.source_row_bytes = sum(heads[k][1].itemsize * int(np.prod(heads[k][0][1:], dtype=np.int64)) for k in self.sources)
         obs_row = heads['observations'][0][1:]
         if compact_dataset:
             self.keep, rows, next_rows = None, n, None
@@ -420,9 +525,34 @@ class _FileStream:
             self.fields['valids'] = (np.dtype(np.float32), (rows,))
         else:
             self.fields['next_observations'] = (self.casts['observations'], (next_rows, *obs_row))
+        # the derived fields' dtypes and row shapes: the relabellings applied to no rows of the members
+        empty = {k: np.zeros((0, *heads[k][0][1:]), heads[k][1]) for k in self.sources}
+        for relabelling in self.relabellings:
+            self.fields.update({k: (a.dtype, (rows, *a.shape[1:])) for k, a in relabelling.rows(empty).items()})
 
     def producers(self, block_rows: Optional[int] = None):
-        return [self._member_writes(k, block_rows) for k in self.members] + [self._terminal_writes(block_rows)]
+        derived = [self._derived_writes(block_rows)] if self.relabellings else []
+        return [self._member_writes(k, block_rows) for k in self.members] + derived + [self._terminal_writes(block_rows)]
+
+    def _derived_writes(self, block_rows):
+        """The relabellings' fields (and the info fields they read, when kept), from the info members read in blocks of
+        the same rows and laid out as _member_writes lays out a member."""
+        rows = block_rows or max(1, _BLOCK_BYTES // max(1, self.source_row_bytes))
+        r0 = dest = 0
+        with contextlib.ExitStack() as stack:
+            readers = [stack.enter_context(contextlib.closing(read_member_blocks(self.path, k, rows))) for k in self.sources]
+            for blocks in _lockstep(readers):
+                r1 = r0 + len(blocks[0])
+                info = dict(zip(self.sources, blocks))
+                if not self.compact:
+                    keep = self.keep[r0:r1]
+                    info = {k: b[keep] for k, b in info.items()}
+                out = {k: b for k, b in info.items() if k in self.fields}
+                for relabelling in self.relabellings:
+                    out.update(relabelling.rows(info))
+                yield (r0 if self.compact else dest), out
+                dest += len(next(iter(out.values())))
+                r0 = r1
 
     def _member_writes(self, key, block_rows):
         cast = self.casts.get(key)
@@ -533,10 +663,33 @@ def upload_dataset(dataset_path, ob_dtype=np.float32, action_dtype=np.float32, c
     thread per member, cast and laid out per block, and written into HBM, so host memory holds a few blocks per member
     and a few bytes per row instead of the whole file.  The dataset samples byte for byte what the host-loaded one does;
     it keeps no host copy of its fields (ResidentDataset)."""
-    stream = _FileStream(dataset_path, ob_dtype, action_dtype, compact_dataset, add_info)
+    return _upload(_FileStream(dataset_path, ob_dtype, action_dtype, compact_dataset, add_info), device)
+
+
+def upload_datasets(dataset_name, dataset_dir='~/.ogbench/data', dataset_path=None, compact_dataset=False, add_info=False,
+                    env=None, num_cubes=None, num_buttons=None, device: int = 0):
+    """`make_datasets(...)` in HBM: (train, val) as ResidentDatasets, each sampling byte for byte what
+    `Dataset.create(**make_datasets(...)[i])` samples, for plain, '-oraclerep-' and 'singletask' names alike.  Each split
+    is streamed as upload_dataset streams a file; the relabelled fields are computed per block of `qpos` /
+    `button_states` rows with make_datasets' own expressions, so host memory holds a few blocks per member whatever the
+    file's size.  The name and the files are checked before any file is read, with make_datasets' errors; a single-task
+    `env` is reset once per split, as make_datasets resets it."""
+    return tuple(_upload(stream, device) for stream in _split_streams(dataset_name, dataset_dir, dataset_path, compact_dataset,
+                                                                       add_info, env, num_cubes, num_buttons))
+
+
+def _split_streams(dataset_name, dataset_dir, dataset_path, compact_dataset, add_info, env, num_cubes, num_buttons):
+    """make_datasets' (train, val) as a generator of _FileStreams.  The name and the files are checked at the call; a split's
+    relabellings are resolved when its stream is made, after the previous split has been consumed."""
+    name = _parse_dataset_name(dataset_name, add_info, env)
+    paths = name.paths(dataset_dir, dataset_path)
+    return (name.stream(path, compact_dataset, add_info, env, num_cubes, num_buttons) for path in paths)
+
+
+def _upload(stream: _FileStream, device: int) -> ResidentDataset:
     rows = {k: shape[0] for k, (_, shape) in stream.fields.items()}
     if len(set(rows.values())) != 1:      # a regular layout whose last row is not terminal: Dataset.create refuses it too
-        raise ValueError(f'{dataset_path}: fields of different lengths {rows}')
+        raise ValueError(f'{stream.path}: fields of different lengths {rows}')
     nds = _NativeDataset.empty({k: _ZeroField(shape, dtype) for k, (dtype, shape) in stream.fields.items()}, device)
     stream.write(nds, 0, list(stream.fields))
     n = rows['terminals']
@@ -552,23 +705,33 @@ class ResidentShards:
         shards[i], shards[path]   # Dataset of one shard: a view of the table, equal to Dataset.create(**load(path))
         shards.bounds             # [(row0, n_rows)] per shard
 
-    `load` is the per-file host loader.  By default each file is streamed into the table block by block as upload_dataset
-    does, with the result of load_dataset(p, compact_dataset=True), so host memory holds a few 8 MB blocks per member and
-    a few bytes per row.  A given `load` (`lambda p: make_datasets(name, dataset_path=p)[0]` for '-oraclerep-' and
-    'singletask' names, whose relabelling works on whole arrays) is called on one shard at a time, and each shard is
-    written and freed before the next is loaded, so host memory peaks at one shard plus a pinned staging buffer.  The
-    capacity comes from the files' headers.  Every shard must load with shard 0's fields, dtypes and row shapes.
+    By default each file is streamed into the table block by block as upload_dataset does, with the result of
+    load_dataset(p, compact_dataset=True), so host memory holds a few 8 MB blocks per member and a few bytes per row.
+    With `dataset_name` (and `env` / `num_cubes` / `num_buttons` as make_datasets takes them) each file is streamed the
+    same way with the result of `make_datasets(dataset_name, dataset_path=p, compact_dataset=True, ...)[0]`: that name's
+    dtypes, and for '-oraclerep-' and 'singletask' names its relabelled fields, computed per block (a single-task `env`
+    is reset once per shard).  `load`, a per-file host loader, is the alternative for anything else: it is called on one
+    shard at a time, and each shard is written and freed before the next is loaded, so host memory peaks at one shard
+    plus a pinned staging buffer.  `load` and `dataset_name` do not go together.  The capacity comes from the files'
+    headers.  Every shard must load with shard 0's fields, dtypes and row shapes.
 
     A view keeps the reference's shard-local semantics (goals, trajectory ends and next observations stay inside the
     shard) and a swap costs no upload; sampling `dataset` draws across every shard instead.  Shards end on trajectory
     boundaries, so each rank of a multi-GPU run can build its own ResidentShards over its subset of the paths.
     """
 
-    def __init__(self, paths, load: Optional[Callable[[str], dict]] = None, device: int = 0):
+    def __init__(self, paths, load: Optional[Callable[[str], dict]] = None, device: int = 0, *, dataset_name=None, env=None,
+                 num_cubes=None, num_buttons=None):
+        open_stream = None
+        if dataset_name is not None:
+            if load is not None:
+                raise ValueError('ResidentShards takes load= or dataset_name=, not both')
+            open_stream = functools.partial(_parse_dataset_name(dataset_name, env=env).stream, compact_dataset=True,
+                                            add_info=False, env=env, num_cubes=num_cubes, num_buttons=num_buttons)
         self.paths = [str(p) for p in paths]
         lib = _native.lib()
         nds, keys, nested, valids, self.bounds = None, None, False, [], []
-        for shard in iter_shards(self.paths, load):
+        for shard in iter_shards(self.paths, load, open_stream):
             if nds is None:
                 keys, nested = shard.keys, shard.nested
                 nds = _NativeDataset.empty({k: _ZeroField((shard.capacity, *s), d) for k, (d, s) in shard.schema.items()}, device)
@@ -604,13 +767,13 @@ class _Shard:
     __slots__ = ('path', 'row0', 'n_rows', 'capacity', 'keys', 'nested', 'schema', 'fields', 'stream')
 
 
-def iter_shards(paths, load: Optional[Callable[[str], dict]] = None):
+def iter_shards(paths, load: Optional[Callable[[str], dict]] = None, open_stream: Optional[Callable[[str], _FileStream]] = None):
     """The host half of ResidentShards: load the shards one at a time, in order, and yield each as a record with its
     first row in the concatenation (`row0`), its row count, its flattened fields and the schema -- {name: (dtype, row
     shape)} -- that shard 0 fixed; `capacity` is the rows the files' headers declare in all.  Without `load`, a record
-    holds no fields (`fields` is None) but the stream that writes load_dataset(path, compact_dataset=True) block by
-    block (`stream`, None when `load` is given).  A shard whose fields, dtypes or row shapes differ from shard 0's, or
-    that loads more rows than its header declares, raises ValueError naming it."""
+    holds no fields (`fields` is None) but the stream that writes the shard block by block (`stream`, None when `load`
+    is given): `open_stream(path)`, by default load_dataset(path, compact_dataset=True)'s.  A shard whose fields, dtypes
+    or row shapes differ from shard 0's, or that loads more rows than its header declares, raises ValueError naming it."""
     paths = [str(p) for p in paths]
     if not paths:
         raise ValueError('no shards given')
@@ -618,7 +781,8 @@ def iter_shards(paths, load: Optional[Callable[[str], dict]] = None):
     schema, row0 = None, 0
     for path, cap in zip(paths, declared):
         if load is None:
-            stream, fields = _FileStream(path, compact_dataset=True), None
+            stream = open_stream(path) if open_stream else _FileStream(path, compact_dataset=True)
+            fields = None
             shape = {k: (d, s[1:]) for k, (d, s) in stream.fields.items()}
             names, is_nested = list(stream.fields), False
             lengths = {s[0] for _, s in stream.fields.values()}

@@ -55,7 +55,9 @@ def write_member(zf, name, shape, dtype, chunks):
             f.write(np.ascontiguousarray(c, dtype).tobytes())
 
 
-def write_file(path, kind, rows, seed=0):
+def write_file(path, kind, rows, seed=0, info=False):
+    """With `info`, also float64 qpos[:, 40] (normal random values) and int64 button_states[:, 9] (0 / 1), the members
+    the '-oraclerep-' and 'singletask' relabellings read."""
     rng = np.random.default_rng(seed)
     chunk = 4096
     terminals = np.zeros(rows, bool)
@@ -85,8 +87,13 @@ def write_file(path, kind, rows, seed=0):
         write_member(zf, 'actions', (rows, 5), np.float32,
                      (rng.uniform(-1, 1, (min(chunk, rows - r0), 5)) for r0 in range(0, rows, chunk)))
         write_member(zf, 'terminals', (rows,), bool, [terminals])
+        if info:
+            write_member(zf, 'qpos', (rows, 40), np.float64,
+                         (rng.standard_normal((min(chunk, rows - r0), 40)) for r0 in range(0, rows, chunk)))
+            write_member(zf, 'button_states', (rows, 9), np.int64,
+                         (rng.integers(0, 2, (min(chunk, rows - r0), 9)) for r0 in range(0, rows, chunk)))
     return dict(path=path, rows=rows, file_bytes=os.path.getsize(path),
-                raw_bytes=rows * (int(np.prod(obs_shape[1:])) * np.dtype(obs_dtype).itemsize + 20 + 1))
+                raw_bytes=rows * (int(np.prod(obs_shape[1:])) * np.dtype(obs_dtype).itemsize + 20 + 1 + 392 * info))
 
 
 def child(mode, path, ob_dtype):
